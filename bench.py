@@ -2,7 +2,7 @@
 """bench.py -- the FPL+ hot path on B200: DSBN 3-D U-Net train step (voxels/s) + filtered-pseudo-label
 pass (volumes/s), with the roofline of the dominant kernel and the reference's CPU path beside it.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -420,8 +420,10 @@ def run_ours(args):
     clocks.start()
 
     # ---- kernel-side throughput: inputs resident in HBM; the step is replayed from the agent's CUDA graph ----
+    last_out = [None]
+
     def step_resident():
-        agent.train_step(resident)
+        last_out[0] = agent.train_step(resident)
 
     for _ in range(max(args.warmup, 5)):          # includes the 3 eager steps + capture of the graph
         step_resident()
@@ -431,6 +433,9 @@ def run_ours(args):
     ms = max_over_ranks(ms)
     clk = clocks.stop(t0, t1)
     value = world * vox_per_step * args.steps / (ms / 1e3)
+    if args.dump_outputs and rank == 0:
+        # the legs below keep training the same network: snapshot the timed region's result before they run
+        dump_outputs(args.dump_outputs, last_out[0])
 
     # ---- end to end through the agent with HOST buffers: H2D of the batch + D2H of the loss per step ----
     # the loss of every step is read back to the host (4 bytes into pinned memory); the read of step i is
@@ -620,6 +625,18 @@ def run_ours(args):
         sys.stdout.flush()
         sys.stderr.flush()
         os._exit(0)
+
+
+def dump_outputs(path, step_out):
+    """--dump-outputs: what train_step returned for the last timed step, as DIR/<name>.npy: ``loss`` (float32) and
+    ``hard_dice_d<domain>``, the class-wise hard Dice of each domain pass (float64)."""
+    loss, dices = step_out
+    arrays = {"loss": loss}
+    arrays.update(("hard_dice_d%d" % d, h) for d, h in enumerate(dices) if h is not None)
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy()
+        np.save(os.path.join(path, name + ".npy"), a.astype(np.float64 if a.dtype == np.float64 else np.float32))
 
 
 def bench_filter(agent, rank, world, barrier, max_over_ranks, args):
@@ -994,9 +1011,13 @@ def main():
                     help="feed the PyMIC loader layout (fp32 one-hot labels, folded fp32 weights) instead of uint8 labels / codes")
     ap.add_argument("--config", default="configs2", choices=["configs2", "vs_shipped"],
                     help="configs2 = BASELINE.json configs[2] (default, the headline); vs_shipped = the authors' VS .cfg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the loss and hard Dice of the last one as DIR/<name>.npy")
     args = ap.parse_args()
     apply_workload(args.config)
     if args.impl == "reference":
+        if args.dump_outputs:
+            raise SystemExit("--dump-outputs writes the outputs of the CUDA path (--impl ours)")
         run_reference(args)
         return
     if args.warmup < 3:

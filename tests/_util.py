@@ -33,3 +33,13 @@ def rng(seed):
 
 def randn(seed, *shape, scale=1.0):
     return torch.from_numpy((rng(seed).standard_normal(shape) * scale).astype(np.float32))
+
+
+def golden_voxels(out, g, key):
+    """``out`` [N, C, ...] at the voxels a sampled golden array holds: g[key] is [N, C, M] at the flat voxel indices
+    g[key + '_idx'] of an output of shape g[key + '_shape']."""
+    assert tuple(out.shape) == tuple(int(s) for s in g[key + "_shape"]), (tuple(out.shape), g[key + "_shape"])
+    idx = g[key + "_idx"].astype(np.int64)
+    if torch.is_tensor(out):
+        idx = torch.from_numpy(idx).to(out.device)
+    return out.reshape(out.shape[0], out.shape[1], -1)[:, :, idx]

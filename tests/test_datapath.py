@@ -1,67 +1,24 @@
-"""Device data path (SURVEY 8 f-3): RandomCrop / RandomFlip decisions against the reference's own transforms (CPU, build
-container only) and the gather kernel against numpy slicing (GPU)."""
+"""Device data path (SURVEY 8 f-3): RandomCrop / RandomFlip decisions against the reference transforms' stored decisions
+(CPU) and the gather kernel against numpy slicing (GPU)."""
+import json
 import os
-import random
-import sys
 
 import numpy as np
 import pytest
 import torch
 
-REF = "/root/reference"
+from oracle.gen_golden_datapath import TRIALS, record, volumes as _volumes
 
 
-def _volumes(seed=0):
-    rng = np.random.default_rng(seed)
-    vols = []
-    for i, shape in enumerate([(40, 160, 150), (20, 140, 200), (36, 128, 128)]):          # the second is thinner than the patch
-        img = rng.standard_normal((1,) + shape).astype(np.float32)
-        lab = np.zeros(shape, np.uint8)
-        c = [s // 2 + int(rng.integers(-3, 4)) for s in shape]
-        lab[c[0] - 3:c[0] + 4, c[1] - 10:c[1] + 12, c[2] - 9:c[2] + 10] = 1
-        pw = np.where(rng.random(shape) < 0.1, 0.5, 1.0).astype(np.float32)
-        vols.append({"image": img, "label": lab, "pixel_weight": pw, "image_weight": 0.2 + 0.3 * i, "name": "v%d" % i})
-    return vols
-
-
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "PyMIC")), reason="reference tree not present")
-def test_crop_and_flip_decisions_follow_the_reference_transforms():
-    """Same python `random` stream -> the same crop origin and flip axes as pymic.transform.crop.RandomCrop
-    (crop.py:213-234, foreground focus) followed by pymic.transform.flip.RandomFlip (flip.py:38-47)."""
-    for p in (REF, os.path.join(REF, "PyMIC")):
-        if p not in sys.path:
-            sys.path.insert(0, p)
-    from oracle.gen_golden_fpl import _install_stubs
-    _install_stubs()
-    from pymic.transform.crop import RandomCrop
-    from pymic.transform.flip import RandomFlip
-    from fplplus_b200.datapath import DevicePatchSampler, pad_to
-    patch = (28, 128, 128)
-    vols = _volumes()
-    smp = DevicePatchSampler(vols, patch, 2, "cpu", fg_focus=True, fg_ratio=0.5, flip=(False, True, True), seed=7)
-    params = {"randomcrop_output_size": list(patch), "randomcrop_foreground_focus": True, "randomcrop_foreground_ratio": 0.5,
-              "randomcrop_mask_label": [1], "randomcrop_inverse": False, "task": "segmentation",
-              "randomflip_flip_depth": False, "randomflip_flip_height": True, "randomflip_flip_width": True,
-              "randomflip_inverse": False}
-    crop, flip = RandomCrop(params), RandomFlip(params)
-    state = smp.rng.getstate()
-    for trial in range(40):
-        v = smp.vols[trial % 3]
-        random.setstate(smp.rng.getstate())                                  # the reference draws from the global generator
-        got_min, got_flip = smp.draw(v)
-        img = pad_to(vols[trial % 3]["image"], patch)
-        lab = pad_to(vols[trial % 3]["label"], patch, "constant")[None]
-        sample = {"image": img, "label": lab}
-        _s, cmin, cmax = crop._get_crop_param(sample)
-        cropped = {"image": img[:, cmin[1]:cmax[1], cmin[2]:cmax[2], cmin[3]:cmax[3]]}
-        out = flip(cropped)
-        import json
-        axes = json.loads(out["RandomFlip_Param"])
-        ref_flip = (4 if -1 in axes else 0) | (2 if -2 in axes else 0) | (1 if -3 in axes else 0)
-        assert list(cmin[1:]) == list(got_min), (trial, cmin, got_min)
-        assert ref_flip == got_flip, (trial, axes, got_flip)
-        assert random.getstate() == smp.rng.getstate()                       # the same number of draws was consumed
-    assert smp.rng.getstate() != state
+def test_crop_and_flip_decisions_follow_the_reference_transforms(golden_dir):
+    """Same python `random` stream -> the same crop origin, flip axes and number of draws as pymic.transform.crop.RandomCrop
+    (crop.py:213-234, foreground focus) followed by pymic.transform.flip.RandomFlip (flip.py:38-47), trial by trial against
+    the decisions stored in tests/golden/datapath_decisions.json (oracle/gen_golden_datapath.py)."""
+    with open(os.path.join(golden_dir, "datapath_decisions.json")) as f:
+        g = json.load(f)
+    assert len(g["trials"]) == TRIALS
+    for got, want in zip(record(), g["trials"]):
+        assert got == want, (got, want)
 
 
 @pytest.mark.gpu

@@ -11,7 +11,7 @@ import torch
 
 from oracle import synth
 from oracle.gen_golden import NET_PARAMS, SHAPE
-from tests._util import max_rel, rel_l2
+from tests._util import golden_voxels, max_rel, rel_l2
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
@@ -364,6 +364,7 @@ def test_inferer_matches_reference_golden(golden_dir):
     for d in (0, 1):
         with torch.no_grad():
             out = Inferer(dict(cfg)).run(net, vol, d * torch.ones(1, dtype=torch.long)).cpu()
+        out = golden_voxels(out, g, f"net_tta1_d{d}")
         ref = torch.from_numpy(g[f"net_tta1_d{d}"])
         err = rel_l2(out, ref)
         print(f"inferer d{d}: rel_l2={err:.4f} agreement={_label_agreement(out, ref):.5f}")
@@ -389,8 +390,8 @@ def test_inferer_stitching_exact_with_toy_model(golden_dir):
     for tta in (0, 1):
         cfg = {"sliding_window_enable": True, "sliding_window_size": [16, 32, 32],
                "sliding_window_stride": [8, 16, 32], "tta_mode": tta, "class_num": 3}
-        out = Inferer(cfg).run(Toy(), img, torch.ones(1, dtype=torch.long)).cpu()
-        np.testing.assert_allclose(out.numpy(), g[f"toy_tta{tta}"], rtol=1e-4, atol=1e-5)
+        out = Inferer(cfg).run(Toy(), img, torch.ones(1, dtype=torch.long)).cpu().numpy()
+        np.testing.assert_allclose(golden_voxels(out, g, f"toy_tta{tta}"), g[f"toy_tta{tta}"], rtol=1e-4, atol=1e-5)
 
 
 def test_strict_state_dict_round_trip_and_dropout_hook():

@@ -1,4 +1,5 @@
-"""CPU, build container only (skipped where /root/reference does not exist): INTEGRATION.md section 1 executed -- the
+"""CPU: the drop-in network's state_dict layout against the reference network's (stored under tests/golden/), and, where
+the PyMIC source tree is present, INTEGRATION.md section 1 executed -- the
 REFERENCE's own `pymic.net_run_dsbn.agent_seg.SegmentationAgent` (under the import stubs of oracle/gen_golden_fpl.py for
 the packages its file-I/O side needs) takes the drop-in plugin objects through its own setters and factory methods:
 set_net_dict -> create_network, set_loss_dict -> create_loss_calculator, set_inferer, state_dict round trip with the
@@ -12,7 +13,24 @@ import pytest
 import torch
 
 REF = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "PyMIC")), reason="reference tree not present")
+needs_reference = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "PyMIC")),
+                                     reason="runs the reference agent class: needs the PyMIC source tree")
+
+
+@pytest.mark.parametrize("tag", ["vs_shipped", "configs2"])
+def test_state_dict_layout_matches_the_reference_network(golden_dir, tag):
+    """Checkpoints are interchangeable with the reference's: our state_dict has the reference UNet2D5_dsbn's 484 keys in
+    the same order with the same shapes and dtypes (tests/golden/reference_state_dict.json), and a state_dict of that
+    layout loads strictly."""
+    import json
+    from fplplus_b200.net import UNet2D5_dsbn
+    with open(os.path.join(golden_dir, "reference_state_dict.json")) as f:
+        g = json.load(f)["networks"][tag]
+    net = UNet2D5_dsbn(dict(g["params"]))
+    assert net.ft_chns == g["params"]["feature_chns"] and net.dims == g["params"]["conv_dims"]
+    ours = [[k, list(v.shape), str(v.dtype).replace("torch.", "")] for k, v in net.state_dict().items()]
+    assert len(ours) == 484 and ours == g["state_dict"]
+    net.load_state_dict({k: torch.zeros(shape, dtype=getattr(torch, dt)) for k, shape, dt in g["state_dict"]}, strict=True)
 
 
 @pytest.fixture(scope="module")
@@ -26,6 +44,7 @@ def ref_agent_cls():
     return SegmentationAgent
 
 
+@needs_reference
 @pytest.mark.parametrize("cfg_name", ["vs_t1s_S.cfg", "vs_t1s_g.cfg", "vs_t1s_weights.cfg"])
 def test_reference_agent_accepts_the_drop_in_plugins(ref_agent_cls, cfg_name):
     from pymic.util.parse_config import parse_config, synchronize_config

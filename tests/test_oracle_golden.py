@@ -11,10 +11,33 @@ import torch
 from oracle import fpl_filter, inferer, losses, synth, unet_dsbn
 from oracle.gen_golden import NET_PARAMS, SHAPE
 from oracle.gen_golden_fpl import CASES, fpl_case_logits
+from tests._util import golden_voxels
 
 
 def _load(golden_dir, name):
     return np.load(os.path.join(golden_dir, name), allow_pickle=False)
+
+
+@pytest.fixture(autouse=True)
+def _recording_thread_count():
+    """The golden vectors were recorded with 8 intra-op threads.  torch's CPU backward splits its float32 weight-gradient
+    reductions by thread count, so the oracle runs with the same split here (the forward does not depend on it)."""
+    saved = torch.get_num_threads()
+    torch.set_num_threads(8)
+    yield
+    torch.set_num_threads(saved)
+
+
+# conv biases that feed a training-mode BatchNorm: their gradient is exactly zero, so what backward computes for them
+# (here and in the golden file) is float32 rounding noise whose size depends on the host's thread count and vector width
+_BN_FED_BIASES = ("conv3d_1.bias", "conv3d_2.bias")
+
+
+def _assert_rounding_level(st, name, ref):
+    """Our gradient of ``name`` and the reference's both vanish next to the gradient of the same conv's weight."""
+    scale = st[name[:-len("bias")] + "weight"].grad.double().norm().item()
+    assert st[name].grad.double().norm().item() <= 1e-4 * scale, name
+    assert float(np.linalg.norm(ref)) <= 1e-4 * scale, name
 
 
 def test_state_dict_spec_matches_reference_count():
@@ -50,6 +73,9 @@ def test_net_train_step_grads_and_running_stats(golden_dir):
     n_with_grad = sum(v.numel() for v in st.values() if v.requires_grad and v.grad is not None)
     assert n_with_grad == int(g["n_params_with_grad"])
     for k in g.files:
+        if k.startswith(("grad::", "gradnorm::")) and k.endswith(_BN_FED_BIASES):
+            _assert_rounding_level(st, k.split("::", 1)[1], g[k])
+            continue
         if k.startswith("grad::"):
             name = k[6:]
             ours = st[name].grad.numpy()
@@ -100,14 +126,14 @@ def test_inferer_toy_and_net(golden_dir):
         cfg = {"sliding_window_enable": True, "sliding_window_size": [16, 32, 32],
                "sliding_window_stride": [8, 16, 32], "tta_mode": tta}
         out = inferer.run(toy, img, 3, cfg).numpy()
-        np.testing.assert_allclose(out, g[f"toy_tta{tta}"], rtol=1e-5, atol=1e-6)
+        np.testing.assert_allclose(golden_voxels(out, g, f"toy_tta{tta}"), g[f"toy_tta{tta}"], rtol=1e-5, atol=1e-6)
     vol = torch.from_numpy(synth.synth_image(1, 1, (24, 48, 48), seed=9))
     cfg = {"sliding_window_enable": True, "sliding_window_size": [16, 32, 32],
            "sliding_window_stride": [16, 32, 32], "tta_mode": 1}
     st = unet_dsbn.to_torch_state(synth.synth_state_dict())
     with torch.no_grad():
         out = inferer.run(lambda im: unet_dsbn.forward(st, im, 1, NET_PARAMS), vol, 2, cfg).numpy()
-    np.testing.assert_allclose(out, g["net_tta1_d1"], rtol=1e-4, atol=1e-5)
+    np.testing.assert_allclose(golden_voxels(out, g, "net_tta1_d1"), g["net_tta1_d1"], rtol=1e-4, atol=1e-5)
 
 
 def test_window_enumeration_matches_survey_probe():
