@@ -562,9 +562,12 @@ class SegmentationAgent(object):
             # the two domain passes are independent until the optimiser: run them on two streams so that the
             # tensor-pipe-bound convolutions of one overlap the HBM-bound BatchNorm/activation kernels of the other
             # (autograd replays each backward on the stream its forward ran on)
-            refresh = getattr(self.net, "_refresh_weight_images", None)
-            if refresh is not None:
-                refresh(with_dgrad=True)               # staged once, before the fork
+            # every weight image both passes read is staged here, once, before the fork: a pass that staged one
+            # after the fork would race the other stream's reads
+            prepare = getattr(self.net, "prepare", None)
+            if prepare is not None:
+                for d in present:
+                    prepare(tuple(batches[d]['image'].shape), grad=True)
             if self._side_stream is None:
                 self._side_stream = torch.cuda.Stream()
             self._side_stream.wait_stream(main)

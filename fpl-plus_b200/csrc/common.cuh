@@ -194,100 +194,3 @@ struct EpiAct {
     uint64_t seed, offset;
     const unsigned long long* seed_dev;
 };
-
-// ---- DSBN backward statistics folded into the epilogue of the dgrad that PRODUCES the unit's output gradient ------------
-// conv_k+1's dgrad writes g = dL/da_k, the gradient wrt the activation a_k = dropout(prelu(bn(y_k))) of the previous conv
-// unit; the BatchNorm backward of unit k needs  sum dz, sum dz*xhat  (dz = g * dropout' * prelu') and  dslope = sum z*g|z<=0
-// BEFORE it can write dy_k (fpl_dsbn_act_bwd_reduce: one extra pass over y_k and g, 4 B/element).  The dgrad epilogue has
-// g in registers: it loads y_k for the same voxels (2 B/element) and accumulates the three sums with the butterfly the
-// forward epilogues use for the BatchNorm statistics, so the separate reduce launch disappears for every unit whose
-// activation feeds exactly one convolution (unit 1 of each ConvBlockND, unet2d5_dsbn.py:75-81).
-struct EpiBwdRed {
-    const bf16x8* y;            // raw conv output of unit k, dense C8-planar [N][D][C/8][H][W][8] (C = this kernel's Cout)
-    const float* scale;         // unit k: gamma * invstd
-    const float* shift;         //         beta - mean * scale (+ conv bias folded as in the forward)
-    const float* mean;
-    const float* invstd;
-    const float* slope;
-    float drop_p;               // unit k's dropout (Philox stream regenerated; explicit masks are not supported here)
-    uint64_t seed, offset;
-    const unsigned long long* seed_dev;
-    double* red;                // [2C + 1], ACCUMULATED into: sum dz, sum dz*xhat, dslope
-};
-
-// v[0..15]: fp32 gradient of one voxel wrt 16 consecutive channels (the values the caller stores as bf16); v[16..31] scratch.
-// ya / yb: the voxel's two 16-byte groups of y_k, loaded by the caller (PREFETCHED several steps ahead: the 128 epilogue
-// threads of a CTA cannot hide DRAM latency with loads issued at the point of use).  Afterwards lane L of the warp holds
-// in acc the warp's sum of dz for channel L (L < 16) or of dz*y for channel L - 16 (L >= 16); dsl accumulates this
-// thread's z*g over z <= 0.
-__device__ __forceinline__ void epi_bwdred16(float (&v)[32], bool valid, const int4& ya, const int4& yb, const float* sc,
-                                             const float* sh, float slope, bool drop, uint32_t keep0, uint32_t keep1,
-                                             float keep_scale, int lane, float& acc, float& dsl) {
-    float yf[16];
-    bf16x8_to_float(*reinterpret_cast<const bf16x8*>(&ya), yf);
-    bf16x8_to_float(*reinterpret_cast<const bf16x8*>(&yb), yf + 8);
-#pragma unroll
-    for (int i = 0; i < 16; ++i) {
-        float g = __bfloat162float(__float2bfloat16_rn(v[i]));          // the stored (rounded) gradient, as the apply pass reads it
-        if (drop) g = (((i < 8 ? keep0 >> i : keep1 >> (i - 8)) & 1u) != 0u) ? g * keep_scale : 0.0f;
-        const float z = fmaf(yf[i], sc[i], sh[i]);
-        const bool pos = z > 0.0f;
-        const float dz = valid ? (pos ? g : g * slope) : 0.0f;
-        if (valid && !pos) dsl = fmaf(z, g, dsl);
-        v[i] = dz;
-        v[16 + i] = dz * yf[i];
-    }
-    warp_transpose_sum32(v, lane);
-    acc += v[0];
-}
-
-// Per-thread form: acc32[0..15] += dz, acc32[16..31] += dz*y of THIS thread's voxel; the caller transposes acc32 across
-// the warp (warp_transpose_sum32) once, after its last step.
-__device__ __forceinline__ void epi_bwdred16_acc(const float (&v)[32], bool valid, const int4& ya, const int4& yb, const float* sc,
-                                                 const float* sh, float slope, bool drop, uint32_t keep0, uint32_t keep1,
-                                                 float keep_scale, float (&acc32)[32], float& dsl) {
-    if (!valid) return;
-    float yf[16];
-    bf16x8_to_float(*reinterpret_cast<const bf16x8*>(&ya), yf);
-    bf16x8_to_float(*reinterpret_cast<const bf16x8*>(&yb), yf + 8);
-#pragma unroll
-    for (int i = 0; i < 16; ++i) {
-        float g = __bfloat162float(__float2bfloat16_rn(v[i]));
-        if (drop) g = (((i < 8 ? keep0 >> i : keep1 >> (i - 8)) & 1u) != 0u) ? g * keep_scale : 0.0f;
-        const float z = fmaf(yf[i], sc[i], sh[i]);
-        const bool pos = z > 0.0f;
-        const float dz = pos ? g : g * slope;
-        if (!pos) dsl = fmaf(z, g, dsl);
-        acc32[i] += dz;
-        acc32[16 + i] = fmaf(dz, yf[i], acc32[16 + i]);
-    }
-}
-
-// the two y_k groups of one (voxel, 16-channel chunk) step; zeros outside the volume
-struct BrPre {
-    int4 a, b;
-};
-__device__ __forceinline__ BrPre epi_bwdred_load(const bf16x8* y, int64_t vec0, int64_t HW, bool valid) {
-    BrPre r;
-    r.a = make_int4(0, 0, 0, 0);
-    r.b = make_int4(0, 0, 0, 0);
-    if (valid) {
-        r.a = ld_stream16(y + vec0);
-        r.b = ld_stream16(y + vec0 + HW);
-    }
-    return r;
-}
-constexpr int kBrPrefetch = 4;      // steps of look-ahead (a step = one 16-channel chunk of one 128-voxel tile / plane)
-
-// end of a slice: lane L < 16 owns sum dz of channel ch0 + L, lane L + 16 the matching sum dz*y
-__device__ __forceinline__ void epi_bwdred_flush(const EpiBwdRed& R, int C, int ch0, float acc, int lane) {
-    const float s1 = __shfl_sync(0xffffffffu, acc, lane & 15);
-    const int c = ch0 + (lane & 15);
-    if (lane < 16) {
-        atomicAdd(R.red + c, (double)acc);
-    } else {
-        // sum dz*xhat = invstd * (sum dz*y - mean * sum dz)
-        atomicAdd(R.red + C + c, (double)__ldg(R.invstd + c) * ((double)acc - (double)__ldg(R.mean + c) * (double)s1));
-    }
-}
-

@@ -64,7 +64,7 @@ bool make_config(int cin, int cout, TcConfig& c) {
     int cols = 2 * c.nb;
     c.tmem_cols = 32;
     while (c.tmem_cols < cols) c.tmem_cols *= 2;
-    c.smem_bytes = c.stages * c.stage_bytes + 1024 /*align*/ + 256 /*barriers*/ + 4 * cout * (int)sizeof(float) + 16;
+    c.smem_bytes = c.stages * c.stage_bytes + 1024 /*align*/ + 256 /*barriers*/ + 2 * cout * (int)sizeof(float) + 16;
     return true;
 }
 
@@ -83,7 +83,6 @@ struct TcParams {
     float* logits;        // head mode: fp32 NCDHW output of the first `classes` channels instead of bf16 C8-planar
     int classes;
     EpiAct act;           // act.scale != NULL: inference epilogue (affine + PReLU + dropout) instead of + bias
-    EpiBwdRed br;         // br.red != NULL (dgrad): BatchNorm-backward sums of the unit whose activation gradient is written
 };
 
 struct TileCoord {
@@ -130,13 +129,9 @@ __global__ void __launch_bounds__(kNumThreads) conv3d_tc_kernel(const __grid_con
     FPL_PDL_WAIT();      // prologue above overlapped the previous kernel's tail; from here on its results are visible
     float* scale_sm = bias_sm + P.cout;
     const bool fuse_act = P.act.scale != nullptr;
-    float* br_sc = scale_sm + P.cout;
-    float* br_sh = br_sc + P.cout;
-    const bool fuse_br = P.br.red != nullptr;
     for (int i = threadIdx.x; i < P.cout; i += kNumThreads) {
         bias_sm[i] = fuse_act ? P.act.shift[i] : (P.bias != nullptr ? P.bias[i] : 0.0f);
         scale_sm[i] = fuse_act ? P.act.scale[i] : 1.0f;
-        if (fuse_br) { br_sc[i] = P.br.scale[i]; br_sh[i] = P.br.shift[i]; }
     }
     tc_fence_before();
     __syncthreads();
@@ -246,24 +241,17 @@ __global__ void __launch_bounds__(kNumThreads) conv3d_tc_kernel(const __grid_con
         for (int k = 0; k < kMaxChunks; ++k) run[k] = 0.0f;
         const bool want_stats = P.stats != nullptr;
         const int nchunk16 = P.nb / 16;
-        // fused BatchNorm-backward statistics (dgrad only; exclusive with want_stats, so `run` is shared)
-        const float br_slope = fuse_br ? __ldg(P.br.slope) : 0.0f;
-        const bool br_drop = fuse_br && P.br.drop_p > 0.0f;
-        const float br_keep_scale = br_drop ? 1.0f / (1.0f - P.br.drop_p) : 1.0f;
-        const uint64_t br_seed = br_drop ? P.br.seed + (P.br.seed_dev != nullptr ? (uint64_t)__ldg(P.br.seed_dev) : 0ull) : 0ull;
-        float br_dsl = 0.0f;
         const float act_slope = fuse_act ? __ldg(P.act.slope) : 0.0f;
         const float act_keep_scale = (fuse_act && P.act.drop_p > 0.0f) ? 1.0f / (1.0f - P.act.drop_p) : 1.0f;
         const uint64_t act_seed = fuse_act ? P.act.seed + (P.act.seed_dev != nullptr ? (uint64_t)__ldg(P.act.seed_dev) : 0ull) : 0ull;
         for (int t = blockIdx.x; t < P.total_tiles; t += gridDim.x) {
             TileCoord c = decode_tile(P, t);
-            if ((want_stats || fuse_br) && c.slice != cur_slice) {
+            if (want_stats && c.slice != cur_slice) {
                 if (cur_slice >= 0) {
 #pragma unroll
                     for (int k = 0; k < kMaxChunks; ++k) {
                         if (k < nchunk16) {
-                            if (want_stats) atomicAdd(P.stats + (lane >> 4) * P.cout + cur_slice * P.nb + k * 16 + (lane & 15), (double)run[k]);
-                            else epi_bwdred_flush(P.br, P.cout, cur_slice * P.nb + k * 16, run[k], lane);
+                            atomicAdd(P.stats + (lane >> 4) * P.cout + cur_slice * P.nb + k * 16 + (lane & 15), (double)run[k]);
                             run[k] = 0.0f;
                         }
                     }
@@ -273,15 +261,6 @@ __global__ void __launch_bounds__(kNumThreads) conv3d_tc_kernel(const __grid_con
             const int h = c.h0 + hl, w = c.w0 + wl;
             const bool valid = h < P.H && w < P.W;
             const int64_t HW = (int64_t)P.H * P.W;
-            // fused BatchNorm-backward sums: the tile's y_k chunks are requested BEFORE waiting for the tile's MMAs and
-            // kept kBrPrefetch steps ahead in a rotating register window
-            BrPre br_pre[kBrPrefetch];
-            const int64_t br_vec_tile = (((int64_t)c.n * P.D + c.d) * (P.cout >> 3) + (c.slice * P.nb) / 8) * HW + (int64_t)h * P.W + w;
-            if (fuse_br) {
-#pragma unroll
-                for (int q = 0; q < kBrPrefetch; ++q)
-                    br_pre[q] = epi_bwdred_load(P.br.y, br_vec_tile + (int64_t)(2 * q) * HW, HW, valid && q < nchunk16);
-            }
             mbar_wait(&tmem_full[acc], acc_phase);
             tc_fence_after();
             const int64_t out_base = (((int64_t)c.n * P.D + c.d) * P.y_c8tot + P.y_c8off + (c.slice * P.nb) / 8) * HW +
@@ -349,20 +328,6 @@ __global__ void __launch_bounds__(kNumThreads) conv3d_tc_kernel(const __grid_con
                         }
                         warp_transpose_sum32(v, lane);
                         run[k] += v[0];
-                    } else if (fuse_br) {
-                        const int64_t vec0 = br_vec_tile + (int64_t)(2 * k) * HW;
-                        uint32_t keep0 = 0xffu, keep1 = 0xffu;
-                        if (br_drop && valid) {
-                            keep0 = dropout_keep8(br_seed, P.br.offset, (uint64_t)vec0, P.br.drop_p);
-                            keep1 = dropout_keep8(br_seed, P.br.offset, (uint64_t)(vec0 + HW), P.br.drop_p);
-                        }
-                        const BrPre cur = br_pre[0];
-#pragma unroll
-                        for (int q = 0; q + 1 < kBrPrefetch; ++q) br_pre[q] = br_pre[q + 1];
-                        br_pre[kBrPrefetch - 1] = epi_bwdred_load(P.br.y, br_vec_tile + (int64_t)(2 * (k + kBrPrefetch)) * HW, HW,
-                                                                  valid && k + kBrPrefetch < nchunk16);
-                        epi_bwdred16(v, valid, cur.a, cur.b, br_sc + c.slice * P.nb + c0, br_sh + c.slice * P.nb + c0,
-                                     br_slope, br_drop, keep0, keep1, br_keep_scale, lane, run[k], br_dsl);
                     }
                 }
             }
@@ -376,15 +341,6 @@ __global__ void __launch_bounds__(kNumThreads) conv3d_tc_kernel(const __grid_con
             for (int k = 0; k < kMaxChunks; ++k)
                 if (k < nchunk16)
                     atomicAdd(P.stats + (lane >> 4) * P.cout + cur_slice * P.nb + k * 16 + (lane & 15), (double)run[k]);
-        }
-        if (fuse_br) {
-            if (cur_slice >= 0) {
-#pragma unroll
-                for (int k = 0; k < kMaxChunks; ++k)
-                    if (k < nchunk16) epi_bwdred_flush(P.br, P.cout, cur_slice * P.nb + k * 16, run[k], lane);
-            }
-            br_dsl = warp_sum(br_dsl);
-            if (lane == 0 && br_dsl != 0.0f) atomicAdd(P.br.red + 2 * P.cout, (double)br_dsl);
         }
     }
     tc_fence_before();
@@ -535,8 +491,7 @@ extern "C" void fpl_debug_set(int key, long long value) {
 
 static int conv3d_tc_launch(const void* x, int x_c8tot, int x_c8off, const void* image, const float* bias, void* y,
                             int y_c8tot, int y_c8off, double* stats, int n, int d, int h, int w, int cin, int cout,
-                            int kd, float* logits, int classes, void* stream, const EpiAct* act = nullptr,
-                            const EpiBwdRed* br = nullptr) {
+                            int kd, float* logits, int classes, void* stream, const EpiAct* act = nullptr) {
     TcConfig c;
     FPL_REQUIRE(make_config(cin, cout, c), "fpl_conv3d_tc: unsupported channels (%d -> %d); need multiples of 16", cin, cout);
     FPL_REQUIRE(kd == 1 || kd == 3, "fpl_conv3d_tc: kd=%d must be 1 or 3", kd);
@@ -576,7 +531,6 @@ static int conv3d_tc_launch(const void* x, int x_c8tot, int x_c8off, const void*
     P.total_tiles = (int)total;
     P.dbg_swap_lbo_sbo = g_dbg_swap;
     P.logits = logits; P.classes = classes;
-    if (br != nullptr) P.br = *br; else { P.br.y = nullptr; P.br.scale = P.br.shift = P.br.mean = P.br.invstd = P.br.slope = nullptr; P.br.drop_p = 0.0f; P.br.seed = P.br.offset = 0; P.br.seed_dev = nullptr; P.br.red = nullptr; }
     if (act != nullptr) P.act = *act; else { P.act.scale = nullptr; P.act.shift = nullptr; P.act.slope = nullptr; P.act.drop_p = 0.0f; P.act.seed = P.act.offset = 0; P.act.seed_dev = nullptr; }
     FPL_CHECK_CUDA(cudaFuncSetAttribute(conv3d_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, c.smem_bytes));
     int ctas_per_sm = c.smem_bytes <= 110 * 1024 ? 2 : 1;
@@ -628,22 +582,3 @@ extern "C" int fpl_head_conv_tc(const void* x, int x_c8tot, int x_c8off, const v
     return conv3d_tc_launch(x, x_c8tot, x_c8off, image16, bias16, nullptr, 0, 0, nullptr, n, d, h, w, cin, 16, 1, logits,
                             classes, stream);
 }
-
-/* dgrad form of fpl_conv3d_tc that ALSO accumulates the BatchNorm-backward sums of the unit whose activation gradient it
- * writes (see EpiBwdRed in common.cuh): y_prev = that unit's raw conv output (dense, `cout` channels), red = double[2*cout+1]
- * ACCUMULATED into {sum dz, sum dz*xhat, dslope}.  Replaces the fpl_dsbn_act_bwd_reduce launch of that unit. */
-extern "C" int fpl_conv3d_tc_bwdred(const void* x, int x_c8tot, int x_c8off, const void* image, void* y, int y_c8tot,
-                                    int y_c8off, int n, int d, int h, int w, int cin, int cout, int kd, const void* y_prev,
-                                    const float* scale, const float* shift, const float* mean, const float* invstd,
-                                    const float* slope, float drop_p, uint64_t seed, uint64_t offset, const uint64_t* seed_dev,
-                                    double* red, void* stream) {
-    FPL_REQUIRE(y_prev != nullptr && scale != nullptr && shift != nullptr && mean != nullptr && invstd != nullptr &&
-                slope != nullptr && red != nullptr, "fpl_conv3d_tc_bwdred: NULL argument");
-    FPL_REQUIRE(drop_p >= 0.0f && drop_p < 1.0f, "fpl_conv3d_tc_bwdred: dropout p=%f out of [0,1)", drop_p);
-    EpiBwdRed br;
-    br.y = (const bf16x8*)y_prev; br.scale = scale; br.shift = shift; br.mean = mean; br.invstd = invstd; br.slope = slope;
-    br.drop_p = drop_p; br.seed = seed; br.offset = offset; br.seed_dev = (const unsigned long long*)seed_dev; br.red = red;
-    return conv3d_tc_launch(x, x_c8tot, x_c8off, image, nullptr, y, y_c8tot, y_c8off, nullptr, n, d, h, w, cin, cout, kd,
-                            nullptr, 0, stream, nullptr, &br);
-}
-

@@ -39,7 +39,6 @@ struct DfParams {
     int taps;                        // 9 (k 3x3x3) or 1 (k 3x1x1: only the centre in-plane tap)
     int a_ksteps;                    // distinct 16-channel K steps of A (B K step j reads A K step j % a_ksteps)
     EpiAct act;                      // act.scale != NULL: inference epilogue (affine + PReLU) instead of + bias
-    EpiBwdRed br;                    // br.red != NULL (dgrad): BatchNorm-backward sums of the unit whose activation gradient is written
     int dbg_epi, dbg_nomma, dbg_tma;
     long long* dbg_trace;            // fpl_debug_set 47: CTA 0 logs clock64() per role and plane ([role][4096] entries)          // timing experiments only (fpl_debug_set 42 / 44): results are wrong when set
 };
@@ -84,7 +83,7 @@ __device__ __forceinline__ DfItem decode_item(const DfParams& P, int t) {
 }
 
 // NCH = nb / 16.  For NCH == 1 (Cout 16: the full-resolution layers, where a CTA walks ~60 planes per launch; 64
-// accumulator registers for Cout 32 would cost the second resident CTA) the per-channel sums of the epilogue (forward BatchNorm statistics or the fused BatchNorm-backward sums) are
+// accumulator registers for Cout 32 would cost the second resident CTA) the per-channel sums of the epilogue (forward BatchNorm statistics) are
 // accumulated PER THREAD (32 registers per chunk) and transposed across the warp once per CTA; the transposing
 // butterfly per plane (31 shuffles + ~90 ALU instructions on warps that have an SM sub-partition to themselves) made
 // the epilogue the pacing stage of the 16 -> 16 layers (52 us without statistics, 65 us with; tools/epi_probe.py).
@@ -119,13 +118,9 @@ __global__ void __launch_bounds__(kThreadsD, 2) conv3d_tc_dfold_kernel(const __g
     FPL_PDL_WAIT();      // prologue above overlapped the previous kernel's tail; from here on its results are visible
     float* scale_sm = bias_sm + P.cout;
     const bool fuse_act = P.act.scale != nullptr;
-    float* br_sc = scale_sm + P.cout;
-    float* br_sh = br_sc + P.cout;
-    const bool fuse_br = P.br.red != nullptr;
     for (int i = threadIdx.x; i < P.cout; i += kThreadsD) {
         bias_sm[i] = fuse_act ? P.act.shift[i] : (P.bias != nullptr ? P.bias[i] : 0.0f);
         scale_sm[i] = fuse_act ? P.act.scale[i] : 1.0f;
-        if (fuse_br) { br_sc[i] = P.br.scale[i]; br_sh[i] = P.br.shift[i]; }
     }
     tc_fence_before();
     __syncthreads();
@@ -288,16 +283,10 @@ __global__ void __launch_bounds__(kThreadsD, 2) conv3d_tc_dfold_kernel(const __g
         int cur_slice = -1;
         int ntr3 = 0;
         const float act_slope = fuse_act ? __ldg(P.act.slope) : 0.0f;
-        // fused BatchNorm-backward statistics (dgrad only; exclusive with want_stats, so `run` is shared)
-        const float br_slope = fuse_br ? __ldg(P.br.slope) : 0.0f;
-        const bool br_drop = fuse_br && P.br.drop_p > 0.0f;
-        const float br_keep_scale = br_drop ? 1.0f / (1.0f - P.br.drop_p) : 1.0f;
-        const uint64_t br_seed = br_drop ? P.br.seed + (P.br.seed_dev != nullptr ? (uint64_t)__ldg(P.br.seed_dev) : 0ull) : 0ull;
-        float br_dsl = 0.0f;
         for (int t = blockIdx.x; t < P.total_items; t += gridDim.x) {
             const DfItem c = decode_item(P, t);
             if (c.dcount == 0) continue;
-            if ((want_stats || fuse_br) && c.slice != cur_slice) {
+            if (want_stats && c.slice != cur_slice) {
                 if (cur_slice >= 0) {
 #pragma unroll
                     for (int k = 0; k < kMaxChunks; ++k)
@@ -308,8 +297,7 @@ __global__ void __launch_bounds__(kThreadsD, 2) conv3d_tc_dfold_kernel(const __g
 #pragma unroll
                                 for (int i = 0; i < 32; ++i) tacc[k][i] = 0.0f;
                             }
-                            if (want_stats) atomicAdd(P.stats + (lane >> 4) * P.cout + cur_slice * P.nb + k * 16 + (lane & 15), (double)run[k]);
-                            else epi_bwdred_flush(P.br, P.cout, cur_slice * P.nb + k * 16, run[k], lane);
+                            atomicAdd(P.stats + (lane >> 4) * P.cout + cur_slice * P.nb + k * 16 + (lane & 15), (double)run[k]);
                             run[k] = 0.0f;
                         }
                 }
@@ -318,7 +306,6 @@ __global__ void __launch_bounds__(kThreadsD, 2) conv3d_tc_dfold_kernel(const __g
             const int h = c.h0 + hl, w = c.w0 + wl;
             const bool valid = h < P.H && w < P.W;
             const int64_t HW = (int64_t)P.H * P.W;
-            const int64_t br_vec_item = ((int64_t)c.n * P.D + c.d0) * (P.cout >> 3) * HW + (int64_t)(c.slice * P.nb / 8) * HW + (int64_t)h * P.W + w;
             for (int p = 0; p < c.dcount; ++p) {
                 mbar_wait(&done_bar[p], item_phase);
                 tc_fence_after();
@@ -381,20 +368,6 @@ __global__ void __launch_bounds__(kThreadsD, 2) conv3d_tc_dfold_kernel(const __g
                                 warp_transpose_sum32(v, lane);
                                 run[k] += v[0];
                             }
-                        } else if (fuse_br) {
-                            const int64_t vec0 = br_vec_item + ((int64_t)p * (P.cout >> 3) + 2 * k) * HW;
-                            uint32_t keep0 = 0xffu, keep1 = 0xffu;
-                            if (br_drop && valid) {
-                                keep0 = dropout_keep8(br_seed, P.br.offset, (uint64_t)vec0, P.br.drop_p);
-                                keep1 = dropout_keep8(br_seed, P.br.offset, (uint64_t)(vec0 + HW), P.br.drop_p);
-                            }
-                            const BrPre cur = epi_bwdred_load(P.br.y, vec0, HW, valid);
-                            if (kThreadAcc)
-                                epi_bwdred16_acc(v, valid, cur.a, cur.b, br_sc + c.slice * P.nb + c0, br_sh + c.slice * P.nb + c0,
-                                                 br_slope, br_drop, keep0, keep1, br_keep_scale, tacc[k], br_dsl);
-                            else
-                                epi_bwdred16(v, valid, cur.a, cur.b, br_sc + c.slice * P.nb + c0, br_sh + c.slice * P.nb + c0,
-                                             br_slope, br_drop, keep0, keep1, br_keep_scale, lane, run[k], br_dsl);
                         }
                     }
                 }
@@ -417,15 +390,6 @@ __global__ void __launch_bounds__(kThreadsD, 2) conv3d_tc_dfold_kernel(const __g
             for (int k = 0; k < kMaxChunks; ++k)
                 if (k < nchunk16)
                     atomicAdd(P.stats + (lane >> 4) * P.cout + cur_slice * P.nb + k * 16 + (lane & 15), (double)run[k]);
-        }
-        if (fuse_br) {
-            if (cur_slice >= 0) {
-#pragma unroll
-                for (int k = 0; k < kMaxChunks; ++k)
-                    if (k < nchunk16) epi_bwdred_flush(P.br, P.cout, cur_slice * P.nb + k * 16, run[k], lane);
-            }
-            br_dsl = warp_sum(br_dsl);
-            if (lane == 0 && br_dsl != 0.0f) atomicAdd(P.br.red + 2 * P.cout, (double)br_dsl);
         }
     }
     tc_fence_before();
@@ -489,7 +453,7 @@ bool make_df_cfg(int cin, int cout, int d, DfCfg& c, int taps = 9, int cin_a = 0
     c.pb = g_df_pb > 0 ? g_df_pb : (c.a_bytes <= 2 * kPlaneBytes ? 3 : 2);      // measured: tools/dfold_knob_probe.py pb
     // (ONE commit per box -- the producer waiting on the epilogue's plane barriers instead of its own empty barriers --
     //  was measured SLOWER for the Cin 16 layers: 16 -> 16 41.5 -> 46.3 us, pb 1: 47.0 -> 55.7 us; kept two barriers)
-    const int fixed = c.b_bytes + 1024 + 512 + 4 * cout * (int)sizeof(float) + 16;
+    const int fixed = c.b_bytes + 1024 + 512 + 2 * cout * (int)sizeof(float) + 16;
     c.stages = 0;
     for (int s = c.pb == 1 ? 6 : 4; s >= 2 && c.stages == 0; --s)
         if (fixed + s * c.pb * c.a_bytes <= 110 * 1024) c.stages = s;
@@ -613,7 +577,7 @@ extern "C" int fpl_conv3d_dfold_prep_weight_batch(int count, const float* const*
 
 static int dfold_launch(const void* x, int x_c8tot, int x_c8off, const void* image, const float* bias, void* y,
                         int y_c8tot, int y_c8off, double* stats, int n, int d, int h, int w, int cin, int cout, int taps,
-                        int cin_a, void* stream, const EpiAct* act = nullptr, const EpiBwdRed* br = nullptr) {
+                        int cin_a, void* stream, const EpiAct* act = nullptr) {
     if (cin_a <= 0) cin_a = cin;
     DfCfg c;
     FPL_REQUIRE(make_df_cfg(cin, cout, d, c, taps, cin_a), "fpl_conv3d_tc_dfold: unsupported shape (%d -> %d, depth %d)", cin, cout, d);
@@ -655,7 +619,6 @@ static int dfold_launch(const void* x, int x_c8tot, int x_c8off, const void* ima
     P.total_items = P.full_items + 2 * ((int)total - P.full_items);
     P.taps = taps; P.a_ksteps = cin_a / 16;
     P.dbg_epi = g_df_epi; P.dbg_nomma = g_df_nomma; P.dbg_tma = g_df_tma; P.dbg_trace = g_df_trace;
-    if (br != nullptr) P.br = *br; else { P.br.y = nullptr; P.br.scale = P.br.shift = P.br.mean = P.br.invstd = P.br.slope = nullptr; P.br.drop_p = 0.0f; P.br.seed = P.br.offset = 0; P.br.seed_dev = nullptr; P.br.red = nullptr; }
     if (act != nullptr) P.act = *act; else { P.act.scale = nullptr; P.act.shift = nullptr; P.act.slope = nullptr; P.act.drop_p = 0.0f; P.act.seed = P.act.offset = 0; P.act.seed_dev = nullptr; }
     if (c.nb == 16) {
         FPL_CHECK_CUDA(cudaFuncSetAttribute(conv3d_tc_dfold_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, c.smem_bytes));
@@ -706,21 +669,3 @@ extern "C" int fpl_conv3d_tc_k311_act(const void* x, int x_c8tot, int x_c8off, c
     return dfold_launch(x, x_c8tot, x_c8off, image, nullptr, a, a_c8tot, a_c8off, nullptr, n, d, h, w, cin, cout, 1, a_channels,
                         stream, &act);
 }
-
-/* dgrad form of fpl_conv3d_tc_dfold that also accumulates the BatchNorm-backward sums of the unit whose activation
- * gradient it writes (fpl_conv3d_tc_bwdred, EpiBwdRed in common.cuh). */
-extern "C" int fpl_conv3d_tc_dfold_bwdred(const void* x, int x_c8tot, int x_c8off, const void* image, void* y, int y_c8tot,
-                                          int y_c8off, int n, int d, int h, int w, int cin, int cout, const void* y_prev,
-                                          const float* scale, const float* shift, const float* mean, const float* invstd,
-                                          const float* slope, float drop_p, uint64_t seed, uint64_t offset,
-                                          const uint64_t* seed_dev, double* red, void* stream) {
-    FPL_REQUIRE(y_prev != nullptr && scale != nullptr && shift != nullptr && mean != nullptr && invstd != nullptr &&
-                slope != nullptr && red != nullptr, "fpl_conv3d_tc_dfold_bwdred: NULL argument");
-    FPL_REQUIRE(drop_p >= 0.0f && drop_p < 1.0f, "fpl_conv3d_tc_dfold_bwdred: dropout p=%f out of [0,1)", drop_p);
-    EpiBwdRed br;
-    br.y = (const bf16x8*)y_prev; br.scale = scale; br.shift = shift; br.mean = mean; br.invstd = invstd; br.slope = slope;
-    br.drop_p = drop_p; br.seed = seed; br.offset = offset; br.seed_dev = (const unsigned long long*)seed_dev; br.red = red;
-    return dfold_launch(x, x_c8tot, x_c8off, image, nullptr, y, y_c8tot, y_c8off, nullptr, n, d, h, w, cin, cout, 9, 0, stream,
-                        nullptr, &br);
-}
-

@@ -100,9 +100,9 @@ class Inferer(object):
             accs1, cnt1 = [torch.zeros_like(acc) for _ in range(K)], torch.zeros_like(cnt)
             # stale weight images are re-staged HERE, on the main stream, before the side stream forks: lane 0 would
             # otherwise stage them lazily after the fork and lane 1 could read half-written images
-            prepare = getattr(self.model, "prepare_inference", None)
+            prepare = getattr(self.model, "prepare", None)
             if prepare is not None:
-                prepare((b,) + tuple(image.shape[1:2]) + tuple(win))
+                prepare((b,) + tuple(image.shape[1:2]) + tuple(win), grad=False)
             self._side.wait_stream(main)
             group = max(1, group // 2)
         lane = 0

@@ -80,8 +80,6 @@ _SIGNATURES = {
     "fpl_dsbn_act_bwd_apply": (_I, [_P, _P, _I, _I, _P, _I, _I, _P, _I, _P, _P, _P, _P, _P, _F, _P, _U, _U, _P, _P, _I, _P]
                                + [_I] * 5 + [_P]),
     "fpl_dsbn_bwd_finalize": (_I, [_P, _P, _P, _I, _P, _P, _P, _P, _I, _P]),
-    "fpl_conv3d_tc_bwdred": (_I, [_P, _I, _I, _P, _P, _I, _I] + [_I] * 7 + [_P, _P, _P, _P, _P, _P, _F, _U, _U, _P, _P, _P]),
-    "fpl_conv3d_tc_dfold_bwdred": (_I, [_P, _I, _I, _P, _P, _I, _I] + [_I] * 6 + [_P, _P, _P, _P, _P, _P, _F, _U, _U, _P, _P, _P]),
     "fpl_gather_patches": (_I, [_P, _I, _I, _I, _I, _I, _P, _P, _P, _P]),
     "fpl_adam_multi_tensor": (_I, [_P, _I, _P, _I, _P, c_double, c_double, c_double, c_double, c_double, _P, _P]),
     "fpl_adam_chunk_elems": (_I, []),

@@ -125,8 +125,15 @@ class _Lease(object):
             pass
 
 
-def _conv_impl():
-    return os.environ.get("FPL_CONV_IMPL", "tc")
+class _Plan(object):
+    """The kernel of every launch site of one pass (UNet2D5_dsbn._plan) and the weight images they read."""
+
+    def __init__(self):
+        self.fwd, self.dgrad, self.wgrad = {}, {}, {}   # conv unit name -> kernel
+        self.head = None                                # "cc" (csrc/head.cu), "tc" (zero-padded), "direct"
+        self.up = []                                    # up1..up4: "proj" (bilinear), "tc" / "direct" (transposed conv)
+        self.images = []                                # (kind, conv, transpose or convT mode, kd): prepare() stages them
+        self.eval_fuse = False                          # conv + eval-mode BatchNorm + PReLU in one kernel (EpiAct)
 
 
 class UNet2D5_dsbn(nn.Module):
@@ -168,10 +175,13 @@ class UNet2D5_dsbn(nn.Module):
         self._graph_ws_keep = []        # workspaces baked into captured graphs: never recycled
         self._infer_wss = {}            # eager no-grad workspaces per graph lane
         self.cuda_graphs = os.environ.get("FPL_CUDA_GRAPH", "1") != "0"
-        self.wgrad_side_stream = os.environ.get("FPL_WGRAD_STREAM", "0") != "0"   # measured: no gain on top of the dual-domain streams
-        self._aux_streams = {}
-        self._dfold_cache = {}
-        self._unit_depth = {}
+        # the reference paths tests compare against: "direct" = CUDA-core convolutions, the two-kernel inference
+        # epilogue, gradients handed back to autograd
+        self.conv_impl = os.environ.get("FPL_CONV_IMPL", "tc")
+        self.eval_fuse = os.environ.get("FPL_EVAL_FUSE", "1") != "0"
+        self.grad_direct = os.environ.get("FPL_GRAD_DIRECT", "1") != "0"
+        self.wgrad_side_stream = False  # callers save / restore it; weight gradients run on the stream of their pass
+        self._plans = {}
         self.grad_ready_hook = None     # callable(flat_grad, start, end, last) fired as buckets complete (DDP)
         self.grad_wait_hook = None      # callable() that makes the current stream wait for those all-reduces
         self.grad_bucket_bytes = 4 << 20
@@ -179,15 +189,12 @@ class UNet2D5_dsbn(nn.Module):
         self._master = None             # persistent flat gradient buffer (see _deliver_grads)
         self._head = UNet2D5_dsbn._HeadConv(self.out_conv)
         self._stem = None
-        self._head_unit = None
         self._head_dirty = True
         self._stem_dirty = True
-        self._geo0 = (0, 0, 0)
-        self._grad_pass = False         # inside _UNetFunction.forward (autograd disables grad mode there)
-        self._build_plan()
+        self._build_units()
 
-    # -- plan -------------------------------------------------------------------------------
-    def _build_plan(self):
+    # -- units ------------------------------------------------------------------------------
+    def _build_units(self):
         for c in self.ft_chns:
             if c % 8 != 0:
                 raise ValueError("feature_chns must be multiples of 8, got {0:}".format(self.ft_chns))
@@ -288,31 +295,6 @@ class UNet2D5_dsbn(nn.Module):
                 call("fpl_conv3d_k311_prep_weight", ptr(self.weight), 48, co, ptr(self.image), stream_ptr())
                 self.seen = w._version
 
-    def _stem_tc(self, depth):
-        u = self._down_units[0][0]
-        return (u.cin == 1 and u.kd == 3 and depth >= 2 and u.cout in (16, 32, 64) and ops.is_sm100()
-                and _conv_impl() == "tc" and os.environ.get("FPL_STEM_IMPL", "tc") == "tc")
-
-    def _stem_direct(self, geo):
-        """Training step: the stem forward / weight gradient straight from the fp32 image (csrc/stem_tc.cu: the 27-tap
-        operand is built in shared memory from a rolling window of image planes) instead of patch tensor + k(3,1,1)
-        kernels: 41 + 35 us against 81 + 40 us per launch pair at 4x32x128x128, no 134 MB patch tensor kept until
-        backward; same-box A/B of the step 4.348 -> 4.283 ms.  FPL_STEM_TRAIN=patch restores the patch-tensor path
-        (which no-grad forwards keep: its conv carries the activation in the epilogue)."""
-        u = self._down_units[0][0]
-        d, h, w = geo
-        return (u.cin == 1 and u.kd == 3 and u.cout == 16 and w >= 32 and h >= 4 and ops.is_sm100()
-                and _conv_impl() == "tc" and os.environ.get("FPL_STEM_TRAIN", "direct") == "direct")
-
-    def _head_cc(self, n, d):
-        """CUDA-core head kernels (csrc/head.cu): the default for the shipped shapes; FPL_HEAD_IMPL=tc selects the
-        zero-padded tensor-core path."""
-        return (self.ft_chns[0] in (16, 32) and self.n_class <= 8 and d >= 2 and n * d <= 65535 and ops.is_sm100()
-                and os.environ.get("FPL_HEAD_IMPL", "cc") == "cc" and os.environ.get("FPL_CONV_IMPL", "tc") == "tc")
-
-    def _head_tc(self):
-        return self._use_tc(self.ft_chns[0], 16) and self.n_class <= 8 and os.environ.get("FPL_HEAD_IMPL", "tc") == "tc"
-
     def _grad_params(self, domain):
         """Parameters that receive gradients, in the order backward completes them."""
         out = [self.out_conv.weight, self.out_conv.bias]
@@ -357,8 +339,6 @@ class UNet2D5_dsbn(nn.Module):
             raise ValueError('expected 5D input (got {}D input)'.format(x.dim()))
         if not x.is_cuda:
             raise RuntimeError("fplplus_b200.UNet2D5_dsbn runs on CUDA (sm_100a) only; got a %s tensor" % x.device)
-        if self.bilinear and not all(self._use_tc(u.cin, u.cout) for u in self._proj_units):
-            raise NotImplementedError("bilinear=True needs feature_chns that are multiples of 16 (tensor-core 1x1 projection)")
         domain = int(domain_label[0])
         if not 0 <= domain < self.num_domains:
             raise IndexError("domain_label %d out of range" % domain)
@@ -415,8 +395,7 @@ class UNet2D5_dsbn(nn.Module):
             logits, _ = self._run_forward(x, domain, ws, repeats)
             return logits
         rng = self.ensure_rng(x.device, lane)
-        self._note_depths(self._geometry(x.shape))
-        self._refresh_weight_images(with_dgrad=False)      # eager: a captured graph never restages weights
+        self.prepare(x.shape)                               # eager: a captured graph never restages weights
         if ent["graph"] is None:
             if len(self._graphs) > 24:                     # bound the memory held by stale shapes
                 for k in [k for k in self._graphs if k != key][:8]:
@@ -457,9 +436,6 @@ class UNet2D5_dsbn(nn.Module):
             geo.append((d // kd, h // 2, w // 2))
         return geo
 
-    def _use_tc(self, cin, cout):
-        return _conv_impl() == "tc" and cin % 16 == 0 and cout % 16 == 0 and ops.is_sm100()
-
     def invalidate_weight_images(self):
         """Forget the staged bf16 weight images.  They are keyed on ``weight._version``, which every
         ordinary in-place update bumps (torch.optim's default implementations, ``load_state_dict``);
@@ -470,185 +446,172 @@ class UNet2D5_dsbn(nn.Module):
         self._head_dirty = True
         self._stem_dirty = True
 
-    def prepare_inference(self, shape):
-        """Stage every stale weight image for no-grad forwards of inputs shaped ``shape`` [N,C,D,H,W] on the CURRENT
-        stream.  Callers that fan no-grad forwards out over several streams (Inferer's two lanes) call this before
-        the fork, so no lane stages lazily while another reads the images."""
-        self._note_depths(self._geometry(tuple(shape)))
-        self._refresh_weight_images(with_dgrad=False)
+    # -- kernel plan ------------------------------------------------------------------------
+    def _plan(self, n, geo, grad, sm100):
+        """The kernel of every launch site of a forward (``grad``: and its backward) over ``n`` inputs with the level
+        geometries ``geo`` (see _geometry), and the weight images those kernels read.  It depends on nothing else but
+        the construction parameters and the library's image-size queries (no device work), so it is memoised."""
+        key = (n, tuple(geo), bool(grad), bool(sm100))
+        plan = self._plans.get(key)
+        if plan is None:
+            plan = self._plans[key] = self._make_plan(n, geo, grad, sm100)
+        return plan
 
-    def _tc_convs(self):
-        out = []
-        for u1, u2 in self._down_units + self._up_units:
-            for u in (u1, u2):
-                if not u.is_stem and self._use_tc(u.cin, u.cout):
-                    out.append(u)
-        for u in self._proj_units:
-            u.conv.sync(self._head_dirty)
-            out.append(u)
-        if self._head_tc():
-            if self._head_unit is None:
-                self._head_unit = _Unit("head", self._head, None, None, None, 1)
-            self._head.sync(self._head_dirty)
-            out.append(self._head_unit)
-        self._head_dirty = False
-        return out
-
-    def _refresh_weight_images(self, with_dgrad):
-        """(Re)stage every stale weight image with ONE batched launch."""
+    def _make_plan(self, n, geo, grad, sm100):
         lib = ops._lib.load()
-        if self._stem_tc(self._unit_depth.get("block0.conv#1", 0)) and not (with_dgrad and self._stem_direct(self._geo0)):
-            # the patch-tensor stem serves the no-grad forwards (activation in its epilogue); the training step builds
-            # the stem operand in shared memory and needs no staged image
-            if self._stem is None:
-                self._stem = UNet2D5_dsbn._StemConv(self._down_units[0][0].conv)
-            self._stem.sync(self._stem_dirty)
-            self._stem_dirty = False
-        todo, todo_df, todo_ct = [], [], []
-        for u in self._tc_convs():
-            w = u.conv.weight
-            depth = self._unit_depth.get(u.name, 0)
-            for transpose in ((False, True) if with_dgrad else (False,)):
-                if transpose and not self._use_tc(u.cout, u.cin):
-                    continue
-                if u.name != "head" and self._dfold_ok(u.cout if transpose else u.cin, u.cin if transpose else u.cout,
-                                                       u.kd, depth):
-                    if not (transpose and u.name == "block0.conv#1"):
-                        self._dfold_image(u.conv, transpose, todo_df)   # depth-folded kernel: its own image layout
-                    continue
-                key = (id(w), transpose)
-                ent = self._img_cache.get(key)
-                if ent is None or ent[1].device != w.device:
-                    nbytes = lib.fpl_conv3d_weight_image_bytes(u.cout if transpose else u.cin,
-                                                               u.cin if transpose else u.cout, u.kd)
-                    ent = self._img_cache[key] = [-1, torch.empty(nbytes // 2, dtype=torch.bfloat16, device=w.device)]
-                if ent[0] != w._version:
-                    todo.append((w, u.cin, u.cout, u.kd, 1 if transpose else 0, ent))
-        if os.environ.get("FPL_CONVT_IMPL", "tc") == "tc":
-            for up in (self.up1, self.up2, self.up3, self.up4):
-                trans = up.trans3d if up.dim == 3 else up.trans2d
-                if self._use_tc(trans.weight.shape[0], trans.weight.shape[1]):
-                    kd2 = 2 if up.dim == 3 else 1
-                    self._convt_image(trans, kd2, 0, todo_ct)
-                    if with_dgrad:
-                        self._convt_image(trans, kd2, 1, todo_ct)
-        for i in range(0, len(todo_df), 64):
-            part = todo_df[i:i + 64]
-            n = len(part)
-            arr_w = (ctypes.c_void_p * n)(*[t[0].data_ptr() for t in part])
-            arr_img = (ctypes.c_void_p * n)(*[t[4][1].data_ptr() for t in part])
-            ints = [(ctypes.c_int * n)(*[t[k] for t in part]) for k in (1, 2, 3)]
-            call("fpl_conv3d_dfold_prep_weight_batch", n, arr_w, ints[0], ints[1], ints[2], arr_img, stream_ptr())
-            for t in part:
-                t[4][0] = t[0]._version
-        if todo_ct:
-            n = len(todo_ct)
-            arr_w = (ctypes.c_void_p * n)(*[t[0].data_ptr() for t in todo_ct])
-            arr_img = (ctypes.c_void_p * n)(*[t[5][1].data_ptr() for t in todo_ct])
-            ints = [(ctypes.c_int * n)(*[t[k] for t in todo_ct]) for k in (1, 2, 3, 4)]
-            call("fpl_convt_prep_weight_batch", n, arr_w, ints[0], ints[1], ints[2], ints[3], arr_img, stream_ptr())
-            for t in todo_ct:
-                t[5][0] = t[0]._version
-        for i in range(0, len(todo), 80):
-            part = todo[i:i + 80]
-            n = len(part)
-            arr_w = (ctypes.c_void_p * n)(*[t[0].data_ptr() for t in part])
-            arr_img = (ctypes.c_void_p * n)(*[t[5][1].data_ptr() for t in part])
-            ints = [(ctypes.c_int * n)(*[t[k] for t in part]) for k in (1, 2, 3, 4)]
-            call("fpl_conv3d_prep_weight_batch", n, arr_w, ints[0], ints[1], ints[2], ints[3], arr_img, stream_ptr())
-            for t in part:
-                t[5][0] = t[0]._version
+        impl_tc = self.conv_impl == "tc" and sm100
+        ft, k_cls = self.ft_chns, self.n_class
 
-    def _note_depths(self, geo):
-        """Depth of every conv unit for the current input geometry (kernel selection of the weight staging)."""
-        self._geo0 = tuple(geo[0])
-        for i in range(5):
-            for u in self._down_units[i]:
-                self._unit_depth[u.name] = geo[i][0]
-        for k, lvl in zip(range(4), (3, 2, 1, 0)):
-            for u in self._up_units[k]:
-                self._unit_depth[u.name] = geo[lvl][0]
+        def tc(cin, cout):
+            return impl_tc and cin % 16 == 0 and cout % 16 == 0
 
-    def _dfold_ok(self, cin, cout, kd, depth):
-        """Depth-folded tensor-core kernel (csrc/conv_tc_dfold.cu) for the small-channel k3 layers."""
-        if kd != 3 or depth < 2 or not self._use_tc(cin, cout) or os.environ.get("FPL_DFOLD", "1") == "0":
-            return False
-        key = (cin, cout)
-        ok = self._dfold_cache.get(key)
-        if ok is None:
-            ok = self._dfold_cache[key] = ops._lib.load().fpl_conv3d_dfold_image_bytes(cin, cout) > 0
-        return ok
+        def conv(cin, cout, kd, depth):
+            if not tc(cin, cout):
+                return "direct"
+            # depth-folded tensor-core kernel (csrc/conv_tc_dfold.cu) for the small-channel k3 layers
+            if kd == 3 and depth >= 2 and lib.fpl_conv3d_dfold_image_bytes(cin, cout) > 0:
+                return "dfold"
+            return "tc"
 
-    def _dfold_image(self, conv, transpose, defer=None):
-        w = conv.weight
-        key = (id(w), "df%d" % (1 if transpose else 0))
-        ent = self._img_cache.get(key)
-        cin, cout = conv.in_channels, conv.out_channels
-        if ent is None or ent[1].device != w.device:
-            nbytes = ops._lib.load().fpl_conv3d_dfold_image_bytes(cout if transpose else cin, cin if transpose else cout)
-            ent = self._img_cache[key] = [-1, torch.empty(nbytes // 2, dtype=torch.bfloat16, device=w.device)]
-        if ent[0] != w._version:
-            if defer is not None:
-                defer.append((w, cin, cout, 1 if transpose else 0, ent))
-            else:
-                call("fpl_conv3d_dfold_prep_weight", ptr(w), cin, cout, 1 if transpose else 0, ptr(ent[1]), stream_ptr())
-                ent[0] = w._version
-        return ent[1]
+        plan = _Plan()
+        plan.eval_fuse = self.eval_fuse and sm100
+        # the 1-channel stem.  Training: "stem_direct" builds the 27-tap operand from the fp32 image in shared memory
+        # (csrc/stem_tc.cu; 41 + 35 us against 81 + 40 us per forward + wgrad at 4x32x128x128, and no 134 MB patch
+        # tensor kept until backward).  No-grad forwards keep "stem_patch" (fpl_patch9_c8 + a k(3,1,1) conv) whose
+        # conv carries the activation in its epilogue.  "stem_cc": fpl_stem_conv_fwd for the other shapes.
+        stem = self._down_units[0][0]
+        d0, h0, w0 = geo[0]
+        stem_tc = impl_tc and stem.cin == 1 and stem.kd == 3
+        if grad and stem_tc and stem.cout == 16 and w0 >= 32 and h0 >= 4:
+            plan.fwd[stem.name] = "stem_direct"
+        elif stem_tc and d0 >= 2 and stem.cout in (16, 32, 64):
+            plan.fwd[stem.name] = "stem_patch"
+            plan.images.append(("stem", stem.conv, 0, 3))
+        else:
+            plan.fwd[stem.name] = "stem_cc"
+        if grad:
+            wg = plan.fwd[stem.name]
+            if wg == "stem_cc" and tc(16, stem.cout) and stem.cin <= 8:
+                wg = "stem_c8"          # the image packed into one zero-padded channel group, tensor-core wgrad
+            plan.wgrad[stem.name] = wg
+        units = [(u, geo[i][0]) for i in range(5) for u in self._down_units[i] if not u.is_stem]
+        units += [(u, geo[3 - k][0]) for k in range(4) for u in self._up_units[k]]
+        for u, depth in units:
+            kern = plan.fwd[u.name] = conv(u.cin, u.cout, u.kd, depth)
+            if kern != "direct":
+                plan.images.append((kern, u.conv, 0, u.kd))
+            if grad:
+                kern = plan.dgrad[u.name] = conv(u.cout, u.cin, u.kd, depth)
+                if kern != "direct":
+                    plan.images.append((kern, u.conv, 1, u.kd))
+                plan.wgrad[u.name] = "tapmajor" if sm100 and u.cin % 8 == 0 and u.cout % 16 == 0 else "direct"
+        for k in range(4):
+            c, c_low = ft[3 - k], ft[4 - k]
+            if not self.bilinear:
+                plan.up.append("tc" if tc(c_low, c) else "direct")
+                continue
+            if not tc(c_low, c):
+                raise NotImplementedError("bilinear=True needs feature_chns that are multiples of 16 (tensor-core 1x1 "
+                                          "projection)")
+            plan.up.append("proj")
+            pu = self._proj_units[k]
+            plan.images += [("tc", pu.conv, t, 1) for t in ((0, 1) if grad else (0,))]
+        if impl_tc and ft[0] in (16, 32) and k_cls <= 8 and d0 >= 2 and n * d0 <= 65535:
+            plan.head = "cc"
+        elif tc(ft[0], 16) and k_cls <= 8:
+            plan.head = "tc"
+        else:
+            plan.head = "direct"
+        # the images of the zero-padded head and of the tensor-core transposed convs are staged wherever those kernels
+        # could run, also when this plan picks head.cu or bilinear up-sampling: unread there, but they only add
+        # entries to the batched staging launches
+        if tc(ft[0], 16) and k_cls <= 8:
+            plan.images += [("tc", self._head, t, 1) for t in ((0, 1) if grad else (0,))]
+        for up in (self.up1, self.up2, self.up3, self.up4):
+            trans = up.trans3d if up.dim == 3 else up.trans2d
+            if tc(trans.in_channels, trans.out_channels):
+                plan.images += [("convt", trans, t, 2 if up.dim == 3 else 1) for t in ((0, 1) if grad else (0,))]
+        return plan
 
-    def _convt_tc(self, cin, cout):
-        return (self._use_tc(cin, cout) and os.environ.get("FPL_CONVT_IMPL", "tc") == "tc")
+    def prepare(self, shape, grad=False):
+        """Stage every stale weight image that a forward (``grad``: and its backward) over inputs shaped ``shape``
+        [N,C,D,H,W] reads, on the CURRENT stream, in batched launches; returns the pass's kernel plan.  Callers that fan
+        passes out over several streams (the agent's two domain passes, the Inferer's two lanes) call this before the
+        fork, so that no stream stages images while another reads them."""
+        plan = self._plan(shape[0], self._geometry(tuple(shape)), grad, ops.is_sm100())
+        lib = ops._lib.load()
+        todo = {"dfold": [], "convt": [], "tc": []}
+        synced = set()
+        for kind, conv, t, kd in plan.images:
+            if kind == "stem":
+                if self._stem is None:
+                    self._stem = UNet2D5_dsbn._StemConv(conv)
+                self._stem.sync(self._stem_dirty)
+                self._stem_dirty = False
+                continue
+            if hasattr(conv, "sync") and id(conv) not in synced:      # the padded head, the bilinear projections
+                conv.sync(self._head_dirty)
+                synced.add(id(conv))
+            w = conv.weight
+            key = (id(w), kind, t)
+            ent = self._img_cache.get(key)
+            if ent is None or ent[1].device != w.device:
+                cin, cout = conv.in_channels, conv.out_channels
+                if kind == "dfold":
+                    nbytes = lib.fpl_conv3d_dfold_image_bytes(cout if t else cin, cin if t else cout)
+                elif kind == "convt":
+                    nbytes = lib.fpl_convt_weight_image_bytes(cin, cout, kd)
+                else:
+                    nbytes = lib.fpl_conv3d_weight_image_bytes(cout if t else cin, cin if t else cout, kd)
+                ent = self._img_cache[key] = [-1, torch.empty(nbytes // 2, dtype=torch.bfloat16, device=w.device)]
+            if ent[0] != w._version:
+                todo[kind].append((w, conv.in_channels, conv.out_channels, kd, t, ent))
+        self._head_dirty = False
+        for kind, fn, cols, batch in (("dfold", "fpl_conv3d_dfold_prep_weight_batch", (1, 2, 4), 64),
+                                      ("convt", "fpl_convt_prep_weight_batch", (1, 2, 3, 4), 16),
+                                      ("tc", "fpl_conv3d_prep_weight_batch", (1, 2, 3, 4), 80)):
+            for i in range(0, len(todo[kind]), batch):
+                part = todo[kind][i:i + batch]
+                m = len(part)
+                arr_w = (ctypes.c_void_p * m)(*[e[0].data_ptr() for e in part])
+                arr_img = (ctypes.c_void_p * m)(*[e[5][1].data_ptr() for e in part])
+                ints = [(ctypes.c_int * m)(*[e[c] for e in part]) for c in cols]
+                call(fn, m, arr_w, *ints, arr_img, stream_ptr())
+                for e in part:
+                    e[5][0] = e[0]._version
+        return plan
 
-    def _convt_image(self, trans, kd2, mode, defer=None):
-        """Staged bf16 GEMM operand of a transposed conv (mode 0 forward, 1 dgrad), cached on the weight version."""
-        w = trans.weight
-        key = (id(w), "ct%d" % mode)
-        ent = self._img_cache.get(key)
-        if ent is None or ent[1].device != w.device:
-            nbytes = ops._lib.load().fpl_convt_weight_image_bytes(w.shape[0], w.shape[1], kd2)
-            ent = self._img_cache[key] = [-1, torch.empty(nbytes // 2, dtype=torch.bfloat16, device=w.device)]
-        if ent[0] != w._version:
-            if defer is not None:
-                defer.append((w, w.shape[0], w.shape[1], kd2, mode, ent))
-            else:
-                call("fpl_convt_prep_weight", ptr(w), w.shape[0], w.shape[1], kd2, mode, ptr(ent[1]), stream_ptr())
-                ent[0] = w._version
-        return ent[1]
+    def _image(self, kind, conv, transpose=0):
+        """A weight image staged by prepare() ("tc" / "dfold": transpose 1 = dgrad; "convt": mode 1 = dgrad)."""
+        return self._img_cache[(id(conv.weight), kind, transpose)][1]
 
-    def _weight_image(self, conv, kd, transpose, ws):
-        ent = self._img_cache.get((id(conv.weight), transpose))
-        if ent is None or ent[0] != conv.weight._version:
-            self._refresh_weight_images(with_dgrad=transpose)
-            ent = self._img_cache[(id(conv.weight), transpose)]
-        return ent[1]
-
-    def _conv_fwd(self, u, xin, x_img, y, stats, n, geo, ws):
+    def _conv_fwd(self, u, kern, xin, x_img, y, stats, n, geo, ws):
         d, h, w = geo
         st = stream_ptr()
-        if u.is_stem and self._stem_tc(d) and not (self._grad_pass and self._stem_direct(geo)):
+        if kern == "stem_patch":
             xs = ws.c8("XS:stem", n, d, 32, h, w)
             call("fpl_patch9_c8", ptr(x_img), ptr(xs), 1, n, d, h, w, st)
             call("fpl_conv3d_tc_k311", ptr(xs), 4, 0, ptr(self._stem.image), ptr(u.conv.bias), ptr(y), y.shape[2], 0,
                  ptr(stats), n, d, h, w, 48, u.cout, 32, st)
-        elif u.is_stem:
+        elif kern in ("stem_direct", "stem_cc"):
             call("fpl_stem_conv_fwd", ptr(x_img), ptr(u.conv.weight), ptr(u.conv.bias), ptr(y), y.shape[2], 0,
                  ptr(stats), n, u.cin, d, h, w, u.cout, u.kd, st)
-        elif self._dfold_ok(u.cin, u.cout, u.kd, d):
-            call("fpl_conv3d_tc_dfold", *xin.args(), ptr(self._dfold_image(u.conv, False)), ptr(u.conv.bias), ptr(y),
+        elif kern == "dfold":
+            call("fpl_conv3d_tc_dfold", *xin.args(), ptr(self._image("dfold", u.conv)), ptr(u.conv.bias), ptr(y),
                  y.shape[2], 0, ptr(stats), n, d, h, w, u.cin, u.cout, st)
-        elif self._use_tc(u.cin, u.cout):
-            img = self._weight_image(u.conv, u.kd, False, ws)
-            call("fpl_conv3d_tc", *xin.args(), ptr(img), ptr(u.conv.bias), ptr(y), y.shape[2], 0, ptr(stats),
-                 n, d, h, w, u.cin, u.cout, u.kd, st)
+        elif kern == "tc":
+            call("fpl_conv3d_tc", *xin.args(), ptr(self._image("tc", u.conv)), ptr(u.conv.bias), ptr(y), y.shape[2], 0,
+                 ptr(stats), n, d, h, w, u.cin, u.cout, u.kd, st)
         else:
             call("fpl_conv3d_direct", *xin.args(), ptr(u.conv.weight), ptr(u.conv.bias), ptr(y), y.shape[2], 0,
                  ptr(stats), n, d, h, w, u.cin, u.cout, u.kd, 0, 0, st)
 
-    def _eval_affine_refresh(self, domain, ws):
+    def _eval_affine_refresh(self, domain, ws, plan):
         """Inference epilogue (csrc/common.cuh EpiAct): scale / shift of every conv unit whose BatchNorm is in eval mode,
         from the CURRENT running statistics, in one launch at the start of a no-grad forward (part of the captured
         graph, so replays follow the running statistics).  Returns {unit name: (scale, shift)}."""
         units = [u for pair in self._down_units + self._up_units for u in pair if not u.dsbn.bns[domain].training]
-        if not units or os.environ.get("FPL_EVAL_FUSE", "1") == "0" or not ops.is_sm100():
+        if not units or not plan.eval_fuse:
             return {}
         key = "eval_affine:%d" % domain
         total = sum(2 * u.cout for u in units)
@@ -666,30 +629,30 @@ class UNet2D5_dsbn(nn.Module):
              (ctypes.c_int * m)(*[u.cout for u in units]), float(bns[0].eps), stream_ptr())
         return out
 
-    def _unit_fwd_fused(self, u, xin, x_img, out, aff, p, seed, offset, seed_dev, n, geo, ws):
+    def _unit_fwd_fused(self, u, kern, xin, x_img, out, aff, p, seed, offset, seed_dev, n, geo, ws):
         """Inference: conv with the eval-mode BatchNorm + PReLU (+ dropout) in its epilogue; writes the activation into
         ``out``.  Returns False when no fused kernel serves this unit (the caller runs the two-kernel path)."""
         d, h, w = geo
         st = stream_ptr()
         scale, shift = aff
-        if u.is_stem:
-            if not self._stem_tc(d) or p > 0.0:
+        if kern == "stem_patch":
+            if p > 0.0:
                 return False
             xs = ws.c8("XS:stem", n, d, 32, h, w)
             call("fpl_patch9_c8", ptr(x_img), ptr(xs), 1, n, d, h, w, st)
             call("fpl_conv3d_tc_k311_act", ptr(xs), 4, 0, ptr(self._stem.image), *out.args(), n, d, h, w, 48, u.cout, 32,
                  ptr(scale), ptr(shift), ptr(u.prelu.weight), st)
             return True
-        if self._dfold_ok(u.cin, u.cout, u.kd, d):
+        if kern == "dfold":
             if p > 0.0:
                 return False
-            call("fpl_conv3d_tc_dfold_act", *xin.args(), ptr(self._dfold_image(u.conv, False)), *out.args(), n, d, h, w,
+            call("fpl_conv3d_tc_dfold_act", *xin.args(), ptr(self._image("dfold", u.conv)), *out.args(), n, d, h, w,
                  u.cin, u.cout, ptr(scale), ptr(shift), ptr(u.prelu.weight), st)
             return True
-        if self._use_tc(u.cin, u.cout):
-            img = self._weight_image(u.conv, u.kd, False, ws)
-            call("fpl_conv3d_tc_act", *xin.args(), ptr(img), *out.args(), n, d, h, w, u.cin, u.cout, u.kd, ptr(scale),
-                 ptr(shift), ptr(u.prelu.weight), p, seed, offset, ptr(seed_dev) if p > 0.0 else None, st)
+        if kern == "tc":
+            call("fpl_conv3d_tc_act", *xin.args(), ptr(self._image("tc", u.conv)), *out.args(), n, d, h, w, u.cin,
+                 u.cout, u.kd, ptr(scale), ptr(shift), ptr(u.prelu.weight), p, seed, offset,
+                 ptr(seed_dev) if p > 0.0 else None, st)
             return True
         return False
 
@@ -697,6 +660,7 @@ class UNet2D5_dsbn(nn.Module):
         """conv -> finalize -> act.  ``out``/``pooled`` are C8 views."""
         d, h, w = geo
         c = u.cout
+        kern = rec["plan"].fwd[u.name]
         aff = rec["eval_affine"].get(u.name)
         if aff is not None:
             # no-grad forward, BatchNorm in eval mode: one kernel instead of two (dropout keeps the same Philox stream
@@ -707,7 +671,7 @@ class UNet2D5_dsbn(nn.Module):
             if not explicit:
                 if drop:
                     p, seed, offset = float(u.dropout.p), rec["seed"], rec["next_offset"]
-                if self._unit_fwd_fused(u, xin, x_img, out, aff, p, seed, offset, rec["seed_dev"], n, geo, ws):
+                if self._unit_fwd_fused(u, kern, xin, x_img, out, aff, p, seed, offset, rec["seed_dev"], n, geo, ws):
                     if drop:
                         rec["next_offset"] += 2 * n * d * (c // 8) * h * w
                     if pooled is not None:
@@ -715,7 +679,7 @@ class UNet2D5_dsbn(nn.Module):
                     return
         y = ws.c8("Y:" + u.name, n, d, c, h, w)
         stats = small.f64(2 * c)
-        self._conv_fwd(u, xin, x_img, y, stats, n, geo, ws)
+        self._conv_fwd(u, kern, xin, x_img, y, stats, n, geo, ws)
         bn = u.dsbn.bns[domain]
         if bn.weight.dtype != torch.float32:
             raise RuntimeError("fplplus_b200 supports tensor_type=float only")
@@ -738,8 +702,7 @@ class UNet2D5_dsbn(nn.Module):
              n, d, h, w, c, stream_ptr())
         rec[u.name] = dict(y=y, xin=xin, scale=scale, shift=shift, mean=mean, invstd=invstd, training=training,
                            p=p, mask=mask, seed=seed, offset=offset, geo=geo, bn=bn,
-                           seed_dev=rec["seed_dev"] if p > 0.0 and mask is None else None,
-                           stem_direct=u.is_stem and self._grad_pass and self._stem_direct(geo))
+                           seed_dev=rec["seed_dev"] if p > 0.0 and mask is None else None)
 
     # -- whole-network forward --------------------------------------------------------------
     def _first_dropout_level(self):
@@ -751,24 +714,23 @@ class UNet2D5_dsbn(nn.Module):
                 return i
         return 5
 
-    def _run_forward(self, x, domain, ws, repeats=1):
-        """``repeats`` > 1 (no-grad only): K MC-dropout passes over the same input in one call -- the encoder levels in
-        front of the first active dropout run ONCE, the rest of the network K times with K dropout seeds; returns a
-        list of K logits tensors (bit-identical to K separate forwards drawing the same seeds)."""
+    def _run_forward(self, x, domain, ws, repeats=1, grad=False):
+        """``grad``: the forward of a training pass (its records feed _run_backward).  ``repeats`` > 1 (no-grad only):
+        K MC-dropout passes over the same input in one call -- the encoder levels in front of the first active dropout
+        run ONCE, the rest of the network K times with K dropout seeds; returns a list of K logits tensors
+        (bit-identical to K separate forwards drawing the same seeds)."""
         n = x.shape[0]
         geo = self._geometry(x.shape)
-        ft = self.ft_chns
         small = _SmallPool(ws, "fwd", x.device)
-        self._note_depths(geo)
-        self._refresh_weight_images(with_dgrad=self._grad_pass)
+        plan = self.prepare(x.shape, grad)
         # dropout stream: (seed, per-layer offset) drawn from torch's CPU generator, so torch.manual_seed
         # makes MC-dropout passes reproducible; backward regenerates the same Philox stream
         if self._seed_from_device:
             seed, seed_dev = 0, self.ensure_rng(x.device, self._cur_lane)
         else:
             seed, seed_dev = self._draw_seed(), None
-        rec = {"seed": seed, "seed_dev": seed_dev, "next_offset": 0, "geo": geo, "n": n, "x": x}
-        rec["eval_affine"] = {} if self._grad_pass else self._eval_affine_refresh(domain, ws)
+        rec = {"seed": seed, "seed_dev": seed_dev, "next_offset": 0, "geo": geo, "n": n, "x": x, "plan": plan}
+        rec["eval_affine"] = {} if grad else self._eval_affine_refresh(domain, ws, plan)
         if repeats > 1:
             assert not torch.is_grad_enabled()
             seeds = [(seed, seed_dev if seed_dev is None else seed_dev[0:1])]
@@ -826,17 +788,18 @@ class UNet2D5_dsbn(nn.Module):
             cat = ws.t["cat%d" % lvl]
             trans = up.trans3d if up.dim == 3 else up.trans2d
             kd2 = 2 if up.dim == 3 else 1
-            if self.bilinear:
+            kern = rec["plan"].up[k]
+            if kern == "proj":
                 # 1x1 projection at low resolution (a (1,3,3) conv with zero off-centre taps), then trilinear / bilinear
                 # x2 up-sampling (align_corners=True) straight into the second half of the concat buffer
                 pu = self._proj_units[k]
                 t_low = ws.c8("T:up%d" % (k + 1), n, dl, c, hl, wl)
-                call("fpl_conv3d_tc", *low.args(), ptr(self._weight_image(pu.conv, 1, False, ws)), ptr(pu.conv.bias), ptr(t_low),
+                call("fpl_conv3d_tc", *low.args(), ptr(self._image("tc", pu.conv)), ptr(pu.conv.bias), ptr(t_low),
                      c // 8, 0, None, n, dl, hl, wl, c_low, c, 1, stream_ptr())
                 call("fpl_upsample2x_c8", ptr(t_low), c // 8, 0, ptr(cat), 2 * c // 8, c // 8, n, dl, hl, wl, c, kd2,
                      stream_ptr())
-            elif self._convt_tc(c_low, c):
-                call("fpl_convt_k2s2_fwd_tc", *low.args(), ptr(self._convt_image(trans, kd2, 0)), ptr(trans.bias), ptr(cat),
+            elif kern == "tc":
+                call("fpl_convt_k2s2_fwd_tc", *low.args(), ptr(self._image("convt", trans)), ptr(trans.bias), ptr(cat),
                      2 * c // 8, c // 8, n, dl, hl, wl, c_low, c, kd2, stream_ptr())
             else:
                 call("fpl_convt_k2s2_fwd", *low.args(), ptr(trans.weight), ptr(trans.bias), ptr(cat), 2 * c // 8, c // 8,
@@ -849,13 +812,12 @@ class UNet2D5_dsbn(nn.Module):
             low = a2
         d, h, w = geo[0]
         logits = torch.empty((n, self.n_class, d, h, w), dtype=torch.float32, device=x.device)
-        if self._head_cc(n, d):
+        if rec["plan"].head == "cc":
             call("fpl_head_fwd", *low.args(), ptr(self.out_conv.weight), ptr(self.out_conv.bias), ptr(logits), n, d, h, w,
                  ft[0], self.n_class, stream_ptr())
-        elif self._head_tc():
-            img = self._weight_image(self._head, 1, False, ws)
-            call("fpl_head_conv_tc", *low.args(), ptr(img), ptr(self._head.bias), ptr(logits), n, d, h, w, ft[0],
-                 self.n_class, stream_ptr())
+        elif rec["plan"].head == "tc":
+            call("fpl_head_conv_tc", *low.args(), ptr(self._image("tc", self._head)), ptr(self._head.bias), ptr(logits),
+                 n, d, h, w, ft[0], self.n_class, stream_ptr())
         else:
             call("fpl_head_conv_fwd", *low.args(), ptr(self.out_conv.weight), ptr(self.out_conv.bias), ptr(logits),
                  n, d, h, w, ft[0], self.n_class, stream_ptr())
@@ -863,19 +825,8 @@ class UNet2D5_dsbn(nn.Module):
         return logits, rec
 
     # -- whole-network backward -------------------------------------------------------------
-    def _bwdred_ok(self, u_prev, r_prev):
-        """The BatchNorm-backward sums of ``u_prev`` can be accumulated by the epilogue of the dgrad that writes its
-        activation gradient (csrc/common.cuh EpiBwdRed): Philox dropout (no injected mask), tensor-core dgrad."""
-        # default OFF: measured (tools/epi_probe.py, profiles/README.md round 2) the 128 epilogue threads of a CTA pay more
-        # for the extra y_k loads and arithmetic (+23..+50 us on the full-resolution dfold layers, +2.5..3.5 us on the deep
-        # ones) than the standalone HBM-streaming reduce costs (30 / 3..5 us); FPL_BWD_FUSE=1 enables it for A/B runs
-        return (u_prev is not None and r_prev.get("mask") is None and os.environ.get("FPL_BWD_FUSE", "0") != "0"
-                and ops.is_sm100())
-
-    def _unit_bwd(self, u, r, g1, g_pool, pool_idx, pool_kd, n, ws, small, grads, need_dx, fold=None, prev=None):
-        """Backward of one conv unit.  Returns the C8 gradient wrt the unit's input (or None).
-        ``prev`` = (unit, record) of the unit whose activation is this unit's ONLY consumer-input (unit 1 of the same
-        ConvBlockND): its BatchNorm-backward reduce pass is then folded into this unit's dgrad epilogue."""
+    def _unit_bwd(self, u, r, g1, g_pool, pool_idx, pool_kd, n, ws, small, grads, need_dx, fold, plan):
+        """Backward of one conv unit.  Returns the C8 gradient wrt the unit's input (or None)."""
         d, h, w = r["geo"]
         c = u.cout
         st = stream_ptr()
@@ -883,19 +834,18 @@ class UNet2D5_dsbn(nn.Module):
         gpa = g_pool.args() if g_pool is not None else (None, 0, 0)
         common = (ptr(r["y"]), *g1a, *gpa, ptr(pool_idx), pool_kd, ptr(r["scale"]), ptr(r["shift"]), ptr(r["mean"]),
                   ptr(r["invstd"]), ptr(u.prelu.weight), r["p"], ptr(r["mask"]), r["seed"], r["offset"], ptr(r["seed_dev"]))
-        red = r.pop("red_fused", None)
-        if red is None:
-            red = small.f64(2 * c + 1)
-            call("fpl_dsbn_act_bwd_reduce", *common, ptr(red), n, d, h, w, c, st)
-        dy = ws.c8("dY:" + u.name, n, d, c, h, w)       # per unit: the side-stream wgrad may still be reading it
+        red = small.f64(2 * c + 1)
+        call("fpl_dsbn_act_bwd_reduce", *common, ptr(red), n, d, h, w, c, st)
+        dy = ws.c8("dY:" + u.name, n, d, c, h, w)
         bn = r["bn"]
         call("fpl_dsbn_act_bwd_apply_fin", *common, ptr(red), r["training"], ptr(dy), n, d, h, w, c, st,
              ptr(grads[bn.weight]), ptr(grads[bn.bias]), ptr(grads[u.prelu.weight]), ptr(grads[u.conv.bias]))
         dw = grads[u.conv.weight]
-        if u.is_stem and r.get("stem_direct"):
+        wgrad = plan.wgrad[u.name]
+        if wgrad in ("stem_direct", "stem_cc"):
             call("fpl_stem_conv_wgrad", ptr(r["x_img"]), ptr(dy), c // 8, 0, ptr(dw), n, u.cin, d, h, w, c, u.kd, st)
             return None
-        if u.is_stem and self._stem_tc(d):
+        if wgrad == "stem_patch":
             # the patch tensor of the forward is still in the workspace: k(3,1,1) wgrad, one MMA per K step
             xs = ws.c8("XS:stem", n, d, 32, h, w)
             dw16 = ws.get("dW16s", (c, 16, 3), torch.float32)
@@ -903,94 +853,41 @@ class UNet2D5_dsbn(nn.Module):
             call("fpl_conv3d_wgrad_tc_k311", ptr(xs), 4, 0, ptr(dy), c // 8, 0, ptr(dw16), n, d, h, w, 16, c, st)   # hi half
             dw.view(c, 1, 3, 3, 3).add_(dw16[:, :9, :].permute(0, 2, 1).reshape(c, 1, 3, 3, 3))
             return None
-        if u.is_stem:
-            if self._use_tc(16, c) and u.cin <= 8 and os.environ.get("FPL_WGRAD_IMPL", "tc") == "tc":
-                # image -> one bf16 channel group (zero padded), then the tensor-core wgrad with Cin = 8
-                x8 = ws.c8("X8", n, d, 8, h, w)
-                call("fpl_pack_ncdhw_to_c8", ptr(r["x_img"]), u.cin, ptr(x8), 1, 0, 1, None, n, d, h, w, st)
-                dw8 = ws.get("dW8", (c, 8, u.kd, 3, 3), torch.float32)
-                dw8.zero_()
-                call("fpl_conv3d_wgrad_tc", ptr(x8), 1, 0, ptr(dy), c // 8, 0, ptr(dw8), n, d, h, w, 8, c, u.kd, st)
-                dw.view(c, u.cin, u.kd, 3, 3).add_(dw8[:, :u.cin])
-            else:
-                call("fpl_stem_conv_wgrad", ptr(r["x_img"]), ptr(dy), c // 8, 0, ptr(dw), n, u.cin, d, h, w, c, u.kd, st)
+        if wgrad == "stem_c8":
+            # image -> one bf16 channel group (zero padded), then the tensor-core wgrad with Cin = 8
+            x8 = ws.c8("X8", n, d, 8, h, w)
+            call("fpl_pack_ncdhw_to_c8", ptr(r["x_img"]), u.cin, ptr(x8), 1, 0, 1, None, n, d, h, w, st)
+            dw8 = ws.get("dW8", (c, 8, u.kd, 3, 3), torch.float32)
+            dw8.zero_()
+            call("fpl_conv3d_wgrad_tc", ptr(x8), 1, 0, ptr(dy), c // 8, 0, ptr(dw8), n, d, h, w, 8, c, u.kd, st)
+            dw.view(c, u.cin, u.kd, 3, 3).add_(dw8[:, :u.cin])
             return None
         xin = r["xin"]
-        aux = self._aux_stream()
-        if aux is not None:
-            # dW does not feed the rest of backward: issue it on a side stream so that it fills the tensor pipe
-            # while the main stream runs the HBM-bound BatchNorm kernels of the next unit
-            cur = torch.cuda.current_stream()
-            ready = torch.cuda.Event()
-            ready.record(cur)
-            aux.wait_event(ready)
-            with torch.cuda.stream(aux):
-                self._wgrad(u, xin, dy, dw, n, d, h, w, fold)
+        if wgrad == "tapmajor":
+            # tap-major scratch (coalesced epilogue atomics); folded into dw by one batched launch later
+            scr = fold["alloc"](u.cout * u.cin * u.kd * 9)
+            call("fpl_conv3d_wgrad_tc_tapmajor", *xin.args(), ptr(dy), u.cout // 8, 0, ptr(scr), n, d, h, w, u.cin,
+                 u.cout, u.kd, st)
+            fold["pending"].append((scr, dw, u.cout, u.cin, u.kd * 9))
         else:
-            self._wgrad(u, xin, dy, dw, n, d, h, w, fold)
+            call("fpl_conv3d_wgrad", *xin.args(), ptr(dy), u.cout // 8, 0, ptr(dw), n, d, h, w, u.cin, u.cout, u.kd, st)
         if not need_dx:
             return None
         dx = ws.c8("dX:" + u.name, n, d, u.cin, h, w)
-        br = None
-        if prev is not None and self._bwdred_ok(*prev) and (self._dfold_ok(u.cout, u.cin, u.kd, d) or self._use_tc(u.cout, u.cin)):
-            up, rp = prev
-            rp["red_fused"] = small.f64(2 * up.cout + 1)
-            br = (ptr(rp["y"]), ptr(rp["scale"]), ptr(rp["shift"]), ptr(rp["mean"]), ptr(rp["invstd"]), ptr(up.prelu.weight),
-                  rp["p"], rp["seed"], rp["offset"], ptr(rp["seed_dev"]), ptr(rp["red_fused"]))
-        if self._dfold_ok(u.cout, u.cin, u.kd, d):
-            if br is not None:
-                call("fpl_conv3d_tc_dfold_bwdred", ptr(dy), c // 8, 0, ptr(self._dfold_image(u.conv, True)), ptr(dx),
-                     u.cin // 8, 0, n, d, h, w, c, u.cin, *br, st)
-            else:
-                call("fpl_conv3d_tc_dfold", ptr(dy), c // 8, 0, ptr(self._dfold_image(u.conv, True)), None, ptr(dx),
-                     u.cin // 8, 0, None, n, d, h, w, c, u.cin, st)
-        elif self._use_tc(u.cout, u.cin):
-            img = self._weight_image(u.conv, u.kd, True, ws)
-            if br is not None:
-                call("fpl_conv3d_tc_bwdred", ptr(dy), c // 8, 0, ptr(img), ptr(dx), u.cin // 8, 0, n, d, h, w, c, u.cin,
-                     u.kd, *br, st)
-            else:
-                call("fpl_conv3d_tc", ptr(dy), c // 8, 0, ptr(img), None, ptr(dx), u.cin // 8, 0, None,
-                     n, d, h, w, c, u.cin, u.kd, st)
+        kern = plan.dgrad[u.name]
+        if kern == "dfold":
+            call("fpl_conv3d_tc_dfold", ptr(dy), c // 8, 0, ptr(self._image("dfold", u.conv, 1)), None, ptr(dx),
+                 u.cin // 8, 0, None, n, d, h, w, c, u.cin, st)
+        elif kern == "tc":
+            call("fpl_conv3d_tc", ptr(dy), c // 8, 0, ptr(self._image("tc", u.conv, 1)), None, ptr(dx), u.cin // 8, 0,
+                 None, n, d, h, w, c, u.cin, u.kd, st)
         else:
             call("fpl_conv3d_direct", ptr(dy), c // 8, 0, ptr(u.conv.weight), None, ptr(dx), u.cin // 8, 0, None,
                  n, d, h, w, c, u.cin, u.kd, 1, 0, st)
         return C8(dx)
 
-    def _aux_stream(self):
-        """The wgrad side stream paired with the current stream (None when disabled)."""
-        if not self.wgrad_side_stream:
-            return None
-        cur = torch.cuda.current_stream()
-        key = cur.cuda_stream
-        st = self._aux_streams.get(key)
-        if st is None:
-            st = self._aux_streams[key] = torch.cuda.Stream(device=cur.device)
-        return st
-
-    def _join_aux(self):
-        aux = self._aux_stream()
-        if aux is not None:
-            torch.cuda.current_stream().wait_stream(aux)
-
-    def _wgrad(self, u, xin, dy, dw, n, d, h, w, fold=None):
-        impl = os.environ.get("FPL_WGRAD_IMPL", "tc")
-        if impl == "tc" and u.cin % 8 == 0 and u.cout % 16 == 0 and ops.is_sm100():
-            if fold is not None:
-                # tap-major scratch (coalesced epilogue atomics); folded into dw by one batched launch later
-                scr = fold["alloc"](u.cout * u.cin * u.kd * 9)
-                call("fpl_conv3d_wgrad_tc_tapmajor", *xin.args(), ptr(dy), u.cout // 8, 0, ptr(scr), n, d, h, w, u.cin,
-                     u.cout, u.kd, stream_ptr())
-                fold["pending"].append((scr, dw, u.cout, u.cin, u.kd * 9))
-                return
-            call("fpl_conv3d_wgrad_tc", *xin.args(), ptr(dy), u.cout // 8, 0, ptr(dw), n, d, h, w, u.cin, u.cout,
-                 u.kd, stream_ptr())
-        else:
-            call("fpl_conv3d_wgrad", *xin.args(), ptr(dy), u.cout // 8, 0, ptr(dw), n, d, h, w, u.cin, u.cout, u.kd,
-                 stream_ptr())
-
     def _run_backward(self, rec, dlogits, domain, ws):
-        n, geo, ft = rec["n"], rec["geo"], self.ft_chns
+        n, geo, ft, plan = rec["n"], rec["geo"], self.ft_chns, rec["plan"]
         params = self._grad_params(domain)
         sizes = [(p.numel() + 3) // 4 * 4 for p in params]
         flat = torch.zeros(sum(sizes), dtype=torch.float32, device=dlogits.device)
@@ -1002,39 +899,24 @@ class UNet2D5_dsbn(nn.Module):
         fired = [0]
         # tap-major scratch of the conv weight gradients (one flat zeroed buffer per backward) + the list of layers
         # whose scratch still has to be folded into the PyTorch layout
-        fold = None
-        if os.environ.get("FPL_WGRAD_TAPMAJOR", "1") != "0" and ops.is_sm100():
-            total = sum((u.conv.weight.numel() + 3) // 4 * 4 for pair in self._down_units + self._up_units for u in pair
-                        if not u.is_stem) + 16 * self.ft_chns[0] * 9 + sum(
-                            (t.weight.numel() + 3) // 4 * 4 for up in (self.up1, self.up2, self.up3, self.up4)
-                            for t in (up.trans3d, up.trans2d) if t is not None) + sum(
-                            9 * u.cin * u.cout for u in self._proj_units)
-            scratch = ws.get("wgrad_scratch", (total,), torch.float32)
-            aux0 = self._aux_stream()
-            if aux0 is not None:
-                # 20+ MB zero fill: on the weight-gradient side stream, under the head dgrad (whose bias gradient needs
-                # `flat`, not the scratch); the main stream picks the event up before its first scratch user
-                cur0 = torch.cuda.current_stream()
-                aux0.wait_stream(cur0)
-                with torch.cuda.stream(aux0):
-                    scratch.zero_()
-                scratch_zeroed = torch.cuda.Event()
-                scratch_zeroed.record(aux0)
-            else:
-                scratch.zero_()
-                scratch_zeroed = None
-            cursor = [0]
+        total = sum((u.conv.weight.numel() + 3) // 4 * 4 for pair in self._down_units + self._up_units for u in pair
+                    if not u.is_stem) + 16 * self.ft_chns[0] * 9 + sum(
+                        (t.weight.numel() + 3) // 4 * 4 for up in (self.up1, self.up2, self.up3, self.up4)
+                        for t in (up.trans3d, up.trans2d) if t is not None) + sum(
+                        9 * u.cin * u.cout for u in self._proj_units)
+        scratch = ws.get("wgrad_scratch", (total,), torch.float32)
+        scratch.zero_()
+        cursor = [0]
 
-            def alloc(numel):
-                t = scratch[cursor[0]:cursor[0] + numel]
-                cursor[0] += (numel + 3) // 4 * 4
-                return t
-            fold = {"alloc": alloc, "pending": []}
+        def alloc(numel):
+            t = scratch[cursor[0]:cursor[0] + numel]
+            cursor[0] += (numel + 3) // 4 * 4
+            return t
+        fold = {"alloc": alloc, "pending": []}
 
         def flush_fold():
-            if fold is None or not fold["pending"]:
+            if not fold["pending"]:
                 return
-            self._join_aux()
             part = fold["pending"]
             m = len(part)
             arr_s = (ctypes.c_void_p * m)(*[t[0].data_ptr() for t in part])
@@ -1056,7 +938,6 @@ class UNet2D5_dsbn(nn.Module):
                 if end > fired[0] and (last or pending_b >= self.grad_bucket_bytes
                                        or (remaining_b <= self.grad_tail_bytes and pending_b >= (1 << 20))):
                     flush_fold()
-                    self._join_aux()
                     self.grad_ready_hook(flat, fired[0], end, n_params_done == len(params))
                     fired[0] = end
 
@@ -1064,55 +945,35 @@ class UNet2D5_dsbn(nn.Module):
         st = stream_ptr()
         d, h, w = geo[0]
         head_in = rec["head_in"]
-
-        def scratch_ready():
-            if fold is not None and scratch_zeroed is not None:
-                torch.cuda.current_stream().wait_event(scratch_zeroed)
         g = C8(ws.c8("dX:head", n, d, ft[0], h, w))
         dlogits = dlogits.contiguous()
-        if self._head_cc(n, d):
+        k = self.n_class
+        if plan.head == "cc":
             # CUDA-core head dgrad (csrc/head.cu): one pass reads the fp32 logit gradient and writes the input gradient,
             # the one-channel-group bf16 copy the tensor-core wgrad consumes and the bias gradient
-            k = self.n_class
             dl8 = ws.c8("dL8", n, d, 8, h, w)
             call("fpl_head_dgrad", ptr(dlogits), ptr(self.out_conv.weight), *g.args(), ptr(dl8), 1, 0,
                  ptr(grads[self.out_conv.bias]), n, d, h, w, ft[0], k, st)
-            scratch_ready()
-            if fold is not None:
-                scr = fold["alloc"](8 * ft[0] * 9)
-                call("fpl_conv3d_wgrad_tc_tapmajor", *head_in.args(), ptr(dl8), 1, 0, ptr(scr), n, d, h, w, ft[0], 8, 1, st)
-                fold["pending"].append((scr, grads[self.out_conv.weight], k, ft[0], 9, 8))
-            else:
-                dw8 = ws.get("dW16", (8, ft[0], 1, 3, 3), torch.float32)
-                dw8.zero_()
-                call("fpl_conv3d_wgrad_tc", *head_in.args(), ptr(dl8), 1, 0, ptr(dw8), n, d, h, w, ft[0], 8, 1, st)
-                grads[self.out_conv.weight].view(k, ft[0], 1, 3, 3).add_(dw8[:k])
-        elif self._head_tc():
+            scr = fold["alloc"](8 * ft[0] * 9)
+            call("fpl_conv3d_wgrad_tc_tapmajor", *head_in.args(), ptr(dl8), 1, 0, ptr(scr), n, d, h, w, ft[0], 8, 1, st)
+            fold["pending"].append((scr, grads[self.out_conv.weight], k, ft[0], 9, 8))
+        elif plan.head == "tc":
             # dlogits -> bf16 C8-planar (zero padded to 16 channels) + the bias gradient; then the ordinary
             # tensor-core dgrad / wgrad with the padded head weights
-            k = self.n_class
             dl16 = ws.c8("dL16", n, d, 16, h, w)
             call("fpl_pack_ncdhw_to_c8", ptr(dlogits), k, ptr(dl16), 2, 0, 2, ptr(grads[self.out_conv.bias]), n, d, h, w, st)
-            img_t = self._weight_image(self._head, 1, True, ws)
-            call("fpl_conv3d_tc", ptr(dl16), 2, 0, ptr(img_t), None, *g.args(), None, n, d, h, w, 16, ft[0], 1, st)
+            call("fpl_conv3d_tc", ptr(dl16), 2, 0, ptr(self._image("tc", self._head, 1)), None, *g.args(), None,
+                 n, d, h, w, 16, ft[0], 1, st)
             # wgrad against the first channel group of dl16 only (classes padded to 8): 4 depth planes are stacked in
-            # M and N, so one MMA set covers 4 planes (csrc/conv_wgrad_tc.cu, ndy = 4)
+            # M and N, so one MMA set covers 4 planes (csrc/conv_wgrad_tc.cu, ndy = 4); only the k real classes are
+            # folded into the head's gradient
             co = 8 if (ft[0] <= 32 and d >= 2) else 16
-            scratch_ready()
-            if fold is not None:
-                # tap-major scratch; only the k real classes are folded into the head's gradient
-                scr = fold["alloc"](co * ft[0] * 9)
-                call("fpl_conv3d_wgrad_tc_tapmajor", *head_in.args(), ptr(dl16), 2, 0, ptr(scr), n, d, h, w, ft[0], co, 1, st)
-                fold["pending"].append((scr, grads[self.out_conv.weight], k, ft[0], 9, co))
-            else:
-                dw16 = ws.get("dW16", (co, ft[0], 1, 3, 3), torch.float32)
-                dw16.zero_()
-                call("fpl_conv3d_wgrad_tc", *head_in.args(), ptr(dl16), 2, 0, ptr(dw16), n, d, h, w, ft[0], co, 1, st)
-                grads[self.out_conv.weight].view(k, ft[0], 1, 3, 3).add_(dw16[:k])
+            scr = fold["alloc"](co * ft[0] * 9)
+            call("fpl_conv3d_wgrad_tc_tapmajor", *head_in.args(), ptr(dl16), 2, 0, ptr(scr), n, d, h, w, ft[0], co, 1, st)
+            fold["pending"].append((scr, grads[self.out_conv.weight], k, ft[0], 9, co))
         else:
             call("fpl_head_conv_bwd", *head_in.args(), ptr(self.out_conv.weight), ptr(dlogits), *g.args(),
                  ptr(grads[self.out_conv.weight]), ptr(grads[self.out_conv.bias]), n, d, h, w, ft[0], self.n_class, st)
-        scratch_ready()
         ups = [self.up1, self.up2, self.up3, self.up4]
         skip_grads = {}
         done = 2
@@ -1121,45 +982,34 @@ class UNet2D5_dsbn(nn.Module):
             u1, u2 = self._up_units[k]
             up = ups[k]
             c, c_low = ft[lvl], ft[lvl + 1]
-            r1 = rec[u1.name]
-            g = self._unit_bwd(u2, rec[u2.name], g, None, None, 0, n, ws, small, grads, True, fold, prev=(u1, r1))
+            g = self._unit_bwd(u2, rec[u2.name], g, None, None, 0, n, ws, small, grads, True, fold, plan)
             # dgrad of unit 1 produces the gradient of the whole concat buffer; keep it alive per level
-            dcat = self._unit_bwd(u1, r1, g, None, None, 0, n, ws, small, grads, True, fold)
+            dcat = self._unit_bwd(u1, rec[u1.name], g, None, None, 0, n, ws, small, grads, True, fold, plan)
             skip_grads[lvl] = C8(dcat.buf, 0, c)
             trans = up.trans3d if up.dim == 3 else up.trans2d
             kd2 = 2 if up.dim == 3 else 1
             dl, hl, wl = geo[lvl + 1]
             low = rec["up%d.low" % (k + 1)]
             glow = C8(ws.c8("dlow%d" % lvl, n, dl, c_low, hl, wl))
-            if self.bilinear:
+            if plan.up[k] == "proj":
                 pu = self._proj_units[k]
                 proj = up.conv3d if up.dim == 3 else up.conv2d
                 g_t = ws.c8("dT:up%d" % (k + 1), n, dl, c, hl, wl)
                 call("fpl_upsample2x_c8_bwd", ptr(dcat.buf), 2 * c // 8, c // 8, ptr(g_t), c // 8, 0, n, dl, hl, wl, c, kd2, st)
                 call("fpl_channel_sum_c8", ptr(g_t), c // 8, 0, ptr(grads[proj.bias]), n, dl, hl, wl, c, st)
                 # wgrad of the (1,3,3) stand-in: only its centre tap is the 1x1 weight
-                if fold is not None:
-                    scr = fold["alloc"](9 * c * c_low)
-                    call("fpl_conv3d_wgrad_tc_tapmajor", *low.args(), ptr(g_t), c // 8, 0, ptr(scr), n, dl, hl, wl, c_low, c, 1, st)
-                    fold["pending"].append((scr[4 * c * c_low:5 * c * c_low], grads[proj.weight], c, c_low, 1))
-                else:
-                    dw9 = ws.get("dW9:up%d" % (k + 1), (c, c_low, 1, 3, 3), torch.float32)
-                    dw9.zero_()
-                    call("fpl_conv3d_wgrad_tc", *low.args(), ptr(g_t), c // 8, 0, ptr(dw9), n, dl, hl, wl, c_low, c, 1, st)
-                    grads[proj.weight].view(c, c_low).add_(dw9[:, :, 0, 1, 1])
-                call("fpl_conv3d_tc", ptr(g_t), c // 8, 0, ptr(self._weight_image(pu.conv, 1, True, ws)), None, *glow.args(),
+                scr = fold["alloc"](9 * c * c_low)
+                call("fpl_conv3d_wgrad_tc_tapmajor", *low.args(), ptr(g_t), c // 8, 0, ptr(scr), n, dl, hl, wl, c_low, c, 1, st)
+                fold["pending"].append((scr[4 * c * c_low:5 * c * c_low], grads[proj.weight], c, c_low, 1))
+                call("fpl_conv3d_tc", ptr(g_t), c // 8, 0, ptr(self._image("tc", pu.conv, 1)), None, *glow.args(),
                      None, n, dl, hl, wl, c, c_low, 1, st)
-            elif self._convt_tc(c_low, c):
-                call("fpl_convt_k2s2_dgrad_tc", ptr(dcat.buf), 2 * c // 8, c // 8, ptr(self._convt_image(trans, kd2, 1)),
+            elif plan.up[k] == "tc":
+                call("fpl_convt_k2s2_dgrad_tc", ptr(dcat.buf), 2 * c // 8, c // 8, ptr(self._image("convt", trans, 1)),
                      *glow.args(), n, dl, hl, wl, c_low, c, kd2, st)
-                if fold is not None:
-                    scr = fold["alloc"](c_low * c * 4 * kd2)
-                    call("fpl_convt_k2s2_wgrad_tc_tapmajor", *low.args(), ptr(dcat.buf), 2 * c // 8, c // 8, ptr(scr),
-                         n, dl, hl, wl, c_low, c, kd2, st)
-                    fold["pending"].append((scr, grads[trans.weight], c, c_low, -4 * kd2))
-                else:
-                    call("fpl_convt_k2s2_wgrad_tc", *low.args(), ptr(dcat.buf), 2 * c // 8, c // 8, ptr(grads[trans.weight]),
-                         n, dl, hl, wl, c_low, c, kd2, st)
+                scr = fold["alloc"](c_low * c * 4 * kd2)
+                call("fpl_convt_k2s2_wgrad_tc_tapmajor", *low.args(), ptr(dcat.buf), 2 * c // 8, c // 8, ptr(scr),
+                     n, dl, hl, wl, c_low, c, kd2, st)
+                fold["pending"].append((scr, grads[trans.weight], c, c_low, -4 * kd2))
                 call("fpl_convt_k2s2_bwd", *low.args(), ptr(trans.weight), ptr(dcat.buf), 2 * c // 8, c // 8, None, 0, 0,
                      None, ptr(grads[trans.bias]), n, dl, hl, wl, c_low, c, kd2, st)       # bias gradient only
             else:
@@ -1173,21 +1023,20 @@ class UNet2D5_dsbn(nn.Module):
             u1, u2 = self._down_units[i]
             r1 = rec[u1.name]
             if i == 4:
-                g = self._unit_bwd(u2, rec[u2.name], g, None, None, 0, n, ws, small, grads, True, fold, prev=(u1, r1))
+                g = self._unit_bwd(u2, rec[u2.name], g, None, None, 0, n, ws, small, grads, True, fold, plan)
             else:
                 idx, pool_kd = rec["idx%d" % i]
                 g = self._unit_bwd(u2, rec[u2.name], skip_grads[i], g_pool, idx, pool_kd, n, ws, small, grads, True, fold,
-                                   prev=(u1, r1))
+                                   plan)
             r1["x_img"] = rec["x"]
             if i > 0:
-                g_pool = self._unit_bwd(u1, r1, g, None, None, 0, n, ws, small, grads, True, fold)
+                g_pool = self._unit_bwd(u1, r1, g, None, None, 0, n, ws, small, grads, True, fold, plan)
             else:
-                self._unit_bwd(u1, r1, g, None, None, 0, n, ws, small, grads, False, fold)
+                self._unit_bwd(u1, r1, g, None, None, 0, n, ws, small, grads, False, fold, plan)
             done += 10
             fire(done)
         assert done == len(params)
         flush_fold()
-        self._join_aux()
         return self._deliver_grads(params, offs, flat, grads)
 
     # -- gradient delivery --------------------------------------------------------------------
@@ -1211,10 +1060,10 @@ class UNet2D5_dsbn(nn.Module):
         """Hands one backward pass's gradients to the optimiser.  Default: ONE fpl_grad_scatter_add launch adds the
         pass's flat buffer into the master buffer and p.grad is a view of that buffer (autograd gets None: its ~65
         per-parameter AccumulateGrad adds for the second domain pass disappear).  The first pass after a
-        zero_grad(set_to_none=True) zeroes the master buffer.  FPL_GRAD_DIRECT=0, or a p.grad that is not ours,
-        falls back to returning the gradients to autograd."""
+        zero_grad(set_to_none=True) zeroes the master buffer.  FPL_GRAD_DIRECT=0 (read at construction), or a p.grad that
+        is not ours, falls back to returning the gradients to autograd."""
         views = [grads[p].view(p.shape) for p in params]
-        if os.environ.get("FPL_GRAD_DIRECT", "1") == "0":
+        if not self.grad_direct:
             return views
         m = self._master_grads(flat.device)
         base, off = m["buf"].data_ptr(), m["off"]
@@ -1283,11 +1132,7 @@ class _UNetFunction(torch.autograd.Function):
             ws, home = (net._pool.pop() if net._pool else _Workspace(x.device)), net._pool
             if ws.device != x.device:
                 ws = _Workspace(x.device)
-        net._grad_pass = True
-        try:
-            logits, rec = net._run_forward(x, domain, ws)
-        finally:
-            net._grad_pass = False
+        logits, rec = net._run_forward(x, domain, ws, grad=True)
         ctx.net, ctx.domain, ctx.rec = net, domain, rec
         ctx.lease = _Lease(home, ws)
         return logits

@@ -128,24 +128,6 @@ int fpl_wgrad_tapmajor_to_dw_batch(int count, const float* const* h_scratch, flo
  * passes run on two streams).  max_numel = the largest count (grid sizing). */
 int fpl_grad_scatter_add(float* dst, const float* src, const int* d_table, int segments, int max_numel, void* stream);
 
-/* ---- DSBN backward statistics folded into the producing dgrad (autograd of unet2d5_dsbn.py:75-81) -----------------------
- * dgrad forms of fpl_conv3d_tc / fpl_conv3d_tc_dfold (image = the transposed / flipped weight image, no bias, no
- * forward statistics) that ALSO accumulate, for the conv unit whose ACTIVATION gradient they write (dx), the sums its
- * BatchNorm backward needs: red = double[2*cout+1] += {sum dz, sum dz*xhat, dslope} with dz = dx * dropout' * prelu'
- * evaluated from y_prev (that unit's raw conv output, dense C8-planar, `cout` channels), its scale / shift / mean /
- * invstd / PReLU slope and its Philox dropout stream (drop_p, seed, offset, seed_dev as in fpl_dsbn_act_fwd).  They
- * replace the fpl_dsbn_act_bwd_reduce launch (4 B/element) of every unit whose activation feeds exactly one conv. */
-int fpl_conv3d_tc_bwdred(const void* x, int x_c8tot, int x_c8off, const void* image, void* y, int y_c8tot, int y_c8off,
-                         int n, int d, int h, int w, int cin, int cout, int kd, const void* y_prev,
-                         const float* scale, const float* shift, const float* mean, const float* invstd,
-                         const float* slope, float drop_p, uint64_t seed, uint64_t offset, const uint64_t* seed_dev,
-                         double* red, void* stream);
-int fpl_conv3d_tc_dfold_bwdred(const void* x, int x_c8tot, int x_c8off, const void* image, void* y, int y_c8tot,
-                               int y_c8off, int n, int d, int h, int w, int cin, int cout, const void* y_prev,
-                               const float* scale, const float* shift, const float* mean, const float* invstd,
-                               const float* slope, float drop_p, uint64_t seed, uint64_t offset,
-                               const uint64_t* seed_dev, double* red, void* stream);
-
 /* ---- device data path of the training inputs: RandomCrop + RandomFlip (transform/crop.py:170-244, flip.py:14-62) -----
  * d_rows: DEVICE table of n rows of 64 bytes
  *   { const float* image [C][D][H][W]; const uint8_t* label [D][H][W] or NULL; const uint8_t* code [D][H][W] or NULL;

@@ -900,50 +900,6 @@ def test_entropy_term_and_probability_inputs_match_the_oracle():
             {"prediction": pp, "ground_truth": y.to(DEV)})
 
 
-@pytest.mark.parametrize("kernel,cin,cout,shape,drop_p", [
-    ("dfold", 16, 16, (2, 4, 32, 16), 0.0), ("dfold", 32, 16, (1, 5, 20, 12), 0.0), ("dfold", 16, 32, (1, 9, 16, 24), 0.3),
-    ("tc", 64, 64, (2, 4, 16, 16), 0.0), ("tc", 128, 64, (1, 4, 16, 8), 0.4), ("tc", 256, 128, (1, 2, 8, 8), 0.5),
-    ("tc", 256, 256, (4, 2, 8, 8), 0.0)])
-def test_dgrad_epilogue_accumulates_the_dsbn_backward_sums(kernel, cin, cout, shape, drop_p):
-    """Round 2: the dgrad of conv k+1 (cout -> cin here: it writes the gradient wrt unit k's `cin` activation channels)
-    also accumulates unit k's BatchNorm-backward sums {sum dz, sum dz*xhat, dslope}; they must equal what
-    fpl_dsbn_act_bwd_reduce computes from the stored bf16 gradient, and dx must be bit-identical to the plain dgrad."""
-    n, d, h, w = shape
-    c_prev = cin                                    # unit k has `cin` output channels
-    wt = bf16_round(randn(21, cout, cin, 3, 3, 3, scale=0.1)).to(DEV)
-    dy = to_c8(bf16_round(randn(22, n, cout, d, h, w)).to(DEV))
-    y_prev = to_c8((bf16_round(randn(23, n, c_prev, d, h, w, scale=2.0)) + 0.3).to(DEV))
-    scale, shift = (randn(24, c_prev, scale=0.3) + 1.0).to(DEV), randn(25, c_prev, scale=0.5).to(DEV)
-    mean, invstd = randn(26, c_prev, scale=0.5).to(DEV), (randn(27, c_prev, scale=0.2).abs() + 0.5).to(DEV)
-    slope = torch.tensor([0.2], device=DEV)
-    seed, offset = 12345, 64
-    from fplplus_b200 import lib as L
-    if kernel == "dfold":
-        img = torch.empty(L.load().fpl_conv3d_dfold_image_bytes(cout, cin) // 2, dtype=torch.bfloat16, device=DEV)
-        _call("fpl_conv3d_dfold_prep_weight", _p(wt), cin, cout, 1, _p(img), _st())
-    else:
-        img = torch.empty(L.load().fpl_conv3d_weight_image_bytes(cout, cin, 3) // 2, dtype=torch.bfloat16, device=DEV)
-        _call("fpl_conv3d_prep_weight", _p(wt), cin, cout, 3, 1, _p(img), _st())
-    dx_plain = torch.zeros((n, d, cin // 8, h, w, 8), dtype=torch.bfloat16, device=DEV)
-    dx_fused = torch.zeros_like(dx_plain)
-    red_fused = torch.zeros(2 * c_prev + 1, dtype=torch.float64, device=DEV)
-    br = (_p(y_prev), _p(scale), _p(shift), _p(mean), _p(invstd), _p(slope), drop_p, seed, offset, None, _p(red_fused))
-    if kernel == "dfold":
-        _call("fpl_conv3d_tc_dfold", _p(dy), cout // 8, 0, _p(img), None, _p(dx_plain), cin // 8, 0, None, n, d, h, w, cout, cin, _st())
-        _call("fpl_conv3d_tc_dfold_bwdred", _p(dy), cout // 8, 0, _p(img), _p(dx_fused), cin // 8, 0, n, d, h, w, cout, cin, *br, _st())
-    else:
-        _call("fpl_conv3d_tc", _p(dy), cout // 8, 0, _p(img), None, _p(dx_plain), cin // 8, 0, None, n, d, h, w, cout, cin, 3, _st())
-        _call("fpl_conv3d_tc_bwdred", _p(dy), cout // 8, 0, _p(img), _p(dx_fused), cin // 8, 0, n, d, h, w, cout, cin, 3, *br, _st())
-    assert torch.equal(dx_plain, dx_fused)
-    red_ref = torch.zeros(2 * c_prev + 1, dtype=torch.float64, device=DEV)
-    _call("fpl_dsbn_act_bwd_reduce", _p(y_prev), _p(dx_plain), cin // 8, 0, None, 0, 0, None, 0, _p(scale), _p(shift), _p(mean),
-          _p(invstd), _p(slope), drop_p, None, seed, offset, None, _p(red_ref), n, d, h, w, c_prev, _st())
-    a, b = red_fused.cpu(), red_ref.cpu()
-    tol = 2e-5 * float(b.abs().max()) + 1e-6
-    assert float((a - b).abs().max()) <= tol, (float((a - b).abs().max()), tol)
-    assert float(b[:c_prev].abs().max()) > 0 and float(b[-1].abs()) > 0
-
-
 @pytest.mark.parametrize("weighted", [False, True])
 def test_exact_data_parallel_dice_equals_the_global_batch_loss(weighted):
     """SURVEY 8e: nn.DataParallel evaluates Dice / CE over the gathered global batch.  Emulation of two ranks on one

@@ -1,5 +1,5 @@
 """GPU probe: what do the epilogues of the conv kernels cost?  Each variant is captured 10x into a CUDA graph and timed.
-  dfold / conv_tc : plain store | + forward BatchNorm statistics | + fused BatchNorm-backward sums (EpiBwdRed)
+  dfold / conv_tc : plain store | + forward BatchNorm statistics; and the standalone BatchNorm-backward reduce
 Usage: python tools/epi_probe.py"""
 import os
 import sys
@@ -52,21 +52,17 @@ def probe(cin, cout, shape, kind):
         ops.call("fpl_conv3d_dfold_prep_weight", P(wt), cin, cout, 0, P(img), st())
         plain = lambda: ops.call("fpl_conv3d_tc_dfold", P(x), cin // 8, 0, P(img), None, P(y), cout // 8, 0, None, n, d, h, w, cin, cout, st())
         wstat = lambda: ops.call("fpl_conv3d_tc_dfold", P(x), cin // 8, 0, P(img), None, P(y), cout // 8, 0, P(stats), n, d, h, w, cin, cout, st())
-        fused = lambda: ops.call("fpl_conv3d_tc_dfold_bwdred", P(x), cin // 8, 0, P(img), P(y), cout // 8, 0, n, d, h, w, cin, cout,
-                                 P(yprev), P(sc), P(sh), P(mean), P(inv), P(slope), 0.0, 0, 0, None, P(red), st())
     else:
         img = torch.empty(L.fpl_conv3d_weight_image_bytes(cin, cout, 3) // 2, dtype=torch.bfloat16, device=DEV)
         ops.call("fpl_conv3d_prep_weight", P(wt), cin, cout, 3, 0, P(img), st())
         plain = lambda: ops.call("fpl_conv3d_tc", P(x), cin // 8, 0, P(img), None, P(y), cout // 8, 0, None, n, d, h, w, cin, cout, 3, st())
         wstat = lambda: ops.call("fpl_conv3d_tc", P(x), cin // 8, 0, P(img), None, P(y), cout // 8, 0, P(stats), n, d, h, w, cin, cout, 3, st())
-        fused = lambda: ops.call("fpl_conv3d_tc_bwdred", P(x), cin // 8, 0, P(img), P(y), cout // 8, 0, n, d, h, w, cin, cout, 3,
-                                 P(yprev), P(sc), P(sh), P(mean), P(inv), P(slope), 0.0, 0, 0, None, P(red), st())
     reduce_ = lambda: ops.call("fpl_dsbn_act_bwd_reduce", P(yprev), P(y), cout // 8, 0, None, 0, 0, None, 0, P(sc), P(sh), P(mean),
                                P(inv), P(slope), 0.0, None, 0, 0, None, P(red), n, d, h, w, cout, st())
-    t = [graph_time(fn) for fn in (plain, wstat, fused, reduce_)]
+    t = [graph_time(fn) for fn in (plain, wstat, reduce_)]
     gf = 2.0 * n * d * h * w * 27 * cin * cout / 1e9
-    print("%-6s %3d->%3d %-18s plain %6.1f us (%5.0f TF/s) | +stats %6.1f | +bwdred %6.1f | standalone reduce %6.1f" % (
-        kind, cin, cout, shape, t[0], gf / t[0] / 1e-6 / 1e3, t[1], t[2], t[3]), flush=True)
+    print("%-6s %3d->%3d %-18s plain %6.1f us (%5.0f TF/s) | +stats %6.1f | standalone reduce %6.1f" % (
+        kind, cin, cout, shape, t[0], gf / t[0] / 1e-6 / 1e3, t[1], t[2]), flush=True)
 
 
 for args in [(16, 16, (4, 32, 128, 128), "dfold"), (32, 16, (4, 32, 128, 128), "dfold"), (16, 32, (4, 16, 64, 64), "dfold"),
