@@ -571,12 +571,6 @@ class SegmentationAgent(object):
             if self._side_stream is None:
                 self._side_stream = torch.cuda.Stream()
             self._side_stream.wait_stream(main)
-            stagger = float(os.environ.get("FPL_STAGGER_US", "0") or 0)
-            if stagger > 0:
-                # experiment knob: start the second domain pass late, so that the two streams are not in the same phase
-                # (tensor-bound / HBM-bound / latency-bound kernels of one against those of the other)
-                with torch.cuda.stream(self._side_stream):
-                    torch.cuda._sleep(int(stagger * 1965))
         losses, dices = [], []
         for d in present:
             data = batches[d]

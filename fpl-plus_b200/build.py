@@ -28,10 +28,6 @@ def needs_build():
 
 
 def build(force=False, verbose=False):
-    # A/B timing of two builds on one GPU box (tools/ab_step.sh): FPL_LIB_AB names another build of THIS library
-    ab = os.environ.get("FPL_LIB_AB")
-    if ab and os.path.exists(ab):
-        return ab
     if not force and not needs_build():
         return LIB
     nvcc = _nvcc()

@@ -79,7 +79,6 @@ struct TcParams {
     int nb, kc, nslices, nchunks, a_bytes, b_bytes, stages, tmem_cols;   // nb / nslices / b_bytes: of THIS launch (after nsub)
     int nsub, nb_img, b_bytes_img;   // N split of a staged image slice: nb = nb_img / nsub (few-tile layers: more, smaller CTAs)
     int tiles_h, tiles_w, total_tiles;
-    int dbg_swap_lbo_sbo;
     float* logits;        // head mode: fp32 NCDHW output of the first `classes` channels instead of bf16 C8-planar
     int classes;
     EpiAct act;           // act.scale != NULL: inference epilogue (affine + PReLU + dropout) instead of + bias
@@ -172,12 +171,8 @@ __global__ void __launch_bounds__(kNumThreads) conv3d_tc_kernel(const __grid_con
     } else if (warp == 1) {
         // ===================== MMA issuer: the whole warp runs the loop (uniform), one lane issues =====================
         const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(P.nb >> 3) << 17) | (8u << 24);
-        const uint32_t a_lbo = P.dbg_swap_lbo_sbo ? kBoxW * 16 : kPlaneBytes;
-        const uint32_t a_sbo = P.dbg_swap_lbo_sbo ? kPlaneBytes : kBoxW * 16;
-        const uint32_t b_lbo = P.dbg_swap_lbo_sbo ? 128 : P.nb * 16;
-        const uint32_t b_sbo = P.dbg_swap_lbo_sbo ? P.nb * 16 : 128;
         // descriptors = constant high part + (smem byte address >> 4) in the low 14 bits
-        const uint64_t a_hi = make_desc(0, a_lbo, a_sbo), b_hi = make_desc(0, b_lbo, b_sbo);
+        const uint64_t a_hi = make_desc(0, kPlaneBytes, kBoxW * 16), b_hi = make_desc(0, P.nb * 16, 128);
         const uint32_t smem_u = smem_u32(smem) >> 4;
         const uint64_t b_tap_step = (uint64_t)((P.kc / 8) * P.nb);        // 16-byte units between taps of B
         const uint64_t b_k_step = (uint64_t)(2 * P.nb);                   // ... between 16-channel K steps
@@ -474,21 +469,6 @@ extern "C" int fpl_conv3d_prep_weight_batch(int count, const float* const* h_w, 
     return 0;
 }
 
-static int g_dbg_swap = 0, g_tc_allow_nsub = 1;
-void fpl_wgrad_debug_set(int key, long long value);
-void fpl_dsbn_debug_set(int key, long long value);
-void fpl_dfold_debug_knob(int key, long long value);
-void fpl_head_tc_debug_set(int key, long long value);
-void fpl_stem_tc_debug_set(int key, long long value);
-extern "C" void fpl_debug_set(int key, long long value) {
-    if (key == 0) g_dbg_swap = (int)value;
-    if (key == 1) g_tc_allow_nsub = (int)value;
-    if (key >= 10 && key < 30) fpl_wgrad_debug_set(key, value);
-    if (key >= 30 && key < 40) fpl_dsbn_debug_set(key, value);
-    if (key >= 40 && key < 50) fpl_dfold_debug_knob(key, value);
-    if (key >= 50 && key < 60) { fpl_head_tc_debug_set(key, value); fpl_stem_tc_debug_set(key, value); }
-}
-
 static int conv3d_tc_launch(const void* x, int x_c8tot, int x_c8off, const void* image, const float* bias, void* y,
                             int y_c8tot, int y_c8off, double* stats, int n, int d, int h, int w, int cin, int cout,
                             int kd, float* logits, int classes, void* stream, const EpiAct* act = nullptr) {
@@ -521,7 +501,7 @@ static int conv3d_tc_launch(const void* x, int x_c8tot, int x_c8off, const void*
     P.nsub = 1; P.nb_img = c.nb; P.b_bytes_img = c.b_bytes;
     {
         const int64_t mn = (int64_t)P.tiles_h * P.tiles_w * d * n * c.nslices;
-        while (g_tc_allow_nsub && logits == nullptr && P.nsub < 4 && c.nb % (P.nsub * 2 * 16) == 0 && c.nb / (P.nsub * 2) >= 32 &&
+        while (logits == nullptr && P.nsub < 4 && c.nb % (P.nsub * 2 * 16) == 0 && c.nb / (P.nsub * 2) >= 32 &&
                mn * P.nsub < 96)
             P.nsub *= 2;
     }
@@ -529,7 +509,6 @@ static int conv3d_tc_launch(const void* x, int x_c8tot, int x_c8off, const void*
     int64_t total = (int64_t)P.tiles_h * P.tiles_w * d * n * P.nslices;
     FPL_REQUIRE(total < (1ll << 30), "fpl_conv3d_tc: too many tiles");
     P.total_tiles = (int)total;
-    P.dbg_swap_lbo_sbo = g_dbg_swap;
     P.logits = logits; P.classes = classes;
     if (act != nullptr) P.act = *act; else { P.act.scale = nullptr; P.act.shift = nullptr; P.act.slope = nullptr; P.act.drop_p = 0.0f; P.act.seed = P.act.offset = 0; P.act.seed_dev = nullptr; }
     FPL_CHECK_CUDA(cudaFuncSetAttribute(conv3d_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, c.smem_bytes));

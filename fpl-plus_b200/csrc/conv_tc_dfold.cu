@@ -39,8 +39,6 @@ struct DfParams {
     int taps;                        // 9 (k 3x3x3) or 1 (k 3x1x1: only the centre in-plane tap)
     int a_ksteps;                    // distinct 16-channel K steps of A (B K step j reads A K step j % a_ksteps)
     EpiAct act;                      // act.scale != NULL: inference epilogue (affine + PReLU) instead of + bias
-    int dbg_epi, dbg_nomma, dbg_tma;
-    long long* dbg_trace;            // fpl_debug_set 47: CTA 0 logs clock64() per role and plane ([role][4096] entries)          // timing experiments only (fpl_debug_set 42 / 44): results are wrong when set
 };
 
 __device__ __forceinline__ void tmem_st_zero16(uint32_t taddr) {
@@ -105,7 +103,6 @@ __global__ void __launch_bounds__(kThreadsD, 2) conv3d_tc_dfold_kernel(const __g
     float* bias_sm = reinterpret_cast<float*>(bars + 2 * kMaxStagesD + kMaxDC + 4);
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const bool trace = P.dbg_trace != nullptr && blockIdx.x == 0;
     if (warp == 0 && lane == 0) {
         asm volatile("prefetch.tensormap [%0];" ::"l"(&xmap) : "memory");
         for (int s = 0; s < P.stages; ++s) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], 1); }
@@ -132,7 +129,6 @@ __global__ void __launch_bounds__(kThreadsD, 2) conv3d_tc_dfold_kernel(const __g
         if (lane == 0) {
             int cur_slice = -1;
             int stage = 0; uint32_t phase = 0;
-            int ntr0 = 0, ntr5 = 0;
             for (int t = blockIdx.x; t < P.total_items; t += gridDim.x) {
                 const DfItem c = decode_item(P, t);
                 if (c.dcount == 0) continue;
@@ -148,33 +144,12 @@ __global__ void __launch_bounds__(kThreadsD, 2) conv3d_tc_dfold_kernel(const __g
                     }
                 }
                 // ONE box per stage = pb consecutive input planes (planes outside the volume: TMA zero fill).  A box costs
-                // the TMA unit ~400 cycles of fixed overhead + ~8 per row per CTA whatever its size (tools/dfold_knob_probe.py:
+                // the TMA unit ~400 cycles of fixed overhead + ~8 per row per CTA whatever its size (profiles/r02c_dfold_knobs.log:
                 // the load pipeline alone took 28 us of the 47 us of the 16 -> 16 layer with one 5.8 KB box per plane)
                 for (int z = c.d0 - 1; z <= c.d0 + c.dcount; z += P.pb) {
                     mbar_wait(&empty_bar[stage], phase ^ 1);
-                    if (trace) { P.dbg_trace[0 * 4096 + (ntr0++ & 4095)] = clock64(); }
-                    if (P.dbg_tma == 0) {
-                        mbar_expect_tx(&full_bar[stage], stage_bytes);
-                        tma_load_5d(ring + (size_t)stage * stage_bytes, &xmap, &full_bar[stage], (c.w0 - 1) * 8, c.h0 - 1, P.x_c8off, z, c.n);
-                    } else {     // timing experiments: narrower boxes / other element size (see dfold_launch)
-                        const int bw = (P.dbg_tma & 1) ? kTileW : kBoxW, bh = (P.dbg_tma & 8) ? kTileH : kBoxH;
-                        mbar_expect_tx(&full_bar[stage], (uint32_t)(bw * bh * 16 * (P.a_bytes / kPlaneBytes) * P.pb));
-                        tma_load_5d(ring + (size_t)stage * stage_bytes, &xmap, &full_bar[stage],
-                                    ((P.dbg_tma & 1) ? c.w0 : c.w0 - 1) * ((P.dbg_tma & 2) ? 2 : 8), (P.dbg_tma & 8) ? c.h0 : c.h0 - 1,
-                                    P.x_c8off, z, c.n);
-                    }
-                    if (trace) { P.dbg_trace[5 * 4096 + (ntr5++ & 4095)] = clock64(); }
-                    if (++stage == P.stages) { stage = 0; phase ^= 1; }
-                }
-            }
-        } else if (lane == 1 && trace) {
-            // trace only: watches the boxes land (the MMA warp may look at a full barrier late)
-            int stage = 0, ntr6 = 0; uint32_t phase = 0;
-            for (int t = blockIdx.x; t < P.total_items; t += gridDim.x) {
-                const DfItem c = decode_item(P, t);
-                for (int z = c.d0 - 1; z <= c.d0 + c.dcount; z += P.pb) {
-                    mbar_wait(&full_bar[stage], phase);
-                    P.dbg_trace[6 * 4096 + (ntr6++ & 4095)] = clock64();
+                    mbar_expect_tx(&full_bar[stage], stage_bytes);
+                    tma_load_5d(ring + (size_t)stage * stage_bytes, &xmap, &full_bar[stage], (c.w0 - 1) * 8, c.h0 - 1, P.x_c8off, z, c.n);
                     if (++stage == P.stages) { stage = 0; phase ^= 1; }
                 }
             }
@@ -192,7 +167,6 @@ __global__ void __launch_bounds__(kThreadsD, 2) conv3d_tc_dfold_kernel(const __g
         int stage = 0; uint32_t phase = 0;
         uint32_t item_phase = 0, w_phase = 0;
         int cur_slice = -1;
-        int ntr1 = 0, ntr2 = 0, ntr4 = 0;
         for (int t = blockIdx.x; t < P.total_items; t += gridDim.x) {
             const DfItem c = decode_item(P, t);
             if (c.dcount == 0) continue;
@@ -203,11 +177,9 @@ __global__ void __launch_bounds__(kThreadsD, 2) conv3d_tc_dfold_kernel(const __g
             }
             mbar_wait(acc_free, item_phase);                            // accumulators drained + zeroed
             tc_fence_after();
-            if (trace && leader) { P.dbg_trace[4 * 4096 + (ntr4++ & 4095)] = clock64(); }
             for (int r0 = -1; r0 <= c.dcount; r0 += P.pb) {             // one box = input planes z = d0 + r0 .. + pb - 1
                 mbar_wait(&full_bar[stage], phase);
                 tc_fence_after();
-                if (trace && leader) { P.dbg_trace[1 * 4096 + (ntr1++ & 4095)] = clock64(); }
                 for (int q = 0; q < P.pb; ++q) {
                     const int r = r0 + q, z = c.d0 + r;
                     if (r > c.dcount) break;
@@ -226,13 +198,13 @@ __global__ void __launch_bounds__(kThreadsD, 2) conv3d_tc_dfold_kernel(const __g
                         for (int j = 0; j < ksteps; ++j, b_j += b_kstep) {
                             const uint64_t a_j = a_hi + (uint64_t)(a_base + (uint32_t)(j % P.a_ksteps) * (2 * kPlaneBytes / 16));
                             if (P.taps == 1) {
-                                if (leader && !P.dbg_nomma) umma_bf16(d_tmem, a_j + (uint64_t)(kBoxW + 1), b_j, idesc, 1u);
+                                if (leader) umma_bf16(d_tmem, a_j + (uint64_t)(kBoxW + 1), b_j, idesc, 1u);
                             } else {
                                 uint64_t bdesc = b_j;
 #pragma unroll
                                 for (int t9 = 0; t9 < 9; ++t9, bdesc += b_tap) {
                                     const uint64_t adesc = a_j + (uint64_t)((t9 / 3) * kBoxW + (t9 % 3));
-                                    if (leader && !P.dbg_nomma) umma_bf16(d_tmem, adesc, bdesc, idesc, 1u);
+                                    if (leader) umma_bf16(d_tmem, adesc, bdesc, idesc, 1u);
                                 }
                             }
                         }
@@ -244,7 +216,6 @@ __global__ void __launch_bounds__(kThreadsD, 2) conv3d_tc_dfold_kernel(const __g
                 }
                 if (leader) umma_commit(&empty_bar[stage]);
                 __syncwarp();
-                if (trace && leader) { P.dbg_trace[2 * 4096 + (ntr2++ & 4095)] = clock64(); }
                 if (++stage == P.stages) { stage = 0; phase ^= 1; }
             }
             // a short last chunk: complete the unused plane barriers too, so that every barrier flips once per item
@@ -281,7 +252,6 @@ __global__ void __launch_bounds__(kThreadsD, 2) conv3d_tc_dfold_kernel(const __g
         if (lane == 0) mbar_arrive(acc_free);
         uint32_t item_phase = 0;
         int cur_slice = -1;
-        int ntr3 = 0;
         const float act_slope = fuse_act ? __ldg(P.act.slope) : 0.0f;
         for (int t = blockIdx.x; t < P.total_items; t += gridDim.x) {
             const DfItem c = decode_item(P, t);
@@ -309,7 +279,6 @@ __global__ void __launch_bounds__(kThreadsD, 2) conv3d_tc_dfold_kernel(const __g
             for (int p = 0; p < c.dcount; ++p) {
                 mbar_wait(&done_bar[p], item_phase);
                 tc_fence_after();
-                if (trace && warp == 2 && lane == 0) { P.dbg_trace[3 * 4096 + (ntr3++ & 4095)] = clock64(); }
                 const int64_t out_base = (((int64_t)c.n * P.D + c.d0 + p) * P.y_c8tot + P.y_c8off + (c.slice * P.nb) / 8) * HW +
                                          (int64_t)h * P.W + w;
 #pragma unroll
@@ -318,7 +287,6 @@ __global__ void __launch_bounds__(kThreadsD, 2) conv3d_tc_dfold_kernel(const __g
                         const int c0 = k * 16;
                         const uint32_t taddr = lane_base + (uint32_t)(p * P.nb + c0);
                         uint32_t r[16];
-                        if (P.dbg_epi >= 2) continue;
                         tmem_ld16(taddr, r);
                         tmem_ld_wait();
                         tmem_st_zero16(taddr);                          // leave the slot clean for the next item
@@ -347,7 +315,7 @@ __global__ void __launch_bounds__(kThreadsD, 2) conv3d_tc_dfold_kernel(const __g
                                 }
                             }
                         }
-                        if (valid && P.dbg_epi == 0) {
+                        if (valid) {
                             st_bf16x8(P.y + out_base + (int64_t)(c0 / 8) * HW, v);
                             st_bf16x8(P.y + out_base + (int64_t)(c0 / 8 + 1) * HW, v + 8);
                         }
@@ -424,9 +392,6 @@ __global__ void dfold_prep_kernel(const float* __restrict__ w, __nv_bfloat16* im
     }
 }
 
-int g_df_ctas = 0, g_df_dc = 0, g_df_epi = 0, g_df_stages = 0, g_df_nomma = 0, g_df_tma = 0, g_df_pb = 0, g_df_split_tail = 1;   // fpl_debug_set 40..48
-long long* g_df_trace = nullptr;
-
 struct DfCfg {
     int nb, nslices, dc, stages, a_bytes, b_bytes, tmem_cols, smem_bytes, ctas_per_sm, pb;
 };
@@ -442,7 +407,6 @@ bool make_df_cfg(int cin, int cout, int d, DfCfg& c, int taps = 9, int cin_a = 0
     if (c.b_bytes > 112 * 1024) return false;
     c.a_bytes = (cin_a / 8) * kPlaneBytes;
     c.dc = c.nb == 16 ? 16 : 8;
-    if (g_df_dc > 0 && g_df_dc * c.nb <= 512) c.dc = g_df_dc;
     if (c.dc > d) c.dc = d;
     if (c.dc < 2) return false;
     int cols = c.dc * c.nb;
@@ -450,7 +414,7 @@ bool make_df_cfg(int cin, int cout, int d, DfCfg& c, int taps = 9, int cin_a = 0
     while (c.tmem_cols < cols) c.tmem_cols *= 2;
     if (c.tmem_cols > 512) return false;
     // pb input planes per TMA box / pipeline stage; as many stages (2..4) as keep two CTAs per SM, else what fits one
-    c.pb = g_df_pb > 0 ? g_df_pb : (c.a_bytes <= 2 * kPlaneBytes ? 3 : 2);      // measured: tools/dfold_knob_probe.py pb
+    c.pb = c.a_bytes <= 2 * kPlaneBytes ? 3 : 2;      // measured: profiles/r02c_dfold_knobs.log
     // (ONE commit per box -- the producer waiting on the epilogue's plane barriers instead of its own empty barriers --
     //  was measured SLOWER for the Cin 16 layers: 16 -> 16 41.5 -> 46.3 us, pb 1: 47.0 -> 55.7 us; kept two barriers)
     const int fixed = c.b_bytes + 1024 + 512 + 2 * cout * (int)sizeof(float) + 16;
@@ -459,36 +423,14 @@ bool make_df_cfg(int cin, int cout, int d, DfCfg& c, int taps = 9, int cin_a = 0
         if (fixed + s * c.pb * c.a_bytes <= 110 * 1024) c.stages = s;
     for (int s = 4; s >= 2 && c.stages == 0; --s)
         if (fixed + s * c.pb * c.a_bytes <= 220 * 1024) c.stages = s;
-    if (g_df_stages > 0 && g_df_stages <= kMaxStagesD) c.stages = g_df_stages;
     if (c.stages == 0) return false;
     c.smem_bytes = fixed + c.stages * c.pb * c.a_bytes;
     if (c.smem_bytes > 220 * 1024) return false;
     c.ctas_per_sm = (c.smem_bytes <= 110 * 1024 && c.tmem_cols <= 256) ? 2 : 1;
-    if (g_df_ctas > 0 && g_df_ctas <= c.ctas_per_sm) c.ctas_per_sm = g_df_ctas;
     return true;
 }
 
-int g_dfold_enable = 1;
-
 }  // namespace
-
-void fpl_dfold_debug_set(int value) { g_dfold_enable = value; }
-void fpl_dfold_debug_knob(int key, long long value) {
-    if (key == 40) g_df_ctas = (int)value;
-    if (key == 41) g_df_dc = (int)value;
-    if (key == 42) g_df_epi = (int)value;
-    if (key == 43) g_df_stages = (int)value;
-    if (key == 44) g_df_nomma = (int)value;
-    if (key == 45) g_df_tma = (int)value;
-    if (key == 46) g_df_pb = (int)value;
-    if (key == 48) g_df_split_tail = (int)value;
-    if (key == 47) g_df_trace = reinterpret_cast<long long*>(value);
-}
-
-bool fpl_dfold_eligible(int cin, int cout, int kd, int d) {
-    DfCfg c;
-    return g_dfold_enable && kd == 3 && make_df_cfg(cin, cout, d, c);
-}
 
 extern "C" int64_t fpl_conv3d_dfold_image_bytes(int cin, int cout) {
     DfCfg c;
@@ -586,18 +528,13 @@ static int dfold_launch(const void* x, int x_c8tot, int x_c8off, const void* ima
     EncodeTiledFn encode = get_encode_fn();
     FPL_REQUIRE(encode != nullptr, "fpl_conv3d_tc_dfold: cuTensorMapEncodeTiled not available from the driver");
     CUtensorMap xmap;
-    // timing experiments (fpl_debug_set 45, bit mask; wrong results): 1 = box without the W halo (one aligned 128-byte
-    // line per row), 2 = 8-byte elements, 4 = 256-byte L2 promotion, 8 = box without the H halo
-    const int bw = (g_df_tma & 1) ? kTileW : kBoxW, bh = (g_df_tma & 8) ? kTileH : kBoxH;
-    const int esz = (g_df_tma & 2) ? 8 : 2;
-    cuuint64_t gdim[5] = {(cuuint64_t)w * 16 / esz, (cuuint64_t)h, (cuuint64_t)x_c8tot, (cuuint64_t)d, (cuuint64_t)n};
+    cuuint64_t gdim[5] = {(cuuint64_t)w * 8, (cuuint64_t)h, (cuuint64_t)x_c8tot, (cuuint64_t)d, (cuuint64_t)n};
     cuuint64_t gstride[4] = {(cuuint64_t)w * 16, (cuuint64_t)h * w * 16, (cuuint64_t)x_c8tot * h * w * 16,
                              (cuuint64_t)d * x_c8tot * h * w * 16};
-    cuuint32_t box[5] = {(cuuint32_t)bw * 16 / esz, (cuuint32_t)bh, (cuuint32_t)(cin_a / 8), (cuuint32_t)c.pb, 1};
+    cuuint32_t box[5] = {(cuuint32_t)kBoxW * 8, (cuuint32_t)kBoxH, (cuuint32_t)(cin_a / 8), (cuuint32_t)c.pb, 1};
     cuuint32_t estr[5] = {1, 1, 1, 1, 1};
-    CUresult r = encode(&xmap, esz == 8 ? CU_TENSOR_MAP_DATA_TYPE_UINT64 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<void*>(x), gdim,
-                        gstride, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
-                        (g_df_tma & 4) ? CU_TENSOR_MAP_L2_PROMOTION_L2_256B : CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+    CUresult r = encode(&xmap, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<void*>(x), gdim, gstride, box, estr,
+                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
                         CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     FPL_REQUIRE(r == CUDA_SUCCESS, "fpl_conv3d_tc_dfold: cuTensorMapEncodeTiled failed (%d)", (int)r);
     DfParams P;
@@ -615,10 +552,9 @@ static int dfold_launch(const void* x, int x_c8tot, int x_c8off, const void* ima
     // items each if both halves still fit one extra round (see decode_item); single-slice layers only
     P.full_items = (int)total;
     const int rem = (int)(total % grid);
-    if (g_df_split_tail && rem > 0 && 2 * rem <= grid && c.dc >= 8 && c.dc % 2 == 0 && d % c.dc == 0 && c.nslices == 1) P.full_items = (int)total - rem;
+    if (rem > 0 && 2 * rem <= grid && c.dc >= 8 && c.dc % 2 == 0 && d % c.dc == 0 && c.nslices == 1) P.full_items = (int)total - rem;
     P.total_items = P.full_items + 2 * ((int)total - P.full_items);
     P.taps = taps; P.a_ksteps = cin_a / 16;
-    P.dbg_epi = g_df_epi; P.dbg_nomma = g_df_nomma; P.dbg_tma = g_df_tma; P.dbg_trace = g_df_trace;
     if (act != nullptr) P.act = *act; else { P.act.scale = nullptr; P.act.shift = nullptr; P.act.slope = nullptr; P.act.drop_p = 0.0f; P.act.seed = P.act.offset = 0; P.act.seed_dev = nullptr; }
     if (c.nb == 16) {
         FPL_CHECK_CUDA(cudaFuncSetAttribute(conv3d_tc_dfold_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, c.smem_bytes));

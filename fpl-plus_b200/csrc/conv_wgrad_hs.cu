@@ -37,8 +37,7 @@ struct HsParams {
     int sx, sdy;                   // byte stride of one (plane, channel group) slab in the x / dy tile = row pitch
     int x_bytes, dy_bytes, dy_off, stage_bytes, stages;
     int tiles_h, tiles_w, dplanes, tiles_total, split, nchunks;
-    int tapmajor, skip_epilogue;
-    int dbg;                       // timing experiments (fpl_debug_set 19): 1 = no MMAs, 2 = TMA loads only while the ring first fills
+    int tapmajor;
 };
 
 __device__ __forceinline__ void tmem_st_zero16_hs(uint32_t taddr) {
@@ -94,11 +93,6 @@ __global__ void __launch_bounds__(kThreadsH) conv3d_wgrad_hs_kernel(const __grid
                 const int n = r / P.tiles_h;
                 mbar_wait(&empty_bar[stage], phase ^ 1);
                 uint8_t* x_dst = ring + (size_t)stage * P.stage_bytes;
-                if ((P.dbg & 2) && t - tile_begin >= P.stages) {      // timing experiment: stale tiles, no load
-                    mbar_arrive(&full_bar[stage]);
-                    if (++stage == P.stages) { stage = 0; phase ^= 1; }
-                    continue;
-                }
                 mbar_expect_tx(&full_bar[stage], (uint32_t)(P.x_bytes + P.dy_bytes));
                 // map dimensions (w in 8-byte units, c8, d, h, n); planes / rows / columns outside the volume: zero fill
                 tma_load_5d(x_dst, &xmap, &full_bar[stage], 2 * (tw_i * P.tw - 1), P.x_c8off, 2 * dp - 1, th_i * P.th - 1, n);
@@ -119,7 +113,7 @@ __global__ void __launch_bounds__(kThreadsH) conv3d_wgrad_hs_kernel(const __grid
         // warp, not the tensor pipe, the limit (67-78 cycles per 48-cycle MMA).
         const uint64_t xrow = (uint64_t)((uint32_t)(4 * P.G * P.sx) >> 4), dyrow = (uint64_t)((uint32_t)(4 * P.sdy) >> 4);   // row pitch, 16-byte units
         const uint32_t ring_u = smem_u32(ring);
-        const bool leader = elect_one() && !(P.dbg & 1);
+        const bool leader = elect_one();
         const bool committer = elect_one();
         // per-MMA constants of a K step
         uint64_t a_off[12];
@@ -188,7 +182,6 @@ __global__ void __launch_bounds__(kThreadsH) conv3d_wgrad_hs_kernel(const __grid
         if (tile_end > tile_begin) {
             mbar_wait(done_bar, 0);
             tc_fence_after();
-            if (P.skip_epilogue < 2) {
             // every MMA has completed, so every TMA box has landed and been consumed: the stage ring is free
             float* acc_sm = reinterpret_cast<float*>(ring);
             const int et = threadIdx.x - 64;                                   // 0..127
@@ -237,25 +230,22 @@ __global__ void __launch_bounds__(kThreadsH) conv3d_wgrad_hs_kernel(const __grid
                     asm volatile("bar.sync 1, 128;" ::: "memory");
                 }
             }
-            if (!P.skip_epilogue) {
-                const int per_tap = 16 * P.cin;
-                if (P.tapmajor) {
-                    // S[tap][cout][cin]: the CTA's 16 output channels are per_tap contiguous floats per tap
-                    // (starting every slice's walk at another offset, so that concurrent CTAs hit different lines, measured
-                    // SLOWER: 32 -> 16 97.5 -> 105 us; same-address reductions arriving together combine in L2)
-                    for (int e = et; e < tile_elems; e += 128) {
-                        const int tap = e / per_tap, rem = e - tap * per_tap;
-                        atomicAdd(P.dw + ((int64_t)tap * P.cout + nc * 16) * P.cin + rem, acc_sm[e]);
-                    }
-                } else {
-                    // PyTorch layout [cout][cin][27]
-                    for (int e = et; e < tile_elems; e += 128) {
-                        const int tap = e / per_tap, rem = e - tap * per_tap;
-                        const int co = rem / P.cin, ci = rem - co * P.cin;
-                        atomicAdd(P.dw + ((int64_t)(nc * 16 + co) * P.cin + ci) * 27 + tap, acc_sm[e]);
-                    }
+            const int per_tap = 16 * P.cin;
+            if (P.tapmajor) {
+                // S[tap][cout][cin]: the CTA's 16 output channels are per_tap contiguous floats per tap
+                // (starting every slice's walk at another offset, so that concurrent CTAs hit different lines, measured
+                // SLOWER: 32 -> 16 97.5 -> 105 us; same-address reductions arriving together combine in L2)
+                for (int e = et; e < tile_elems; e += 128) {
+                    const int tap = e / per_tap, rem = e - tap * per_tap;
+                    atomicAdd(P.dw + ((int64_t)tap * P.cout + nc * 16) * P.cin + rem, acc_sm[e]);
                 }
-            }
+            } else {
+                // PyTorch layout [cout][cin][27]
+                for (int e = et; e < tile_elems; e += 128) {
+                    const int tap = e / per_tap, rem = e - tap * per_tap;
+                    const int co = rem / P.cin, ci = rem - co * P.cin;
+                    atomicAdd(P.dw + ((int64_t)(nc * 16 + co) * P.cin + ci) * 27 + tap, acc_sm[e]);
+                }
             }
         }
     }
@@ -280,7 +270,7 @@ struct RsParams {
     int th, tw, planes;            // tile rows (multiple of 6), columns (16 / 32), planes per tile
     int sx, sdy, x_plane, dy_plane, dy_off, stage_bytes, stages;
     int tiles_h, tiles_w, dsteps, tiles_total, split;
-    int tapmajor, skip_epilogue;
+    int tapmajor;
 };
 
 __global__ void __launch_bounds__(kThreadsH) conv3d_wgrad_rs_kernel(const __grid_constant__ CUtensorMap xmap,
@@ -408,13 +398,11 @@ __global__ void __launch_bounds__(kThreadsH) conv3d_wgrad_rs_kernel(const __grid
                     asm volatile("bar.sync 1, 128;" ::: "memory");
                 }
             }
-            if (!P.skip_epilogue) {
-                for (int e = et; e < 1152; e += 128) {
-                    if (P.tapmajor) atomicAdd(P.dw + e, acc_sm[e]);            // S[tap][8][16]
-                    else {
-                        const int tap = e >> 7, co = (e >> 4) & 7, c = e & 15;
-                        atomicAdd(P.dw + (co * 16 + c) * 9 + tap, acc_sm[e]);   // [8][16][1][3][3]
-                    }
+            for (int e = et; e < 1152; e += 128) {
+                if (P.tapmajor) atomicAdd(P.dw + e, acc_sm[e]);            // S[tap][8][16]
+                else {
+                    const int tap = e >> 7, co = (e >> 4) & 7, c = e & 15;
+                    atomicAdd(P.dw + (co * 16 + c) * 9 + tap, acc_sm[e]);   // [8][16][1][3][3]
                 }
             }
         }
@@ -462,13 +450,12 @@ bool fpl_wgrad_hs_eligible(int d, int h, int w, int cin, int cout, int kd, int t
 
 /* returns 0 on launch, > 0 on error (fpl_last_error); the caller has checked fpl_wgrad_hs_eligible */
 int fpl_wgrad_hs_launch(const void* x, int x_c8tot, int x_c8off, const void* dy, int dy_c8tot, int dy_c8off, float* dw, int n,
-                        int d, int h, int w, int cin, int cout, void* stream, int tapmajor, int skip_epilogue, int force_tw, int dbg) {
+                        int d, int h, int w, int cin, int cout, void* stream, int tapmajor) {
     HsParams P;
     P.dw = dw; P.N = n; P.D = d; P.H = h; P.W = w; P.cin = cin; P.cout = cout; P.x_c8off = x_c8off; P.dy_c8off = dy_c8off;
     P.G = cin / 8;
     P.th = h >= 8 ? 8 : ((h + 1) / 2) * 2;
     P.tw = (w >= 32 && P.G == 2) ? 32 : 16;
-    if ((force_tw == 16 || force_tw == 32) && force_tw <= w) P.tw = force_tw;      // tuning knob (fpl_debug_set 15)
     P.sx = (P.tw + 2) * 16; P.sdy = P.tw * 16;
     P.x_bytes = (P.th + 2) * 4 * P.G * P.sx;
     P.dy_bytes = P.th * 4 * P.sdy;
@@ -488,7 +475,7 @@ int fpl_wgrad_hs_launch(const void* x, int x_c8tot, int x_c8off, const void* dy,
     if (split > P.tiles_total) split = P.tiles_total;
     if (split < 1) split = 1;
     P.split = split;
-    P.tapmajor = tapmajor; P.skip_epilogue = skip_epilogue; P.dbg = dbg;
+    P.tapmajor = tapmajor;
     FPL_REQUIRE((reinterpret_cast<uintptr_t>(x) & 15) == 0 && (reinterpret_cast<uintptr_t>(dy) & 15) == 0,
                 "fpl_conv3d_wgrad_tc: x/dy must be 16-byte aligned");
     EncodeTiledFn encode = get_encode_fn();
@@ -510,7 +497,7 @@ bool fpl_wgrad_rs_eligible(int d, int h, int w, int cin, int cout, int kd, int t
 
 /* k(1,3,3), Cin 16, Cout 8 (the head); dw = S[9][8][16] (tapmajor) or [8][16][1][3][3], ACCUMULATED into */
 int fpl_wgrad_rs_launch(const void* x, int x_c8tot, int x_c8off, const void* dy, int dy_c8tot, int dy_c8off, float* dw, int n,
-                        int d, int h, int w, void* stream, int tapmajor, int skip_epilogue) {
+                        int d, int h, int w, void* stream, int tapmajor) {
     RsParams P;
     P.dw = dw; P.N = n; P.D = d; P.H = h; P.W = w; P.x_c8off = x_c8off; P.dy_c8off = dy_c8off;
     P.th = h >= 12 ? 12 : 6;
@@ -531,7 +518,7 @@ int fpl_wgrad_rs_launch(const void* x, int x_c8tot, int x_c8off, const void* dy,
     int split = FPL_NUM_SMS;
     if (split > P.tiles_total) split = P.tiles_total;
     P.split = split;
-    P.tapmajor = tapmajor; P.skip_epilogue = skip_epilogue;
+    P.tapmajor = tapmajor;
     FPL_REQUIRE((reinterpret_cast<uintptr_t>(x) & 15) == 0 && (reinterpret_cast<uintptr_t>(dy) & 15) == 0,
                 "fpl_conv3d_wgrad_tc: x/dy must be 16-byte aligned");
     EncodeTiledFn encode = get_encode_fn();

@@ -19,11 +19,6 @@
 
 namespace {
 
-// debug / tuning knobs (fpl_debug_set keys 10..16)
-int g_wg_hs_dbg = 0;      // key 19: timing experiments of the h-stacked kernel
-int g_wg_hs = 1;          // key 18: h-stacked kernel for Cin 16 / 32 (conv_wgrad_hs.cu)
-int g_wg_swap = 0, g_wg_allow_m64 = 1, g_wg_m64_quadrant = 1, g_wg_allow_pair = 1, g_wg_force_tw = 0, g_wg_tiles_per_cta = 2, g_wg_skip_epilogue = 0;
-
 constexpr int kThreadsW = 192;
 constexpr int kMaxStagesW = 8;
 constexpr int kSmemBudgetW = 220 * 1024;
@@ -43,7 +38,7 @@ struct WgCfg {
     int ncols;             // UMMA N = nb * ndy
 };
 
-bool make_wg_cfg(int h, int w, int cin, int cout, int kd, int allow_m64, int allow_pair, WgCfg& c) {
+bool make_wg_cfg(int h, int w, int cin, int cout, int kd, int allow_pair, WgCfg& c) {
     if (cin % 8 != 0 || (cout % 16 != 0 && cout != 8) || cin <= 0 || cout <= 0) return false;
     c.tw = w >= 32 ? 32 : (w >= 16 ? 16 : 8);
     c.th = h >= 8 ? 8 : ((h + 1) / 2) * 2;
@@ -64,13 +59,12 @@ bool make_wg_cfg(int h, int w, int cin, int cout, int kd, int allow_m64, int all
         c.mtiles_c = g_all / c.c8chunk;
     }
     const int groups = c.nkd * c.c8chunk;
-    c.m = (groups <= 8 && allow_m64) ? 64 : 128;
+    c.m = groups <= 8 ? 64 : 128;
     if (cout == 8 && c.m != 64) return false;          // N = 8 needs the M = 64 shape
     c.nb = cout == 8 ? 8 : ((cout % 32 == 0 && c.ndy == 1) ? 32 : 16);
     c.ncols = c.ndy * c.nb;
     c.nchunks = cout / c.nb;
     if (groups > 8 && c.tw == 32 && cin >= 32 && h * w >= 128 * 128) c.tw = 16;   // keep >= 3 stages at full resolution
-    if (g_wg_force_tw > 0 && g_wg_force_tw <= w) c.tw = g_wg_force_tw;
     c.plane_x = (c.th + 2) * (c.tw + 2) * 16;
     c.plane_dy = c.th * c.tw * 16;
     c.x_bytes = groups * c.plane_x;
@@ -92,16 +86,13 @@ bool make_wg_cfg(int h, int w, int cin, int cout, int kd, int allow_m64, int all
 
 struct WgParams {
     float* dw;
-    float* dump;           // debug: raw accumulators [9][128 lanes][nb] of CTA 0 (may be NULL)
     int N, D, H, W, cin, cout, kd;
     int x_c8off, dy_c8off;
     int th, tw, nkd, c8chunk, mtiles_c, mtiles_kd, m, nb, nchunks;
     int plane_x, plane_dy, x_bytes, dy_off, stage_bytes, stages, tmem_cols;
     int tiles_h, tiles_w, tiles_total, split;
-    int swap_lbo_sbo, m64_quadrant_layout;
     int ndy, ncols, dplanes;       // dplanes: tile index range along depth, ceil(D / ndy)
     int taps;                      // 9, or 1 = only the centre in-plane tap (k = (kd,1,1))
-    int skip_epilogue;             // timing experiments only
     int tapmajor;                  // dW written as [tap][cout][cin] (coalesced atomics; see fpl_wgrad_tapmajor_to_dw_batch)
 };
 
@@ -184,12 +175,8 @@ __global__ void __launch_bounds__(kThreadsW) conv3d_wgrad_tc_kernel(const __grid
         const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | (1u << 15) | (1u << 16) |
                                ((uint32_t)(P.ncols >> 3) << 17) | ((uint32_t)(P.m >> 4) << 24);
         const uint32_t pitch_x = (uint32_t)(P.tw + 2) * 16, pitch_dy = (uint32_t)P.tw * 16;
-        const uint32_t a_lbo = P.swap_lbo_sbo ? (uint32_t)P.plane_x : pitch_x;
-        const uint32_t a_sbo = P.swap_lbo_sbo ? pitch_x : (uint32_t)P.plane_x;
-        const uint32_t b_lbo = P.swap_lbo_sbo ? (uint32_t)P.plane_dy : pitch_dy;
-        const uint32_t b_sbo = P.swap_lbo_sbo ? pitch_dy : (uint32_t)P.plane_dy;
         // descriptors = constant high part + (smem byte address >> 4) in the low 14 bits
-        const uint64_t a_hi = make_desc(0, a_lbo, a_sbo), b_hi = make_desc(0, b_lbo, b_sbo);
+        const uint64_t a_hi = make_desc(0, pitch_x, (uint32_t)P.plane_x), b_hi = make_desc(0, pitch_dy, (uint32_t)P.plane_dy);
         uint32_t tap_off[9];                                  // (kh*pitch + kw*16) >> 4
 #pragma unroll
         for (int t9 = 0; t9 < 9; ++t9) tap_off[t9] = ((uint32_t)(t9 / 3) * pitch_x + (uint32_t)(t9 % 3) * 16) >> 4;
@@ -236,7 +223,7 @@ __global__ void __launch_bounds__(kThreadsW) conv3d_wgrad_tc_kernel(const __grid
         const int T = P.kd * P.taps;
         const int tlane = quarter * 32 + lane;               // TMEM lane this thread reads
         int row;                                             // M row held by that lane
-        if (P.m == 128 || !P.m64_quadrant_layout) row = tlane;
+        if (P.m == 128) row = tlane;
         else row = (lane < 16) ? quarter * 16 + lane : -1;   // M=64: 16 rows per 32-lane quadrant
         bool valid = row >= 0 && row < P.m;
         int kdi = 0, ci = 0;
@@ -251,10 +238,6 @@ __global__ void __launch_bounds__(kThreadsW) conv3d_wgrad_tc_kernel(const __grid
                 uint32_t r[16];
                 tmem_ld16(tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(t9 * P.ncols + c0), r);
                 tmem_ld_wait();
-                if (P.dump != nullptr && blockIdx.x == 0) {
-#pragma unroll
-                    for (int i = 0; i < 16; ++i) P.dump[((int64_t)t9 * 128 + tlane) * P.ncols + c0 + i] = __uint_as_float(r[i]);
-                }
                 // stacked mode: column block dd = col / nb is dy plane ndy*dp+dd, row block kdi is x plane ndy*dp-pad+kdi:
                 // depth tap kd = kdi - dd (the (kdi, dd) blocks of one tap are summed by the atomics).  nb is a multiple
                 // of 8, so each half of the 16 loaded columns lies in one block.
@@ -264,7 +247,7 @@ __global__ void __launch_bounds__(kThreadsW) conv3d_wgrad_tc_kernel(const __grid
                     const int dd = P.ndy > 1 ? col / P.nb : 0;
                     const int kd_tap = P.ndy > 1 ? kdi - dd : kdi;
                     const int co0 = wk.nc * P.nb + (col - dd * P.nb);
-                    if (!(valid && kd_tap >= 0 && kd_tap < P.kd && !P.skip_epilogue)) continue;
+                    if (!(valid && kd_tap >= 0 && kd_tap < P.kd)) continue;
                     if (P.tapmajor) {
                         // lanes = consecutive input channels: one 128-byte line per warp instruction
                         float* base = P.dw + ((int64_t)(kd_tap * P.taps + t9) * P.cout + co0) * P.cin + ci;
@@ -288,8 +271,6 @@ __global__ void __launch_bounds__(kThreadsW) conv3d_wgrad_tc_kernel(const __grid
     }
 }
 
-float* g_wg_dump = nullptr;
-
 CUresult encode_5d(EncodeTiledFn encode, CUtensorMap* map, const void* base, int n, int d, int c8tot, int h, int w,
                    int box_w, int box_h, int box_c8, int box_d) {
     // 8-byte elements (4 bf16 channels) so that a 34-voxel halo row fits the 256-element box limit
@@ -307,36 +288,21 @@ CUresult encode_5d(EncodeTiledFn encode, CUtensorMap* map, const void* base, int
 
 bool fpl_wgrad_hs_eligible(int d, int h, int w, int cin, int cout, int kd, int taps);
 int fpl_wgrad_hs_launch(const void* x, int x_c8tot, int x_c8off, const void* dy, int dy_c8tot, int dy_c8off, float* dw, int n,
-                        int d, int h, int w, int cin, int cout, void* stream, int tapmajor, int skip_epilogue, int force_tw, int dbg);
+                        int d, int h, int w, int cin, int cout, void* stream, int tapmajor);
 bool fpl_wgrad_rs_eligible(int d, int h, int w, int cin, int cout, int kd, int taps);
 int fpl_wgrad_rs_launch(const void* x, int x_c8tot, int x_c8off, const void* dy, int dy_c8tot, int dy_c8off, float* dw, int n,
-                        int d, int h, int w, void* stream, int tapmajor, int skip_epilogue);
-
-// debug knobs (keys 10..18), see fpl_debug_set
-void fpl_wgrad_debug_set(int key, long long value) {
-    if (key == 10) g_wg_swap = (int)value;
-    if (key == 11) g_wg_allow_m64 = (int)value;
-    if (key == 12) g_wg_m64_quadrant = (int)value;
-    if (key == 13) g_wg_dump = reinterpret_cast<float*>(value);
-    if (key == 14) g_wg_allow_pair = (int)value;
-    if (key == 15) g_wg_force_tw = (int)value;
-    if (key == 16) g_wg_tiles_per_cta = (int)value;
-    if (key == 17) g_wg_skip_epilogue = (int)value;
-    if (key == 18) g_wg_hs = (int)value;
-    if (key == 19) g_wg_hs_dbg = (int)value;
-}
+                        int d, int h, int w, void* stream, int tapmajor);
 
 static int wgrad_tc_launch(const void* x, int x_c8tot, int x_c8off, const void* dy, int dy_c8tot, int dy_c8off,
                            float* dw, int n, int d, int h, int w, int cin, int cout, int kd, int taps, void* stream,
                            int tapmajor = 0) {
     FPL_REQUIRE(kd == 1 || kd == 3, "fpl_conv3d_wgrad_tc: kd=%d must be 1 or 3", kd);
-    if (g_wg_hs && fpl_wgrad_hs_eligible(d, h, w, cin, cout, kd, taps))
-        return fpl_wgrad_hs_launch(x, x_c8tot, x_c8off, dy, dy_c8tot, dy_c8off, dw, n, d, h, w, cin, cout, stream, tapmajor,
-                                   g_wg_skip_epilogue, g_wg_force_tw, g_wg_hs_dbg);
-    if (g_wg_hs && fpl_wgrad_rs_eligible(d, h, w, cin, cout, kd, taps))
-        return fpl_wgrad_rs_launch(x, x_c8tot, x_c8off, dy, dy_c8tot, dy_c8off, dw, n, d, h, w, stream, tapmajor, g_wg_skip_epilogue);
+    if (fpl_wgrad_hs_eligible(d, h, w, cin, cout, kd, taps))
+        return fpl_wgrad_hs_launch(x, x_c8tot, x_c8off, dy, dy_c8tot, dy_c8off, dw, n, d, h, w, cin, cout, stream, tapmajor);
+    if (fpl_wgrad_rs_eligible(d, h, w, cin, cout, kd, taps))
+        return fpl_wgrad_rs_launch(x, x_c8tot, x_c8off, dy, dy_c8tot, dy_c8off, dw, n, d, h, w, stream, tapmajor);
     WgCfg c;
-    FPL_REQUIRE(make_wg_cfg(h, w, cin, cout, kd, g_wg_allow_m64, g_wg_allow_pair && d >= 2, c),
+    FPL_REQUIRE(make_wg_cfg(h, w, cin, cout, kd, d >= 2, c),
                 "fpl_conv3d_wgrad_tc: unsupported shape (cin %d, cout %d, %dx%d)", cin, cout, h, w);
     FPL_REQUIRE((reinterpret_cast<uintptr_t>(x) & 15) == 0 && (reinterpret_cast<uintptr_t>(dy) & 15) == 0,
                 "fpl_conv3d_wgrad_tc: x/dy must be 16-byte aligned");
@@ -348,7 +314,7 @@ static int wgrad_tc_launch(const void* x, int x_c8tot, int x_c8off, const void* 
     r = encode_5d(encode, &dymap, dy, n, d, dy_c8tot, h, w, c.tw, c.th, c.nb / 8, c.ndy);
     FPL_REQUIRE(r == CUDA_SUCCESS, "fpl_conv3d_wgrad_tc: tensor map (dy) failed (%d)", (int)r);
     WgParams P;
-    P.dw = dw; P.dump = g_wg_dump;
+    P.dw = dw;
     P.N = n; P.D = d; P.H = h; P.W = w; P.cin = cin; P.cout = cout; P.kd = kd;
     P.x_c8off = x_c8off; P.dy_c8off = dy_c8off;
     P.th = c.th; P.tw = c.tw; P.nkd = c.nkd; P.c8chunk = c.c8chunk; P.mtiles_c = c.mtiles_c; P.mtiles_kd = c.mtiles_kd;
@@ -360,14 +326,14 @@ static int wgrad_tc_launch(const void* x, int x_c8tot, int x_c8off, const void* 
     FPL_REQUIRE(tiles < (1ll << 30), "fpl_conv3d_wgrad_tc: too many tiles");
     P.tiles_total = (int)tiles;
     const int pairs = c.mtiles_kd * c.mtiles_c * c.nchunks;
-    // split-K over voxel tiles: every CTA ends with 9*128*N atomics into dW, so a slice should own >= 2 tiles (measured: tools/wgrad_tune.py)
+    // split-K over voxel tiles: every CTA ends with 9*128*N atomics into dW, so a slice should own >= 2 tiles (measured
+    // with a tuning tool that has since been removed)
     // (deep levels: few tiles, many (M,N) pairs -> split 1; full resolution: one CTA per SM)
     int split = FPL_NUM_SMS / pairs;
-    if (split > P.tiles_total / g_wg_tiles_per_cta) split = P.tiles_total / g_wg_tiles_per_cta;
+    if (split > P.tiles_total / 2) split = P.tiles_total / 2;
     if (split < 1) split = 1;
     P.split = split;
-    P.swap_lbo_sbo = g_wg_swap; P.m64_quadrant_layout = g_wg_m64_quadrant;
-    P.taps = taps; P.skip_epilogue = g_wg_skip_epilogue; P.tapmajor = tapmajor;
+    P.taps = taps; P.tapmajor = tapmajor;
     FPL_CHECK_CUDA(cudaFuncSetAttribute(conv3d_wgrad_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, c.smem_bytes));
     fpl_launch(conv3d_wgrad_tc_kernel, pairs * split, kThreadsW, c.smem_bytes, (cudaStream_t)stream, xmap, dymap, P);
     FPL_LAUNCH_CHECK();

@@ -6,11 +6,6 @@
 #include "common.cuh"
 #include "../../include/fplplus_b200.h"
 
-#ifndef FPL_BWD_V
-#define FPL_BWD_V 2
-#define FPL_BWD_BLOCKS 4
-#endif
-
 namespace {
 
 constexpr int kThreads = 256;
@@ -296,7 +291,6 @@ struct ActBwdParams {
     double inv_count;
     int N, D, C8, H, W;
     int w_shift;                // log2(W) when W is a power of two, else -1
-    int reverse;                // apply pass: walk the work items from the END (see dsbn_act_bwd_kernel)
 };
 
 // grid: (blocks per channel group, C8).  A block stays inside one channel group (its per-channel constants live in
@@ -306,8 +300,8 @@ struct ActBwdParams {
 //   reduce: accumulates sum dz, sum dz*y (raw conv output; turned into sum dz*xhat per block in double) and dslope
 //   apply : dy = sc*(dz - m1 - xhat*m2)  rewritten as  sc*dz + cb + cy*y  (cb, cy per channel)
 // __launch_bounds__(256, 4): <= 64 registers, 1024 threads per SM keep >= 64 KB of loads in flight.
-constexpr int kBwdV = FPL_BWD_V;          // vectors per thread per work item
-constexpr int kBwdBlocks = FPL_BWD_BLOCKS; // resident blocks per SM the register budget is tuned for
+constexpr int kBwdV = 2;                  // vectors per thread per work item
+constexpr int kBwdBlocks = 4;             // resident blocks per SM the register budget is tuned for
 template <bool APPLY, bool POOL, bool DROP>
 __global__ void __launch_bounds__(kThreads, kBwdBlocks) dsbn_act_bwd_kernel(const __grid_constant__ ActBwdParams P) {
     FPL_PDL_WAIT();      // everything below may read what earlier kernels of the stream wrote
@@ -353,19 +347,15 @@ __global__ void __launch_bounds__(kThreads, kBwdBlocks) dsbn_act_bwd_kernel(cons
     const int W2 = P.W >> 1, HW2 = (P.H >> 1) * W2;
     // (nd, ch) = divmod(item, chunks) and the plane base pointers are stepped, not recomputed (no division and no
     // 64-bit multiply chains in the loop)
-    // Option (fpl_debug_set 31): the APPLY pass walks its items from the END, so that it starts on the part of y / g the
-    // reduce pass streamed last (still in L2).  Measured neutral in the two-stream step: the other domain's kernels own L2.
     const int step_nd = gridDim.x / chunks, step_ch = gridDim.x - step_nd * chunks;
-    const bool rev = APPLY && P.reverse && (int)blockIdx.x < items;
-    const int first = rev ? (int)blockIdx.x + ((items - 1 - (int)blockIdx.x) / (int)gridDim.x) * (int)gridDim.x : (int)blockIdx.x;
-    int nd = first / chunks, ch = first - nd * chunks;
+    int nd = blockIdx.x / chunks, ch = blockIdx.x - nd * chunks;
     const int64_t y_stride = (int64_t)P.C8 * HW, g_stride = (int64_t)P.g1_c8tot * HW;
     const bf16x8* yp = P.y + ((int64_t)nd * P.C8 + c8) * HW + threadIdx.x;
     const bf16x8* g1p = P.g1 != nullptr ? P.g1 + ((int64_t)nd * P.g1_c8tot + P.g1_c8off + c8) * HW + threadIdx.x : nullptr;
     const int64_t dy_off = APPLY ? reinterpret_cast<const char*>(P.dy) - reinterpret_cast<const char*>(P.y) : 0;
     int pn = 0, pd = 0;          // POOL: (n, d) of plane nd
     if (POOL) { pn = nd / P.D; pd = nd - pn * P.D; }
-    for (int item = first; item >= 0 && item < items; item += rev ? -(int)gridDim.x : (int)gridDim.x) {
+    for (int item = blockIdx.x; item < items; item += gridDim.x) {
         const bf16x8* gpp = nullptr;
         const uint2* idxp = nullptr;
         uint32_t code_d = 0;
@@ -444,22 +434,14 @@ __global__ void __launch_bounds__(kThreads, kBwdBlocks) dsbn_act_bwd_kernel(cons
                 st_bf16x8(const_cast<char*>(reinterpret_cast<const char*>(yp + voff + k * kThreads)) + dy_off, o);
         }
         // next item
-        int dnd;
-        if (!rev) {
-            dnd = step_nd;
-            ch += step_ch;
-            if (ch >= chunks) { ch -= chunks; ++dnd; }
-        } else {
-            dnd = -step_nd;
-            ch -= step_ch;
-            if (ch < 0) { ch += chunks; --dnd; }
-        }
+        int dnd = step_nd;
+        ch += step_ch;
+        if (ch >= chunks) { ch -= chunks; ++dnd; }
         yp += dnd * y_stride;
         if (g1p != nullptr) g1p += dnd * g_stride;
         if (POOL) {
             pd += dnd;
             while (pd >= P.D) { pd -= P.D; ++pn; }
-            while (pd < 0) { pd += P.D; --pn; }
         }
     }
     FPL_PDL_TRIGGER();       // main loop done: the next kernel of the stream may be scheduled as blocks drain
@@ -514,13 +496,7 @@ __global__ void dsbn_bwd_finalize_kernel(const double* __restrict__ red, const f
 
 }  // namespace
 
-static int g_bwd_blocks_per_sm = 8;   // tuning knob (fpl_debug_set key 30)
-int g_bwd_reverse_apply = 0;    // fpl_debug_set 31: measured neutral in the overlapped step (4.346 / 4.339 vs 4.340 / 4.341 ms), off
-
-void fpl_dsbn_debug_set(int key, long long value) {
-    if (key == 30 && value > 0) g_bwd_blocks_per_sm = (int)value;
-    if (key == 31) g_bwd_reverse_apply = (int)value;
-}
+constexpr int g_bwd_blocks_per_sm = 8;
 
 extern "C" int fpl_dsbn_finalize(const double* stats, int64_t count, const float* gamma, const float* beta,
                                  float* running_mean, float* running_var, int64_t* num_batches_tracked,
@@ -627,7 +603,6 @@ static int fill_bwd(ActBwdParams& P, const void* y, const void* g1, int g1_c8tot
     P.N = n; P.D = d; P.C8 = c / 8; P.H = h; P.W = w;
     P.w_shift = -1;
     for (int s = 0; s < 16; ++s) if ((1 << s) == w) P.w_shift = s;
-    P.reverse = g_bwd_reverse_apply;
     return 0;
 }
 

@@ -35,7 +35,6 @@ struct HtParams {
     int a_bytes, stages;
     int mstride, tmem_cols;    // accumulator columns per M tile (32 when nb <= 32: two CTAs per SM), TMEM allocation
     int tiles_h, tiles_w, total_tiles;
-    int dbg;                   // timing experiments (fpl_debug_set 51): 1 = no stores, 2 = no epilogue work
 };
 
 __device__ __forceinline__ void tmem_ld2(uint32_t taddr, uint32_t& a, uint32_t& b) {
@@ -165,10 +164,11 @@ __global__ void __launch_bounds__(kHtThreads) head_fwd_tc_kernel(const __grid_co
             const int w = tw * kHtOutCols + lane - 1;                       // lanes 0 / 31 are the halo columns
             const bool col_ok = lane >= 1 && lane <= kHtOutCols && w < P.W;
 #pragma unroll 1
-            for (int m = pair; m < 4 && !(P.dbg & 2); m += 2) {
+            for (int m = pair; m < 4; m += 2) {
                 const int h = th * kHtOutRows + 4 * m + quarter;
                 const uint32_t taddr = lane_base + (uint32_t)((acc * 4 + m) * P.mstride);
                 float* out = P.logits + (((int64_t)n * C) * P.D + dd) * HW + (int64_t)h * P.W + w;
+                const bool in_bounds = col_ok && h < P.H;
                 if (C == 2) {                                              // the shipped configurations
                     uint32_t v[16], v16, v17;
                     tmem_ld16(taddr, v);
@@ -186,7 +186,7 @@ __global__ void __launch_bounds__(kHtThreads) head_fwd_tc_kernel(const __grid_co
                         const float left = __shfl_up_sync(0xffffffffu, q[cls], 1);          // Q[u-1][kw=0]
                         const float right = __shfl_down_sync(0xffffffffu, q[4 + cls], 1);   // Q[u+1][kw=2]
                         const float y = __ldg(P.bias + cls) + left + q[2 + cls] + right;
-                        if (col_ok && h < P.H && !(P.dbg & 1)) out[(int64_t)cls * P.D * HW] = y;
+                        if (in_bounds) out[(int64_t)cls * P.D * HW] = y;
                     }
                 } else {
                     for (int cls = 0; cls < C; ++cls) {
@@ -205,7 +205,7 @@ __global__ void __launch_bounds__(kHtThreads) head_fwd_tc_kernel(const __grid_co
                         const float left = __shfl_up_sync(0xffffffffu, q[0], 1);
                         const float right = __shfl_down_sync(0xffffffffu, q[2], 1);
                         const float y = __ldg(P.bias + cls) + left + q[1] + right;
-                        if (col_ok && h < P.H && !(P.dbg & 1)) out[(int64_t)cls * P.D * HW] = y;
+                        if (in_bounds) out[(int64_t)cls * P.D * HW] = y;
                     }
                 }
             }
@@ -442,25 +442,17 @@ __global__ void __launch_bounds__(kHdThreads) head_dgrad_tc_kernel(HdParams P) {
     }
 }
 
-int g_head_tc = 1;      // fpl_debug_set 50: tensor-core head forward on / off
-int g_head_tc_dbg = 0;  // fpl_debug_set 51
-
 }  // namespace
 
-void fpl_head_tc_debug_set(int key, long long value) {
-    if (key == 50) g_head_tc = (int)value;
-    if (key == 51) g_head_tc_dbg = (int)value;
-}
-
 bool fpl_head_fwd_tc_eligible(int h, int w, int cin, int classes) {
-    return g_head_tc && cin % 16 == 0 && cin >= 16 && cin <= 64 && classes >= 1 && classes <= 7 && h >= 4 && w >= 32 && (cin == 16 || cin == 32);     // 9 * classes <= 64 accumulator columns per M tile
+    return cin % 16 == 0 && cin >= 16 && cin <= 64 && classes >= 1 && classes <= 7 && h >= 4 && w >= 32 && (cin == 16 || cin == 32);     // 9 * classes <= 64 accumulator columns per M tile
 }
 
 int fpl_head_fwd_tc_launch(const void* x, int x_c8tot, int x_c8off, const float* w, const float* bias, float* logits, int n, int d,
                            int h, int w_, int cin, int classes, void* stream) {
     HtParams P;
     P.w = w; P.bias = bias; P.logits = logits; P.N = n; P.D = d; P.H = h; P.W = w_; P.cin = cin; P.classes = classes;
-    P.x_c8off = x_c8off; P.dbg = g_head_tc_dbg;
+    P.x_c8off = x_c8off;
     P.nb = ((9 * classes + 15) / 16) * 16;
     P.a_bytes = (cin / 8) * kHtPlane;
     const int b_bytes = ((3 * (cin / 8) * P.nb * 16 + 127) / 128) * 128;
@@ -501,7 +493,7 @@ int fpl_head_fwd_tc_launch(const void* x, int x_c8tot, int x_c8off, const float*
 }
 
 bool fpl_head_dgrad_tc_eligible(int h, int w, int cin, int classes) {
-    return g_head_tc && (cin == 16 || cin == 32) && classes >= 1 && classes <= 2 && h >= 4 && w >= 32;
+    return (cin == 16 || cin == 32) && classes >= 1 && classes <= 2 && h >= 4 && w >= 32;
 }
 
 int fpl_head_dgrad_tc_launch(const float* dlogits, const float* w, void* g, int g_c8tot, int g_c8off, void* dl8, int dl_c8tot,

@@ -312,17 +312,6 @@ int resident_blocks(K kernel) {
     return cached;
 }
 
-// groups per thread and batch of the two-class uint8 kernels: 8 (one wave of two register-heavy blocks per SM, one DRAM
-// round trip) or, FPL_LOSS_BATCH=2, 2 (four blocks per SM, two round trips, more warps to hide the exp / log chains)
-int loss_batch() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("FPL_LOSS_BATCH");
-        v = (e != nullptr && atoi(e) == 2) ? 2 : 8;
-    }
-    return v;
-}
-
 // blocks per sample: every thread one batch of U groups, capped at `per_sm` resident blocks per SM over the whole grid
 int grid_x_for(int64_t s4, int n, int u, int per_sm) {
     int64_t bx = (s4 + (int64_t)kThreads * u - 1) / ((int64_t)kThreads * u);
@@ -357,10 +346,6 @@ static int dice_ce_reduce_launch(const float* logits, const LossSrc& src, double
     if (c == 2 && lean) {
         // two classes, uint8 inputs: ONE wave of two 256-thread blocks per SM, every thread one batch of up to 8 groups
         // (~140 KB of loads in flight per SM = the bandwidth-delay product: one DRAM round trip per launch)
-        if (loss_batch() == 2)
-            fpl_launch(dice_ce_reduce_kernel<2, 2, true>, dim3(grid_x_for(s4, n, 2, resident_blocks(dice_ce_reduce_kernel<2, 2, true>)), n), kThreads, 0,
-                       (cudaStream_t)stream, logits, src, sums, n, s4, want_entropy);
-        else
         fpl_launch(dice_ce_reduce_kernel<2, 8, true>, dim3(grid_x_for(s4, n, 8, resident_blocks(dice_ce_reduce_kernel<2, 8, true>)), n), kThreads, 0,
                    (cudaStream_t)stream, logits, src, sums, n, s4, want_entropy);
     } else if (lean) {
@@ -387,13 +372,6 @@ static int dice_ce_grad_launch(const float* logits, const LossSrc& src, const do
     const bool lean = src.soft_y == nullptr && src.weight == nullptr;
     const int gy = dlogits != nullptr ? n : 1;
     if (c == 2 && lean) {
-        if (loss_batch() == 2) {
-            const dim3 grid2(dlogits != nullptr ? grid_x_for(s4, n, 2, resident_blocks(dice_ce_grad_kernel<2, 2, true>)) : 1, gy);
-            fpl_launch(dice_ce_grad_kernel<2, 2, true>, grid2, kThreads, 0, (cudaStream_t)stream, logits, src, sums, w_dice, w_ce, w_ent,
-                       grad_scale, grad_scale_dev, loss, dlogits, n, s4, n_global, hard_dice);
-            FPL_LAUNCH_CHECK();
-            return 0;
-        }
         const dim3 grid(dlogits != nullptr ? grid_x_for(s4, n, 8, resident_blocks(dice_ce_grad_kernel<2, 8, true>)) : 1, gy);
         fpl_launch(dice_ce_grad_kernel<2, 8, true>, grid, kThreads, 0, (cudaStream_t)stream, logits, src, sums, w_dice, w_ce, w_ent,
                    grad_scale, grad_scale_dev, loss, dlogits, n, s4, n_global, hard_dice);

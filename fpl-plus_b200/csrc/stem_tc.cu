@@ -483,8 +483,6 @@ __global__ void __launch_bounds__(kSwThreads) stem_wgrad_tc_kernel(const __grid_
     }
 }
 
-int g_stem_tc = 1;      // fpl_debug_set 52
-
 StemGeo stem_geo(int n, int d, int h, int w) {
     StemGeo G;
     G.N = n; G.D = d; G.H = h; G.W = w;
@@ -495,12 +493,8 @@ StemGeo stem_geo(int n, int d, int h, int w) {
 
 }  // namespace
 
-void fpl_stem_tc_debug_set(int key, long long value) {
-    if (key == 52) g_stem_tc = (int)value;
-}
-
 bool fpl_stem_tc_eligible(int n, int cin, int d, int h, int w, int cout, int kd) {
-    return g_stem_tc && cin == 1 && cout == 16 && kd == 3 && w >= 32 && h >= 4 && (int64_t)n * d * ((h + 15) / 16) * ((w + 31) / 32) < (1 << 30);
+    return cin == 1 && cout == 16 && kd == 3 && w >= 32 && h >= 4 && (int64_t)n * d * ((h + 15) / 16) * ((w + 31) / 32) < (1 << 30);
 }
 
 int fpl_stem_fwd_tc_launch(const float* x, const float* w, const float* bias, void* y, int y_c8tot, int y_c8off, double* stats, int n,

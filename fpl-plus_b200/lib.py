@@ -4,7 +4,6 @@ There is deliberately no fallback: if the library is missing it is built with nv
 that is impossible the import fails loudly.
 """
 import ctypes
-import os
 from ctypes import c_char_p, c_double, c_float, c_int, c_int64, c_longlong, c_uint64, c_void_p
 
 from . import build as _build
@@ -21,7 +20,6 @@ _SIGNATURES = {
     "fpl_set_sm_budget": (_I, [_I]),
     "fpl_launch_count": (c_longlong, [_I]),
     "fpl_device_is_sm100": (_I, []),
-    "fpl_debug_set": (None, [_I, c_longlong]),
     "fpl_conv3d_weight_image_bytes": (_L, [_I, _I, _I]),
     "fpl_conv3d_prep_weight": (_I, [_P, _I, _I, _I, _I, _P, _P]),
     "fpl_conv3d_prep_weight_batch": (_I, [_I, ctypes.POINTER(c_void_p), ctypes.POINTER(_I), ctypes.POINTER(_I),
@@ -97,7 +95,7 @@ _SIGNATURES = {
 }
 
 #: every symbol include/fplplus_b200.h declares (tests check the .so exports them all)
-EXPORTED = [k for k in _SIGNATURES if k != "fpl_debug_set"]
+EXPORTED = list(_SIGNATURES)
 
 _lib = None
 
@@ -115,11 +113,6 @@ def load():
             fn = getattr(lib, name)
             fn.restype = res
             fn.argtypes = args
-        # A/B switches of the tuning knobs (fpl_debug_set): FPL_DEBUG_SET="18=0,16=4" ...
-        for item in os.environ.get("FPL_DEBUG_SET", "").split(","):
-            if "=" in item:
-                k, v = item.split("=", 1)
-                lib.fpl_debug_set(int(k), int(v))
         _lib = lib
     return _lib
 
@@ -134,19 +127,8 @@ def set_call_timer(fn):
     _call_timer = fn
 
 
-#: profiling only (tools/marginal_cost.sh): entry points named in FPL_DEBUG_SKIP are not launched, which shows what a
-#: kernel class costs in the overlapped schedule of the real step.  Results are WRONG with it set; never set it otherwise.
-_debug_skip = frozenset(n for n in os.environ.get("FPL_DEBUG_SKIP", "").split(",") if n)
-if _debug_skip:
-    import sys as _sys
-    print("fplplus_b200: FPL_DEBUG_SKIP is set -- %d entry points are NOT launched; results are wrong (profiling only)"
-          % len(_debug_skip), file=_sys.stderr)
-
-
 def call(name, *args):
     """Invoke a C-ABI function; a non-zero status raises FplError with the library's message."""
-    if _debug_skip and name in _debug_skip:
-        return
     lib = load()
     tok = _call_timer(name, args) if _call_timer is not None else None
     rc = getattr(lib, name)(*args)

@@ -37,16 +37,6 @@ int fpl_set_sm_budget(int sms);
 long long fpl_launch_count(int reset);
 /* 1 when the running device is sm_100 (tcgen05 kernels usable), else 0. */
 int fpl_device_is_sm100(void);
-/* debugging / tuning knobs, used by tools/*_probe.py and tools/*_tune.py only (defaults are the measured optima):
- *   0  swap LBO/SBO of the fwd UMMA descriptors        1  allow the N split of staged weight slices (conv3d_tc)
- *  10  swap LBO/SBO in wgrad   11  allow UMMA M=64 in wgrad   12  M=64 TMEM lane layout   13  raw-accumulator dump pointer
- *  14  allow depth-stacked wgrad tiles   15  force the wgrad tile width   16  minimum voxel tiles per split-K slice
- *  17  skip the wgrad epilogue (timing only: results are wrong)          30  DSBN backward blocks per SM   31  DSBN backward apply pass from the end
- *  18  h-stacked / row-stacked wgrad kernels (conv_wgrad_hs.cu) on / off   19  their timing experiments (no MMAs / no loads)
- *  40..48  depth-folded conv: CTAs per SM, planes per chunk, epilogue / MMA / TMA-box timing experiments, stages,
- *          planes per TMA box, split tail chunks (tools/dfold_knob_probe.py; results are wrong under 42 / 44 / 45)
- *  50  tensor-core head forward / dgrad (head_tc.cu) on / off   51  their timing experiments */
-void fpl_debug_set(int key, long long value);
 
 /* ---- (a) conv3d: PyMIC/pymic/net/net3d/unet2d5_dsbn.py:75,79 (nn.Conv3d k3 p1 / k(1,3,3) p(0,1,1)) ---- */
 

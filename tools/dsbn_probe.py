@@ -6,18 +6,15 @@ import sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
 
-from fplplus_b200 import lib, ops
+from fplplus_b200 import ops
 
 DEV = "cuda:0"
-L = lib.load()
 p = ops.ptr
 # (channels, (n, d, h, w), pooled?)
 SHAPES = [(16, (4, 32, 128, 128), 0), (16, (4, 32, 128, 128), 2), (32, (4, 16, 64, 64), 0), (32, (4, 16, 64, 64), 2),
           (64, (4, 8, 32, 32), 0), (64, (4, 8, 32, 32), 2), (128, (4, 4, 16, 16), 0), (256, (4, 2, 8, 8), 0)]
 REPS = int(os.environ.get("REPS", "5"))
 ONLY = os.environ.get("ONLY", "")
-if os.environ.get("BPS"):
-    L.fpl_debug_set(30, int(os.environ["BPS"]))
 
 
 def timeit(fn):

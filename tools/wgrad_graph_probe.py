@@ -1,16 +1,15 @@
 """GPU probe: every wgrad launch of the bench network (batch 4), captured 10x back to back in a CUDA graph (no host
 enqueue gaps, warm L2) -- the per-launch GPU time the graph-replayed train step pays.  Development tool.
-Usage: python tools/wgrad_graph_probe.py [FN]"""
+Usage: python tools/wgrad_graph_probe.py"""
 import os
 import sys
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
 
-from fplplus_b200 import lib, ops
+from fplplus_b200 import ops
 
 DEV = "cuda:0"
-L = lib.load()
 SHAPES = [(16, 8, 1, (4, 32, 128, 128), 1), (16, 16, 3, (4, 32, 128, 128), 2), (32, 16, 3, (4, 32, 128, 128), 1),
           (16, 32, 3, (4, 16, 64, 64), 1), (32, 32, 3, (4, 16, 64, 64), 2), (64, 32, 3, (4, 16, 64, 64), 1),
           (32, 64, 3, (4, 8, 32, 32), 1), (64, 64, 3, (4, 8, 32, 32), 2), (128, 64, 3, (4, 8, 32, 32), 1),
@@ -42,11 +41,8 @@ def graph_time(fn, iters=10):
 
 def main():
     fn_name = "fpl_conv3d_wgrad_tc_tapmajor"
-    for kv in sys.argv[1:]:          # debug knobs as key=value (fpl_debug_set), e.g. 18=0 (old kernel), 15=16, 17=1
-        k, v = kv.split("=")
-        L.fpl_debug_set(int(k), int(v))
     total = 0.0
-    print("%-30s %9s %9s %9s  (%s %s)" % ("layer", "us", "TFLOP/s", "x/pass", fn_name, " ".join(sys.argv[1:])))
+    print("%-30s %9s %9s %9s  (%s)" % ("layer", "us", "TFLOP/s", "x/pass", fn_name))
     for cin, cout, kd, shape, count in SHAPES:
         n, d, h, w = shape
         x = torch.randn((n, d, cin // 8, h, w, 8), device=DEV).to(torch.bfloat16)
