@@ -23,9 +23,12 @@ What is different underneath (B200-first, SURVEY.md §8):
   syncs per step, agent_seg.py:476,495);
 * the FPL statistics / pseudo labels / agreement weights stay on the device (csrc/filter.cu); only
   the uint8 label volume or two scalars per volume come back to the host;
-* file I/O (NIfTI through SimpleITK) and the CPU transform pipeline are out of scope: loaders are
-  any iterables of batch dicts (``set_loaders`` / ``set_datasets``); ``NpyVolumeDataset`` is the
-  minimal built-in for ``.npy`` volumes.
+* the CPU transform pipeline is replaced: without ``set_loaders`` / ``set_datasets``, a training
+  run builds one ``DevicePatchSampler`` per domain from ``[dataset] {1,2}_train_csv`` and
+  ``train_transform`` (datapath.py: volumes resident in HBM, RandomCrop / RandomFlip /
+  NormalizeWithMeanStd per step on the device); otherwise loaders are any iterables of batch dicts,
+  validation and test loaders always so; ``NpyVolumeDataset`` is the minimal built-in for ``.npy``
+  / ``.nii`` volumes.
 
 As in the reference only ``training_all`` semantics train (``training()`` of the shipped
 ``dual=False`` cfgs has no ``backward()``; SURVEY.md §3.1): ``dual`` is accepted and both values
@@ -296,11 +299,8 @@ class NpyVolumeDataset(torch.utils.data.Dataset):
         return len(self.rows)
 
     def _load(self, rel):
-        path = os.path.join(self.root, rel)
-        if path.endswith(('.nii.gz', '.nii')):
-            from . import artefacts
-            return artefacts.load_nifty_volume_as_4d_array(path)['data_array'][0]
-        return np.load(path)
+        from . import artefacts
+        return artefacts.load_volume(os.path.join(self.root, rel))
 
     def __getitem__(self, i):
         row = self.rows[i]
@@ -416,9 +416,17 @@ class SegmentationAgent(object):
 
     def create_dataset(self):
         """agent_abstract.py:241-318: loaders come from set_loaders(), or are wrapped around the
-        datasets given to set_datasets() with the cfg's batch sizes."""
-        bs = self.config.get('dataset', {}).get('train_batch_size', 1)
+        datasets given to set_datasets() with the cfg's batch sizes.  With neither, the training loaders are
+        ``DevicePatchSampler``s built from ``[dataset] {1,2}_train_csv`` and ``train_transform``
+        (``datapath.samplers_from_config``): the volumes stay on the training GPU."""
+        ds = self.config.get('dataset', {})
+        bs = ds.get('train_batch_size', 1)
         if self.stage == 'train':
+            if (self.train_loaders[0] is None and self.train_set is None
+                    and (ds.get('1_train_csv') or ds.get('2_train_csv'))):
+                from .datapath import samplers_from_config
+                self.train_loaders = samplers_from_config(self.config, self._pick_device('training'), self.rank,
+                                                          self.world)
             if self.train_loaders[0] is None and self.train_set is not None:
                 sets = self.train_set if isinstance(self.train_set, (list, tuple)) else [self.train_set]
 

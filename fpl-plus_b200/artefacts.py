@@ -168,6 +168,14 @@ def load_image_as_nd_array(image_name):
     raise ValueError("unsupported image format")
 
 
+def load_volume(path):
+    """One volume of a training-CSV row: a ``.npy`` array as stored, or the [D,H,W] data of a ``.nii`` / ``.nii.gz``
+    file (``NpyVolumeDataset`` and ``datapath.load_train_csv``)."""
+    if path.endswith(('.nii.gz', '.nii')):
+        return load_nifty_volume_as_4d_array(path)['data_array'][0]
+    return np.load(path)
+
+
 def save_array_as_nifty_volume(data, image_name, reference_name=None):
     """image_read_write.py:92-108: [D,H,W] array, geometry copied from ``reference_name`` when given."""
     meta = {}

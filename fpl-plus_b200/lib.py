@@ -79,6 +79,9 @@ _SIGNATURES = {
                                + [_I] * 5 + [_P]),
     "fpl_dsbn_bwd_finalize": (_I, [_P, _P, _P, _I, _P, _P, _P, _P, _I, _P]),
     "fpl_gather_patches": (_I, [_P, _I, _I, _I, _I, _I, _P, _P, _P, _P]),
+    "fpl_gather_patches_norm_workspace_bytes": (_L, [_I] * 5),
+    "fpl_gather_patches_norm": (_I, [_P, _I, _I, _I, _I, _I, ctypes.POINTER(_I), ctypes.POINTER(_F), ctypes.POINTER(_F), _P,
+                                     _L, _P, _P, _P, _P]),
     "fpl_adam_multi_tensor": (_I, [_P, _I, _P, _I, _P, c_double, c_double, c_double, c_double, c_double, _P, _P]),
     "fpl_adam_chunk_elems": (_I, []),
     "fpl_dice_ce_reduce": (_I, [_P, _P, _P, _P, _I, _I, _L, _P]),

@@ -129,6 +129,18 @@ int fpl_grad_scatter_add(float* dst, const float* src, const int* d_table, int s
 int fpl_gather_patches(const void* d_rows, int n, int c, int pd, int ph, int pw, float* out_image,
                        uint8_t* out_label, uint8_t* out_code, void* stream);
 
+/* fpl_gather_patches followed by NormalizeWithMeanStd of each cut patch (transform/normalize.py applied after RandomCrop).
+ * h_mode, h_mean, h_std: HOST arrays of c entries (c <= 16).  h_mode[i]: 0 = channel i is copied raw; 1 = (x - h_mean[i]) /
+ * h_std[i]; 2 = mean / population std of the channel over the patch; 3 = the same over the patch's voxels > 0 (over the
+ * whole patch when it has none).  The std of modes 2 / 3 is floored at 1e-8; h_mean / h_std are read for mode 1 only
+ * (may be NULL otherwise).  The statistics are fp64 sums written per block into `workspace` (8-byte aligned, at least
+ * fpl_gather_patches_norm_workspace_bytes(n, c, pd, ph, pw) bytes; may be NULL when no channel has mode 2 or 3) and
+ * reduced in a fixed order, so the batch is bitwise reproducible.  Label and code outputs as fpl_gather_patches. */
+int64_t fpl_gather_patches_norm_workspace_bytes(int n, int c, int pd, int ph, int pw);
+int fpl_gather_patches_norm(const void* d_rows, int n, int c, int pd, int ph, int pw, const int* h_mode, const float* h_mean,
+                            const float* h_std, void* workspace, int64_t workspace_bytes, float* out_image,
+                            uint8_t* out_label, uint8_t* out_code, void* stream);
+
 /* ---- optimiser: torch.optim.Adam(params, lr, weight_decay=wd) of net_run/get_optimizer.py:16-17 (coupled L2) ----------
  * ONE launch over all tensors.  d_segs: DEVICE table of nseg rows of 48 bytes
  *   { float* param; const float* grad; float* exp_avg; float* exp_avg_sq; float* step; int32 numel; int32 pad }
