@@ -35,6 +35,46 @@ def randn(seed, *shape, scale=1.0):
     return torch.from_numpy((rng(seed).standard_normal(shape) * scale).astype(np.float32))
 
 
+_M32 = np.uint64(0xFFFFFFFF)
+
+
+def philox4x32_10(ctr, key):
+    """Philox4x32-10 (Salmon et al., Random123) on the host, as csrc/common.cuh computes it.  ctr: integer array
+    [..., 4] of 32-bit words, key: [..., 2]; returns uint64 [..., 4] holding the 32-bit output words."""
+    ctr = np.asarray(ctr, dtype=np.uint64)
+    key = np.asarray(key, dtype=np.uint64)
+    x0, x1, x2, x3 = (ctr[..., i] for i in range(4))
+    k0, k1 = key[..., 0], key[..., 1]
+    m0, m1 = np.uint64(0xD2511F53), np.uint64(0xCD9E8D57)
+    w0, w1 = np.uint64(0x9E3779B9), np.uint64(0xBB67AE85)
+    s32 = np.uint64(32)
+    for _ in range(10):
+        p0, p1 = x0 * m0, x2 * m1                   # < 2^64: exact in uint64
+        x0, x1, x2, x3 = (p1 >> s32) ^ x1 ^ k0, p1 & _M32, (p0 >> s32) ^ x3 ^ k1, p0 & _M32
+        k0, k1 = (k0 + w0) & _M32, (k1 + w1) & _M32
+    return np.stack([x0, x1, x2, x3], -1)
+
+
+def dropout_keep_c8(seed, offset, n, c, d, h, w, p):
+    """Keep mask bool [N,C,D,H,W] of the Philox dropout of csrc/common.cuh (dropout_keep8) for a layer of c channels:
+    vector vec = ((n*D + d)*C8 + c8)*H*W + h*W + w over the layer's own channel groups, counters 2*vec + offset and
+    2*vec + offset + 1 (mod 2^64) as (lo32, hi32, 0, 0), key (lo32(seed), hi32(seed)); the 8 output words feed channels
+    0..7 of the group; keep iff (r >> 8) * 2^-24 >= float32(p), i.e. (r >> 8) >= ceil(float32(p) * 2^24) exactly."""
+    assert c % 8 == 0
+    c8 = c // 8
+    seed, offset = int(seed) % (1 << 64), int(offset) % (1 << 64)
+    vec = np.arange(n * d * c8 * h * w, dtype=np.uint64)
+    ctr = vec * np.uint64(2) + np.uint64(offset)     # wraps mod 2^64 like the device's uint64
+    key = np.array([seed & 0xFFFFFFFF, seed >> 32], dtype=np.uint64)
+    zero = np.zeros_like(vec)
+    words = [philox4x32_10(np.stack([cc & _M32, cc >> np.uint64(32), zero, zero], -1), key)
+             for cc in (ctr, ctr + np.uint64(1))]
+    r = np.concatenate(words, -1)                    # [vec, 8]: a.x..a.w, b.x..b.w
+    thr = int(np.ceil(float(np.float32(p)) * 2.0 ** 24))
+    keep = (r >> np.uint64(8)) >= np.uint64(thr)
+    return torch.from_numpy(keep.reshape(n, d, c8, h, w, 8).transpose(0, 2, 5, 1, 3, 4).reshape(n, c, d, h, w).copy())
+
+
 def golden_voxels(out, g, key):
     """``out`` [N, C, ...] at the voxels a sampled golden array holds: g[key] is [N, C, M] at the flat voxel indices
     g[key + '_idx'] of an output of shape g[key + '_shape']."""

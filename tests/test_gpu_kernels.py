@@ -7,7 +7,7 @@ import pytest
 import torch
 import torch.nn.functional as F
 
-from tests._util import bf16_round, from_c8, max_rel, randn, rel_l2, to_c8
+from tests._util import bf16_round, dropout_keep_c8, from_c8, max_rel, randn, rel_l2, to_c8
 
 pytestmark = pytest.mark.gpu
 
@@ -352,6 +352,8 @@ def test_philox_dropout_statistics_and_backward_consistency():
         outs.append(from_c8(act).cpu())
     assert torch.equal(outs[0], outs[1]) and not torch.equal(outs[0], outs[2])
     kept = outs[0] != 0
+    # the exact mask of the host Philox restatement (also pins a mistake the backward pass would repeat)
+    assert torch.equal(kept, dropout_keep_c8(123, 16, n, c, d, h, w, p))
     assert abs(kept.float().mean().item() - (1 - p)) < 0.02
     assert torch.allclose(outs[0][kept], torch.tensor(1 / (1 - p)), rtol=1e-2)
     # per-channel keep rate is uniform too

@@ -18,7 +18,10 @@ from tests._util import rel_l2
 
 pytestmark = pytest.mark.gpu
 PARAMS = dict(bench.NET_PARAMS, dropout=[0.0] * 5)     # the oracle cannot reproduce the Philox masks; dropout parity is
-#                                                        covered by test_gpu_net.py::test_dropout_mask_injection_matches_oracle
+#                                                        covered by test_gpu_net.py::test_dropout_mask_injection_matches_oracle,
+#                                                        and the masks themselves are pinned bit for bit against the host
+#                                                        Philox of tests/_util.py (test_gpu_infer_kernels.py,
+#                                                        test_gpu_kernels.py::test_philox_dropout_*)
 LR = 1e-3                                              # 10x the bench's rate so that a stale-weight step would show
 
 
