@@ -231,9 +231,11 @@ __global__ void __launch_bounds__(kNumThreads) conv3d_tc_kernel(const __grid_con
         int acc = 0; uint32_t acc_phase = 0;
         int cur_slice = -1;
         constexpr int kMaxChunks = 8;                        // nb <= 128
-        float run[kMaxChunks];
+        // fp64 across tiles: fp32 running sums over the hundreds of tiles a warp walks at 16 SMs lose enough of sum y^2
+        // that var = E[y^2] - mean^2 is off by 2.5e-5 relative at mean/std = 30 (tests/test_gpu_train_kernels.py)
+        double run[kMaxChunks];
 #pragma unroll
-        for (int k = 0; k < kMaxChunks; ++k) run[k] = 0.0f;
+        for (int k = 0; k < kMaxChunks; ++k) run[k] = 0.0;
         const bool want_stats = P.stats != nullptr;
         const int nchunk16 = P.nb / 16;
         const float act_slope = fuse_act ? __ldg(P.act.slope) : 0.0f;
@@ -246,8 +248,8 @@ __global__ void __launch_bounds__(kNumThreads) conv3d_tc_kernel(const __grid_con
 #pragma unroll
                     for (int k = 0; k < kMaxChunks; ++k) {
                         if (k < nchunk16) {
-                            atomicAdd(P.stats + (lane >> 4) * P.cout + cur_slice * P.nb + k * 16 + (lane & 15), (double)run[k]);
-                            run[k] = 0.0f;
+                            atomicAdd(P.stats + (lane >> 4) * P.cout + cur_slice * P.nb + k * 16 + (lane & 15), run[k]);
+                            run[k] = 0.0;
                         }
                     }
                 }
@@ -322,7 +324,7 @@ __global__ void __launch_bounds__(kNumThreads) conv3d_tc_kernel(const __grid_con
                             v[16 + i] = v[i] * v[i];
                         }
                         warp_transpose_sum32(v, lane);
-                        run[k] += v[0];
+                        run[k] += (double)v[0];
                     }
                 }
             }
@@ -335,7 +337,7 @@ __global__ void __launch_bounds__(kNumThreads) conv3d_tc_kernel(const __grid_con
 #pragma unroll
             for (int k = 0; k < kMaxChunks; ++k)
                 if (k < nchunk16)
-                    atomicAdd(P.stats + (lane >> 4) * P.cout + cur_slice * P.nb + k * 16 + (lane & 15), (double)run[k]);
+                    atomicAdd(P.stats + (lane >> 4) * P.cout + cur_slice * P.nb + k * 16 + (lane & 15), run[k]);
         }
     }
     tc_fence_before();

@@ -1,6 +1,56 @@
 import numpy as np
 import torch
 
+DEV = "cuda:0"
+SENTINEL = 7.0
+FULL_SMS = 148
+
+
+def cdiv(a, b):
+    return -(-a // b)
+
+
+def bitwise_equal(a, b):
+    if a.dtype == torch.bfloat16:
+        return torch.equal(a.view(torch.int16), b.view(torch.int16))
+    return torch.equal(a.view(torch.int32), b.view(torch.int32))
+
+
+def slice_buf(x, c8tot, c8off):
+    """x [N,C,D,H,W] at channel group c8off of a C8-planar bf16 buffer of c8tot groups; other channels = SENTINEL."""
+    n, c, d, h, w = x.shape
+    full = torch.full((n, c8tot * 8, d, h, w), SENTINEL, device=x.device)
+    full[:, c8off * 8:c8off * 8 + c] = x
+    return to_c8(full.to(DEV))
+
+
+def sentinel_buf(n, d, c8tot, h, w):
+    return torch.full((n, d, c8tot, h, w, 8), SENTINEL, dtype=torch.bfloat16, device=DEV)
+
+
+def read_slice(buf, c8off, c, device="cpu"):
+    """The c channels at group c8off of a C8-planar buffer, after checking every other channel still holds SENTINEL."""
+    full = from_c8(buf).to(device)
+    lo, hi = c8off * 8, c8off * 8 + c
+    assert torch.all(full[:, :lo] == SENTINEL) and torch.all(full[:, hi:] == SENTINEL), "write outside the target slice"
+    return full[:, lo:hi]
+
+
+def run_sm_budgets(fn):
+    """[fn() under fpl_set_sm_budget(148), fn() under fpl_set_sm_budget(16)].  At 16 SMs the persistent grids are
+    16-32 CTAs, so a CTA walks several tiles (TMEM accumulator ping-pong, barrier phase wrap) or items; the budget is
+    always restored."""
+    from fplplus_b200 import ops
+    outs = []
+    try:
+        for sms in (FULL_SMS, 16):
+            ops.call("fpl_set_sm_budget", sms)
+            outs.append(fn())
+            torch.cuda.synchronize()
+    finally:
+        ops.call("fpl_set_sm_budget", FULL_SMS)
+    return outs
+
 
 def bf16_round(t):
     return t.to(torch.bfloat16).float()

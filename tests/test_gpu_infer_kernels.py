@@ -14,11 +14,8 @@ import pytest
 import torch
 import torch.nn.functional as F
 
-from tests._util import bf16_round, dropout_keep_c8, from_c8, max_rel, philox4x32_10, randn, to_c8
-
-DEV = "cuda:0"
-SENTINEL = 7.0
-FULL_SMS = 148
+from tests._util import (DEV, FULL_SMS, SENTINEL, bf16_round, bitwise_equal, cdiv, dropout_keep_c8, max_rel,
+                         philox4x32_10, randn, read_slice, run_sm_budgets, sentinel_buf, slice_buf, to_c8)
 
 
 def _ops():
@@ -68,46 +65,8 @@ def _st():
 
 @pytest.fixture
 def sm_budgets():
-    """run(fn) -> [fn() under fpl_set_sm_budget(148), fn() under fpl_set_sm_budget(16)].  At 16 SMs the persistent
-    grids are 16-32 CTAs, so a CTA walks several tiles (TMEM accumulator ping-pong, barrier phase wrap) or items; the
-    budget is always restored."""
-    def run(fn):
-        outs = []
-        try:
-            for sms in (FULL_SMS, 16):
-                _call("fpl_set_sm_budget", sms)
-                outs.append(fn())
-                torch.cuda.synchronize()
-        finally:
-            _call("fpl_set_sm_budget", FULL_SMS)
-        return outs
-    return run
-
-
-def _bitwise_equal(a, b):
-    if a.dtype == torch.bfloat16:
-        return torch.equal(a.view(torch.int16), b.view(torch.int16))
-    return torch.equal(a.view(torch.int32), b.view(torch.int32))
-
-
-def _slice_buf(x, c8tot, c8off):
-    """x [N,C,D,H,W] at channel group c8off of a C8-planar bf16 buffer of c8tot groups; other channels = SENTINEL."""
-    n, c, d, h, w = x.shape
-    full = torch.full((n, c8tot * 8, d, h, w), SENTINEL)
-    full[:, c8off * 8:c8off * 8 + c] = x
-    return to_c8(full.to(DEV))
-
-
-def _sentinel_buf(n, d, c8tot, h, w):
-    return torch.full((n, d, c8tot, h, w, 8), SENTINEL, dtype=torch.bfloat16, device=DEV)
-
-
-def _read_slice(buf, c8off, c):
-    """The c channels at group c8off of a C8-planar buffer, after checking every other channel still holds SENTINEL."""
-    full = from_c8(buf).cpu()
-    lo, hi = c8off * 8, c8off * 8 + c
-    assert torch.all(full[:, :lo] == SENTINEL) and torch.all(full[:, hi:] == SENTINEL), "write outside the target slice"
-    return full[:, lo:hi]
+    """run(fn) -> [fn() under fpl_set_sm_budget(148), fn() under fpl_set_sm_budget(16)] (tests/_util.py)."""
+    return run_sm_budgets
 
 
 def _bn_params(seed, c):
@@ -148,15 +107,11 @@ def _tc_image(wt, cin, cout, kd):
 # ------------------------------------------------------------------------------------------
 # host restatements of launch decisions (so that the case lists provably reach them)
 # ------------------------------------------------------------------------------------------
-def _cdiv(a, b):
-    return -(-a // b)
-
-
 def _tc_nsub(cin, cout, n, d, h, w):
     """The N split of conv3d_tc_launch (csrc/conv_tc.cu): make_config's nb, then nsub doubles (up to 4) while
     nb % (2*16*nsub) == 0, nb / (2*nsub) >= 32 and tiles * slices * nsub < 96."""
     nb = cout if cout <= 128 else next(b for b in (128, 64, 32, 16) if cout % b == 0)
-    mn = _cdiv(h, 16) * _cdiv(w, 8) * d * n * (cout // nb)
+    mn = cdiv(h, 16) * cdiv(w, 8) * d * n * (cout // nb)
     nsub = 1
     while nsub < 4 and nb % (nsub * 2 * 16) == 0 and nb // (nsub * 2) >= 32 and mn * nsub < 96:
         nsub *= 2
@@ -181,7 +136,7 @@ def _dfold_tail_split(cin, cout, n, d, h, w, sms):
     while tmem < dc * nb:
         tmem *= 2
     ctas = 2 if smem <= 110 * 1024 and tmem <= 256 else 1
-    total = _cdiv(h, 16) * _cdiv(w, 8) * _cdiv(d, dc) * n
+    total = cdiv(h, 16) * cdiv(w, 8) * cdiv(d, dc) * n
     grid = min(sms * ctas, total)
     rem = total % grid
     return rem > 0 and 2 * rem <= grid and dc >= 8 and dc % 2 == 0 and d % dc == 0
@@ -312,13 +267,13 @@ def _tc_act_setup(cin, cout, kd, shape, seed):
     bn = _bn_params(seed + 2, cout)
     scale, shift = _eval_affine(*bn)
     # input: the second half of a 2*cin concat buffer (the other half holds SENTINEL)
-    xb = _slice_buf(x, 2 * cin // 8, cin // 8)
+    xb = slice_buf(x, 2 * cin // 8, cin // 8)
     return x, wt, bn, scale, shift, xb, _tc_image(wt, cin, cout, kd)
 
 
 def _run_tc_act(xb, img, cin, cout, kd, shape, scale, shift, sl, p, seed, offset, seed_dev):
     n, d, h, w = shape
-    a = _sentinel_buf(n, d, cout // 8 + 2, h, w)                 # output: groups [1, 1 + cout/8) of a wider buffer
+    a = sentinel_buf(n, d, cout // 8 + 2, h, w)                 # output: groups [1, 1 + cout/8) of a wider buffer
     _call("fpl_conv3d_tc_act", _p(xb), 2 * cin // 8, cin // 8, _p(img), _p(a), cout // 8 + 2, 1, n, d, h, w, cin, cout, kd,
           _p(scale), _p(shift), _p(sl), p, seed, offset, _p(seed_dev), _st())
     return a
@@ -341,8 +296,8 @@ def test_conv3d_tc_act_matches_reference_with_the_exact_dropout_mask(cin, cout, 
     seed, offset = 0x5DEECE66D, 6 * n * d * (cout // 8) * h * w
     a148, a16 = sm_budgets(lambda: _run_tc_act(xb, img, cin, cout, kd, shape, scale, shift, sl, p, seed, offset, None))
     # an output voxel's accumulation order is fixed by its tile, not by the CTA that runs it
-    assert _bitwise_equal(a148, a16)
-    out = _read_slice(a148, 1, cout)
+    assert bitwise_equal(a148, a16)
+    out = read_slice(a148, 1, cout)
     pre = _prelu_affine(F.conv3d(x, wt, None, padding=(kd // 2, 1, 1)), scale, shift, slope)
     keep = dropout_keep_c8(seed, offset, n, cout, d, h, w, p) if p > 0 else torch.ones_like(pre, dtype=torch.bool)
     keep_scale = float(np.float32(1.0) / (np.float32(1.0) - np.float32(p)))
@@ -370,7 +325,7 @@ def test_conv3d_tc_act_seed_words_and_the_two_kernel_path():
         # the masks without the high words differ, so the assertions below tell a dropped word apart
         assert not torch.equal(keep, dropout_keep_c8(eff & 0xFFFFFFFF, offset & 0xFFFFFFFF, n, cout, d, h, w, p))
         a = _run_tc_act(xb, img, cin, cout, kd, shape, scale, shift, sl, p, seed, offset, dev)
-        out = _read_slice(a, 1, cout)
+        out = read_slice(a, 1, cout)
         _assert_dropped_exactly(out, pre, keep)
         assert max_rel(out, pre * keep * 2.0) < 6e-3
         # two-kernel path: conv + bias -> bf16 y, eval-mode finalize, activation pass with the same Philox stream
@@ -380,10 +335,10 @@ def test_conv3d_tc_act_seed_words_and_the_two_kernel_path():
         fin = [torch.empty(cout, device=DEV) for _ in range(4)]
         _call("fpl_dsbn_finalize", None, 0, _p(gamma.to(DEV)), _p(beta.to(DEV)), _p(mean.to(DEV)), _p(var.to(DEV)), None,
               0.1, 1e-5, 0, *[_p(t) for t in fin], cout, _st())
-        a2 = _sentinel_buf(n, d, cout // 8 + 2, h, w)
+        a2 = sentinel_buf(n, d, cout // 8 + 2, h, w)
         _call("fpl_dsbn_act_fwd", _p(y), _p(fin[0]), _p(fin[1]), _p(sl), _p(a2), cout // 8 + 2, 1, None, 0, 0, None, 0, p,
               None, seed, offset, _p(dev), n, d, h, w, cout, _st())
-        out2 = _read_slice(a2, 1, cout)
+        out2 = read_slice(a2, 1, cout)
         assert torch.equal(out == 0, out2 == 0)
         # the two-kernel path rounds the conv output to bf16 once more before the affine map
         assert max_rel(out2, out) < 6e-3
@@ -404,19 +359,19 @@ def test_conv3d_tc_dfold_act_matches_reference(cin, cout, shape, sm_budgets):
     sl = torch.tensor([slope], device=DEV)
     img = torch.empty(L.load().fpl_conv3d_dfold_image_bytes(cin, cout) // 2, dtype=torch.bfloat16, device=DEV)
     _call("fpl_conv3d_dfold_prep_weight", _p(wt.to(DEV)), cin, cout, 0, _p(img), _st())
-    xb = _slice_buf(x, 2 * cin // 8, cin // 8)                      # input: the second half of a concat buffer
+    xb = slice_buf(x, 2 * cin // 8, cin // 8)                      # input: the second half of a concat buffer
 
     def run():
         # output: the first half of a concat buffer, as the second unit of a down level writes it
-        a = _sentinel_buf(n, d, 2 * cout // 8, h, w)
+        a = sentinel_buf(n, d, 2 * cout // 8, h, w)
         _call("fpl_conv3d_tc_dfold_act", _p(xb), 2 * cin // 8, cin // 8, _p(img), _p(a), 2 * cout // 8, 0, n, d, h, w, cin,
               cout, _p(scale), _p(shift), _p(sl), _st())
         return a
 
     a148, a16 = sm_budgets(run)
     # an output plane sums its input planes z-1, z, z+1 in that order whichever CTA or (half) item runs it
-    assert _bitwise_equal(a148, a16)
-    out = _read_slice(a148, 0, cout)
+    assert bitwise_equal(a148, a16)
+    out = read_slice(a148, 0, cout)
     ref = _prelu_affine(F.conv3d(x, wt, None, padding=1), scale, shift, slope)
     assert max_rel(out, ref) < 6e-3                                 # bf16 output rounding only
 
@@ -442,14 +397,14 @@ def test_stem_k311_act_hi_lo_matches_fp32_reference(cout, shape, sm_budgets):
     _call("fpl_conv3d_k311_prep_weight", _p(w48.to(DEV)), 48, cout, _p(img), _st())
 
     def run():
-        a = _sentinel_buf(n, d, cout // 8 + 2, h, w)
+        a = sentinel_buf(n, d, cout // 8 + 2, h, w)
         _call("fpl_conv3d_tc_k311_act", _p(xs4), 4, 0, _p(img), _p(a), cout // 8 + 2, 1, n, d, h, w, 48, cout, 32,
               _p(scale), _p(shift), _p(sl), _st())
         return a
 
     a148, a16 = sm_budgets(run)
-    assert _bitwise_equal(a148, a16)
-    out = _read_slice(a148, 1, cout)
+    assert bitwise_equal(a148, a16)
+    out = read_slice(a148, 1, cout)
     ref = _prelu_affine(F.conv3d(xf, wf, None, padding=1), scale, shift, slope)
     assert max_rel(out, ref) < 4e-3                  # fp32-accurate operands (hi + lo), only the bf16 output rounding
 
@@ -470,10 +425,10 @@ def test_maxpool_c8_is_bit_exact(pool_kd, shape, kind):
     elif kind == "ties":
         x = (torch.round(x * 2) + 0.5) / 2               # few distinct non-zero values: many tied maxima
     xb = bf16_round(x)
-    a = _slice_buf(xb, c // 8 + 1, 1)
-    pooled = _sentinel_buf(n, d // pool_kd, c // 8 + 2, h // 2, w // 2)
+    a = slice_buf(xb, c // 8 + 1, 1)
+    pooled = sentinel_buf(n, d // pool_kd, c // 8 + 2, h // 2, w // 2)
     _call("fpl_maxpool_c8", _p(a), c // 8 + 1, 1, _p(pooled), c // 8 + 2, 1, pool_kd, n, d, h, w, c, _st())
-    got = _read_slice(pooled, 1, c)
+    got = read_slice(pooled, 1, c)
     # a max of bf16 values is one of them: exact
     assert torch.equal(got, F.max_pool3d(xb, (pool_kd, 2, 2)))
 
@@ -485,14 +440,14 @@ def test_maxpool_c8_equals_the_pooled_output_of_dsbn_act_fwd(pool_kd):
     y = to_c8(randn(351, n, c, d, h, w, scale=2.0).to(DEV))
     scale, shift = (randn(352, c, scale=0.3) + 1.0).to(DEV), randn(353, c, scale=0.2).to(DEV)
     sl = torch.tensor([0.2], device=DEV)
-    act = _sentinel_buf(n, d, c // 8 + 1, h, w)
+    act = sentinel_buf(n, d, c // 8 + 1, h, w)
     pooled = torch.zeros((n, d // pool_kd, c // 8, h // 2, w // 2, 8), dtype=torch.bfloat16, device=DEV)
     idx = torch.zeros(pooled.shape, dtype=torch.uint8, device=DEV)
     _call("fpl_dsbn_act_fwd", _p(y), _p(scale), _p(shift), _p(sl), _p(act), c // 8 + 1, 1, _p(pooled), c // 8, 0, _p(idx),
           pool_kd, 0.0, None, 0, 0, None, n, d, h, w, c, _st())
-    pooled2 = _sentinel_buf(n, d // pool_kd, c // 8, h // 2, w // 2)
+    pooled2 = sentinel_buf(n, d // pool_kd, c // 8, h // 2, w // 2)
     _call("fpl_maxpool_c8", _p(act), c // 8 + 1, 1, _p(pooled2), c // 8, 0, pool_kd, n, d, h, w, c, _st())
-    assert _bitwise_equal(pooled, pooled2)
+    assert bitwise_equal(pooled, pooled2)
 
 
 @pytest.mark.gpu
@@ -521,7 +476,7 @@ def test_head_conv_tc_matches_reference(classes, cin, shape, sm_budgets):
     w16[:classes], b16[:classes] = wt, b
     img = _tc_image(w16, cin, 16, 1)
     b16d = b16.to(DEV)
-    xb = _slice_buf(x, cin // 8 + 2, 1)                            # input from a slice of a wider buffer
+    xb = slice_buf(x, cin // 8 + 2, 1)                            # input from a slice of a wider buffer
     numel = n * classes * d * h * w
 
     def run():
@@ -530,7 +485,7 @@ def test_head_conv_tc_matches_reference(classes, cin, shape, sm_budgets):
         return buf
 
     b148, b16_run = sm_budgets(run)
-    assert _bitwise_equal(b148[:numel], b16_run[:numel])
+    assert bitwise_equal(b148[:numel], b16_run[:numel])
     assert bool(torch.isnan(b148[numel:]).all()) and bool(torch.isnan(b16_run[numel:]).all())
     got = b148[:numel].view(n, classes, d, h, w).cpu()
     ref = F.conv3d(x.double(), bf16_round(wt).double(), b.double(), padding=(0, 1, 1))
@@ -577,7 +532,7 @@ def _check_batch_staging(single, batch, max_count, ents, bad, wshape, image_byte
     call(ents, ws, imgs)
     torch.cuda.synchronize()
     for e, a, r in zip(ents, imgs, ref):
-        assert _bitwise_equal(a, r), e
+        assert bitwise_equal(a, r), e
 
 
 @pytest.mark.gpu
@@ -625,10 +580,10 @@ def test_pack_ncdhw_to_c8_rounds_to_nearest_even_and_accumulates_sums(c, groups)
     bits[mid] = (bits[mid] & ~0xFFFF) | 0x8000
     x = bits.view(torch.float32)
     tot = groups + 2
-    out = _sentinel_buf(n, d, tot, h, w)
+    out = sentinel_buf(n, d, tot, h, w)
     sums = torch.ones(c, device=DEV)                               # accumulated into
     _call("fpl_pack_ncdhw_to_c8", _p(x.to(DEV)), c, _p(out), tot, 1, groups, _p(sums), n, d, h, w, _st())
-    got = _read_slice(out, 1, groups * 8)
+    got = read_slice(out, 1, groups * 8)
     assert torch.equal(got[:, :c], x.to(torch.bfloat16).float())   # torch's fp32 -> bf16 is round-to-nearest-even
     assert torch.all(got[:, c:] == 0)                              # padding channels of the groups
     xd = x.double()
