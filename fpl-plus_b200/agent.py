@@ -26,9 +26,10 @@ What is different underneath (B200-first, SURVEY.md §8):
 * the CPU transform pipeline is replaced: without ``set_loaders`` / ``set_datasets``, a training
   run builds one ``DevicePatchSampler`` per domain from ``[dataset] {1,2}_train_csv`` and
   ``train_transform`` (datapath.py: volumes resident in HBM, RandomCrop / RandomFlip /
-  NormalizeWithMeanStd per step on the device); otherwise loaders are any iterables of batch dicts,
-  validation and test loaders always so; ``NpyVolumeDataset`` is the minimal built-in for ``.npy``
-  / ``.nii`` volumes.
+  NormalizeWithMeanStd per step on the device), validation sets from ``{1,2}_valid_csv`` and a
+  test set from ``test_csv`` (``DeviceVolumeSet``: NormalizeWithMeanStd + Pad of whole volumes on
+  the device, test predictions cropped back); otherwise loaders are any iterables of batch dicts;
+  ``NpyVolumeDataset`` is the minimal built-in for ``.npy`` / ``.nii`` volumes.
 
 As in the reference only ``training_all`` semantics train (``training()`` of the shipped
 ``dual=False`` cfgs has no ``backward()``; SURVEY.md §3.1): ``dual`` is accepted and both values
@@ -418,7 +419,9 @@ class SegmentationAgent(object):
         """agent_abstract.py:241-318: loaders come from set_loaders(), or are wrapped around the
         datasets given to set_datasets() with the cfg's batch sizes.  With neither, the training loaders are
         ``DevicePatchSampler``s built from ``[dataset] {1,2}_train_csv`` and ``train_transform``
-        (``datapath.samplers_from_config``): the volumes stay on the training GPU."""
+        (``datapath.samplers_from_config``): the volumes stay on the training GPU.  Likewise the validation loaders are
+        resident ``DeviceVolumeSet``s of ``{1,2}_valid_csv`` with ``valid_transform``, and the test loader a
+        ``DeviceVolumeSet`` of ``test_csv`` with ``test_transform`` that reads one volume at a time."""
         ds = self.config.get('dataset', {})
         bs = ds.get('train_batch_size', 1)
         if self.stage == 'train':
@@ -443,8 +446,21 @@ class SegmentationAgent(object):
                 sets = self.valid_set if isinstance(self.valid_set, (list, tuple)) else [self.valid_set]
                 self.valid_loaders = [torch.utils.data.DataLoader(s, batch_size=1, shuffle=False) for s in sets] \
                     + [None] * (2 - len(sets))
+            n_dom = min(2, int(self.config.get('network', {}).get('num_domains', 2)))
+            csvs = [ds.get('%d_valid_csv' % (d + 1)) if d < n_dom else None for d in range(2)]
+            if all(v is None for v in self.valid_loaders) and self.valid_set is None and any(csvs):
+                from .datapath import DeviceVolumeSet, eval_transform_from_config
+                spec = eval_transform_from_config(self.config, 'valid')
+                device = self._pick_device('training')
+                self.valid_loaders = [DeviceVolumeSet(c, device, ds.get('root_dir', '') or '', spec, resident=True)
+                                      if c else None for c in csvs]
         elif self.test_loader is None and self.test_set is not None:
             self.test_loader = torch.utils.data.DataLoader(self.test_set, batch_size=1, shuffle=False)
+        elif self.test_loader is None and ds.get('test_csv'):
+            from .datapath import DeviceVolumeSet, eval_transform_from_config
+            self.test_loader = DeviceVolumeSet(ds['test_csv'], self._pick_device('testing'), ds.get('root_dir', '') or '',
+                                               eval_transform_from_config(self.config, 'test'), resident=False,
+                                               labels=False)
 
     def create_network(self):
         if self.net is None:
@@ -903,7 +919,17 @@ class SegmentationAgent(object):
         return self.config['testing']['ckpt_name']
 
     # -- inference / pseudo labels / FPL image weights (agent_seg.py:834-964) -------------------
+    @staticmethod
+    def _crop(t, pad):
+        """``t`` [..., D, H, W] without the ``pad`` margins ((lo_d, lo_h, lo_w), (hi_d, hi_h, hi_w)) of the test volume's
+        Pad (Pad_inverse, agent_seg.py:938-947)."""
+        (ld, lh, lw), (hd, hh, hw) = pad
+        d, h, w = t.shape[-3:]
+        return t[..., ld:d - hd, lh:h - hh, lw:w - hw].contiguous()
+
     def infer(self, load_checkpoint=True):
+        if self.test_loader is None:
+            raise ValueError("no test volumes: set [dataset] test_csv, or give a test loader (set_loaders / set_datasets)")
         te = self.config['testing']
         domain = te['domian_label']                 # (sic) the reference's key
         self.FPL = te.get('fpl', False)
@@ -931,9 +957,17 @@ class SegmentationAgent(object):
             raise ValueError("fpl_mc_passes = %d not in [1, %d]" % (k_passes, fpl.max_mc_passes()))
         uncertainty_list, pending = {}, []
         outputs = {}
-        volumes = list(self.test_loader)
+        from .datapath import DeviceVolumeSet
+        invert = False
+        if isinstance(self.test_loader, DeviceVolumeSet):
+            # indexable cfg-built set: a rank reads only its own volumes
+            invert = self.test_loader.invert_pad
+            volumes = (self.test_loader[i] for i in shard_round_robin(range(len(self.test_loader)), self.rank, self.world))
+        else:
+            volumes = shard_round_robin(list(self.test_loader), self.rank, self.world)
         with torch.no_grad():
-            for data in shard_round_robin(volumes, self.rank, self.world):
+            for data in volumes:
+                box = data.get('pad') if invert else None
                 images = self._to_device(data['image'])
                 names = data['names']
                 name = names[0] if isinstance(names, (list, tuple)) else names
@@ -944,11 +978,15 @@ class SegmentationAgent(object):
                         passes = self.inferer.run(self.net, images, dl, mc_passes=k_passes)
                     else:
                         passes = [self.inferer.run(self.net, images, domain_label=dl) for _ in range(k_passes)]
+                    if box is not None:             # the uncertainty of the volume as it was read (agent_seg.py:900-910)
+                        passes = [self._crop(p, box) for p in passes]
                     stats, _ = fpl.mc_uncertainty(passes)
                     pending.append((name, stats))          # stays on the device until the loop ends
                 else:
                     pred = self.inferer.run(self.net, images, domain_label=dl)
-                    outputs[name] = fpl.pseudo_label(pred)
+                    lab = fpl.pseudo_label(pred)
+                    # argmax is per voxel: cropping the uint8 labels equals cropping the logits, at 1 byte per voxel
+                    outputs[name] = lab if box is None else self._crop(lab, box)
         if self.FPL:
             for name, stats in pending:
                 uncertainty_list[name] = [fpl.finish_uncertainty(stats)]

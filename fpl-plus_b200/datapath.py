@@ -23,6 +23,10 @@ uint8 [N,D,H,W], ``pixel_weight`` uint8 [N,1,D,H,W], ``image_weight`` fp32 [N] (
 ``sampler_args_from_config`` and ``load_train_csv`` build the samplers of a training ``.cfg`` (``[dataset]
 {1,2}_train_csv``, ``train_batch_size``, ``train_transform`` and its keys); ``SegmentationAgent`` uses them when no
 training loaders were given.
+
+Validation and test volumes are not cropped: ``eval_transform_from_config`` reads ``valid_transform`` / ``test_transform``
+(``NormalizeWithMeanStd``, ``Pad``), and ``DeviceVolumeSet`` reads the rows of ``{1,2}_valid_csv`` / ``test_csv``,
+uploads each raw volume and pads + normalises it in one kernel pair (``fpl_pad_normalize_volume``).
 """
 import random
 import struct
@@ -65,6 +69,33 @@ def pad_to(volume, out_size, mode="reflect"):
 def code_from_pixel_weight(w):
     """Agreement weight map {0, 0.5, 1} (data/get_pixel_weight.py:21-26) -> uint8 code {0, 1, 2}."""
     return np.rint(np.asarray(w, np.float32) * 2.0).astype(np.uint8)
+
+
+def _norm_modes(normalize, c_num):
+    """{channel: {mean, std, mask}} (``DevicePatchSampler``'s ``normalize``) -> (modes, ctypes tables) of the library's
+    normalising entry points: per channel 0 raw, 1 fixed mean / std, 2 statistics, 3 statistics of the voxels > 0."""
+    import ctypes
+    if c_num > 16:
+        raise ValueError("normalize: %d image channels, the device normalisation takes at most 16" % c_num)
+    modes, means, stds = [0] * c_num, [0.0] * c_num, [1.0] * c_num
+    for c, spec in dict(normalize).items():
+        spec = dict(spec or {})
+        unknown = set(spec) - {"mean", "std", "mask"}
+        if unknown:
+            raise ValueError("normalize[%r]: unknown keys %s" % (c, sorted(unknown)))
+        if not (isinstance(c, int) and 0 <= c < c_num):
+            raise ValueError("normalize: channel %r not in [0, %d)" % (c, c_num))
+        m, s = spec.get("mean"), spec.get("std")
+        if (m is None) != (s is None):
+            raise ValueError("normalize[%d]: give both mean and std, or neither" % c)
+        if m is not None:
+            if not float(s) > 0.0:
+                raise ValueError("normalize[%d]: std %r must be > 0" % (c, s))
+            modes[c], means[c], stds[c] = 1, float(m), float(s)
+        else:
+            modes[c] = 3 if spec.get("mask", False) else 2
+    return modes, {"mode": (ctypes.c_int * c_num)(*modes), "mean": (ctypes.c_float * c_num)(*means),
+                   "std": (ctypes.c_float * c_num)(*stds)}
 
 
 class DevicePatchSampler(object):
@@ -137,35 +168,15 @@ class DevicePatchSampler(object):
     def _norm_tables(self, normalize):
         """{channel: {mean, std, mask}} -> the per-channel (mode, mean, std) host arrays of fpl_gather_patches_norm and
         its statistics workspace (modes: 0 raw, 1 fixed, 2 patch statistics, 3 patch statistics of the voxels > 0)."""
-        import ctypes
         c_num = self.in_chns
-        if c_num > 16:
-            raise ValueError("normalize: %d image channels, the device normalisation takes at most 16" % c_num)
-        modes, means, stds = [0] * c_num, [0.0] * c_num, [1.0] * c_num
-        for c, spec in dict(normalize).items():
-            spec = dict(spec or {})
-            unknown = set(spec) - {"mean", "std", "mask"}
-            if unknown:
-                raise ValueError("normalize[%r]: unknown keys %s" % (c, sorted(unknown)))
-            if not (isinstance(c, int) and 0 <= c < c_num):
-                raise ValueError("normalize: channel %r not in [0, %d)" % (c, c_num))
-            m, s = spec.get("mean"), spec.get("std")
-            if (m is None) != (s is None):
-                raise ValueError("normalize[%d]: give both mean and std, or neither" % c)
-            if m is not None:
-                if not float(s) > 0.0:
-                    raise ValueError("normalize[%d]: std %r must be > 0" % (c, s))
-                modes[c], means[c], stds[c] = 1, float(m), float(s)
-            else:
-                modes[c] = 3 if spec.get("mask", False) else 2
+        modes, tables = _norm_modes(normalize, c_num)
         n, (pd, ph, pw) = self.batch, self.patch
         ws = None
         if self.device.type == "cuda" and any(m >= 2 for m in modes):
             from .lib import load
             nbytes = int(load().fpl_gather_patches_norm_workspace_bytes(n, c_num, pd, ph, pw))
             ws = torch.empty(nbytes // 8, dtype=torch.float64, device=self.device)
-        return {"mode": (ctypes.c_int * c_num)(*modes), "mean": (ctypes.c_float * c_num)(*means),
-                "std": (ctypes.c_float * c_num)(*stds), "ws": ws, "ws_bytes": 0 if ws is None else 8 * ws.numel()}
+        return dict(tables, ws=ws, ws_bytes=0 if ws is None else 8 * ws.numel())
 
     # -- the reference's random decisions ------------------------------------------------------------------
     def _next_volume(self):
@@ -355,20 +366,22 @@ def _squeeze3(a):
     return a[0] if a.ndim == 4 and a.shape[0] == 1 else a
 
 
+def _csv_rows(csv_path):
+    """The rows of a dataset CSV after its header row, without blank rows."""
+    import csv
+    with open(csv_path, newline="") as f:
+        return [r for r in list(csv.reader(f))[1:] if r and r[0].strip()]
+
+
 def load_train_csv(csv_path, root_dir="", host_transforms=()):
     """Volume dicts of ``DevicePatchSampler`` from a training CSV: a header row, then rows
     ``image,label[,pixel_weight,image_weight]`` (``artefacts.write_train_csv``) of ``.npy`` / ``.nii`` / ``.nii.gz``
     paths under ``root_dir``.  Labels become uint8, ``pixel_weight`` the agreement code, ``image_weight`` a float
     (1.0 when absent).  ``host_transforms`` (``sampler_args_from_config``) are applied to every volume in order."""
-    import csv
     import os
     from .artefacts import load_volume
-    with open(csv_path, newline="") as f:
-        rows = [r for r in csv.reader(f)][1:]
     vols = []
-    for row in rows:
-        if not row or not row[0].strip():
-            continue
+    for row in _csv_rows(csv_path):
         img = np.asarray(load_volume(os.path.join(root_dir, row[0])), np.float32)
         img = img[None] if img.ndim == 3 else img
         v = {"image": img, "name": row[0], "image_weight": 1.0}
@@ -404,3 +417,150 @@ def samplers_from_config(config, device, rank=0, world=1):
         vols = load_train_csv(a["csv"], a["root_dir"], a["host_transforms"])
         out.append(DevicePatchSampler(vols, device=device, **a["sampler"]))
     return out
+
+
+# -- validation / test volumes from a .cfg -----------------------------------------------------------------------------
+# keys of the evaluation transforms.  Pad's ``ceil_mode`` / ``inverse`` (default True) follow PyMIC 0.3's transform/pad.py;
+# like NormalizeWithMeanStd's ``mask`` / ``random_fill`` above, these names have not been re-checked against the reference
+# tree.
+_EVAL_TRANSFORM_KEYS = {
+    "normalizewithmeanstd": ("channels", "mean", "std", "mask", "random_fill", "inverse"),
+    "pad": ("output_size", "ceil_mode", "inverse"),
+    "labeltoprobability": ("class_num", "inverse"),
+}
+
+
+def eval_transform_from_config(config, stage):
+    """The transforms ``[dataset] <stage>_transform`` (``stage`` 'valid' or 'test') applies to whole volumes, without
+    touching a device or a file: {"normalize": None or {channel: {mean, std, mask}} (as ``DevicePatchSampler``),
+    "pad": None or {"output_size", "ceil_mode", "inverse"}, "stats_after_pad": bool}.
+
+    * ``NormalizeWithMeanStd`` (``_channels``, ``_mean``, ``_std``, ``_mask``): statistics of the source volume, or of
+      the padded volume when ``Pad`` is listed first (``stats_after_pad``);
+    * ``Pad`` (``_output_size``, ``_ceil_mode``, ``_inverse``): each axis of n voxels is padded to ``ceil(n / s) * s``
+      with ``ceil_mode``, to ``max(n, s)`` without; ``inverse`` (default True) crops the test predictions back;
+    * ``LabelToProbability`` is implied by the uint8 label; the ``_inverse`` keys of the other two are ignored.
+    Any other transform, any other key of these transforms, a transform listed twice and
+    ``NormalizeWithMeanStd_random_fill = True`` raise ``ValueError``.  An absent list means no transform."""
+    if stage not in ("valid", "test"):
+        raise ValueError("stage must be 'valid' or 'test', got %r" % (stage,))
+    ds = config.get("dataset", {})
+    names = ds.get(stage + "_transform") or []
+    names = [names] if isinstance(names, str) else names
+    out = {"normalize": None, "pad": None, "stats_after_pad": False}
+    seen = set()
+    for name in names:
+        key = str(name).lower()
+        if key not in _EVAL_TRANSFORM_KEYS:
+            raise ValueError("%s_transform: %s is not supported for whole validation / test volumes" % (stage, name))
+        if key in seen:
+            raise ValueError("%s_transform: %s is listed twice" % (stage, name))
+        seen.add(key)
+        params = {k[len(key) + 1:]: v for k, v in ds.items() if k.startswith(key + "_")}
+        bad = sorted(set(params) - set(_EVAL_TRANSFORM_KEYS[key]))
+        if bad:
+            raise ValueError("%s: unsupported key(s) %s" % (name, ", ".join("%s_%s" % (name, b) for b in bad)))
+        if key == "normalizewithmeanstd":
+            out["normalize"] = _normalize_spec(name, params)
+            out["stats_after_pad"] = out["pad"] is not None
+        elif key == "pad":
+            size = params.get("output_size")
+            if not isinstance(size, (list, tuple)) or len(size) != 3 or not all(isinstance(x, int) and x > 0 for x in size):
+                raise ValueError("%s needs %s_output_size: three positive integers, got %r" % (name, name, size))
+            out["pad"] = {"output_size": [int(x) for x in size], "ceil_mode": bool(params.get("ceil_mode", False)),
+                          "inverse": bool(params.get("inverse", True))}
+    return out
+
+
+def padded_shape(shape, pad):
+    """Spatial shape after ``Pad`` (``pad`` as in ``eval_transform_from_config``; None: unchanged)."""
+    if pad is None:
+        return tuple(int(n) for n in shape)
+    if pad["ceil_mode"]:
+        return tuple(-(-int(n) // s) * s for n, s in zip(shape, pad["output_size"]))
+    return tuple(max(int(n), s) for n, s in zip(shape, pad["output_size"]))
+
+
+def pad_normalize_volume(image, label, transform):
+    """One volume on the device through ``transform`` (``eval_transform_from_config``): ``image`` fp32 [C,D,H,W] and
+    ``label`` uint8 [D,H,W] or None, both contiguous CUDA tensors -> (image [C,oD,oH,oW], label or None, margins
+    ((lo_d, lo_h, lo_w), (hi_d, hi_h, hi_w)) or None when nothing was padded).  Padding and normalisation follow
+    ``pad_to`` and ``normalize_with_mean_std`` applied in the order the transform list gives."""
+    image = image.contiguous()
+    c = int(image.shape[0])
+    shape = tuple(int(n) for n in image.shape[1:])
+    if label is not None:
+        label = label.contiguous()
+        if tuple(label.shape) != shape:
+            raise ValueError("label %s and image %s differ in shape" % (tuple(label.shape), tuple(image.shape)))
+    out_shape = padded_shape(shape, transform["pad"])
+    norm = transform["normalize"]
+    if norm is None and out_shape == shape:
+        return image, label, None
+    modes, tab = _norm_modes(norm or {}, c)
+    ws, ws_bytes = None, 0
+    if any(m >= 2 for m in modes):
+        from .lib import load
+        ws_bytes = int(load().fpl_pad_normalize_volume_workspace_bytes(c, *shape, *out_shape))
+        ws = torch.empty(ws_bytes // 8, dtype=torch.float64, device=image.device)
+    out = torch.empty((c,) + out_shape, dtype=torch.float32, device=image.device)
+    out_lab = None if label is None else torch.empty(out_shape, dtype=torch.uint8, device=image.device)
+    call("fpl_pad_normalize_volume", ptr(image), ptr(label), c, *shape, *out_shape, tab["mode"], tab["mean"], tab["std"],
+         int(transform["stats_after_pad"]), ptr(ws), ws_bytes, ptr(out), ptr(out_lab), stream_ptr())
+    lo = tuple((o - n) // 2 for n, o in zip(shape, out_shape))
+    hi = tuple(o - n - l for n, o, l in zip(shape, out_shape, lo))
+    return out, out_lab, ((lo, hi) if any(lo) or any(hi) else None)
+
+
+class DeviceVolumeSet(object):
+    """The volumes of one validation or test CSV (header row, then ``image[,label]`` rows of ``.npy`` / ``.nii`` /
+    ``.nii.gz`` paths under ``root_dir``; further columns are ignored) on ``device``, each padded and normalised by
+    ``transform`` (``eval_transform_from_config``; None: as stored).
+
+    Item i is the batch dict ``SegmentationAgent.validation`` / ``infer`` consume: ``image`` fp32 [1,C,oD,oH,oW],
+    ``label`` uint8 [1,oD,oH,oW] when the row has one and ``labels`` is set, ``names`` [the row's image path], ``pad``
+    the margins of ``pad_normalize_volume`` (or None).  ``invert_pad``: whether predictions are to be cropped back by
+    ``pad`` (``Pad_inverse``).
+
+    ``resident=True`` (validation: the same volumes every ``iter_valid`` steps) reads, uploads and transforms every
+    volume once, here, and keeps them in device memory; ``resident=False`` (test: each volume is visited once) does it
+    on access, one volume at a time."""
+
+    def __init__(self, csv_path, device, root_dir="", transform=None, resident=True, labels=True):
+        self.rows = _csv_rows(csv_path)
+        self.device = torch.device(device)
+        self.root_dir = root_dir or ""
+        self.transform = transform or {"normalize": None, "pad": None, "stats_after_pad": False}
+        self.labels = bool(labels)
+        pad = self.transform["pad"]
+        self.invert_pad = pad is not None and pad["inverse"]
+        self._items = [self._load(i) for i in range(len(self.rows))] if resident else None
+
+    def __len__(self):
+        return len(self.rows)
+
+    def __getitem__(self, i):
+        if not 0 <= i < len(self.rows):
+            raise IndexError(i)
+        return self._items[i] if self._items is not None else self._load(i)
+
+    def __iter__(self):
+        for i in range(len(self.rows)):
+            yield self[i]
+
+    def _load(self, i):
+        import os
+        from . import artefacts
+        row = self.rows[i]
+        img = np.asarray(artefacts.load_volume(os.path.join(self.root_dir, row[0])), np.float32)
+        img = img[None] if img.ndim == 3 else img
+        x = torch.from_numpy(np.ascontiguousarray(img)).to(self.device)
+        y = None
+        if self.labels and len(row) > 1 and row[1].strip():
+            lab = _squeeze3(artefacts.load_volume(os.path.join(self.root_dir, row[1]))).astype(np.uint8)
+            y = torch.from_numpy(np.ascontiguousarray(lab)).to(self.device)
+        x, y, pad = pad_normalize_volume(x, y, self.transform)
+        batch = {"image": x[None], "names": [row[0]], "pad": pad}
+        if y is not None:
+            batch["label"] = y[None]
+        return batch

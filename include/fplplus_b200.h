@@ -141,6 +141,22 @@ int fpl_gather_patches_norm(const void* d_rows, int n, int c, int pd, int ph, in
                             const float* h_std, void* workspace, int64_t workspace_bytes, float* out_image,
                             uint8_t* out_label, uint8_t* out_code, void* stream);
 
+/* ---- validation / test inputs: Pad (transform/pad.py) and NormalizeWithMeanStd (transform/normalize.py) of ONE volume ----
+ * image: DEVICE fp32 [c][d][h][w]; label: DEVICE uint8 [d][h][w] or NULL (then out_label must be NULL too).  Writes
+ * out_image fp32 [c][od][oh][ow] and out_label uint8 [od][oh][ow] (od >= d, oh >= h, ow >= w; at most 2^30 voxels).
+ * Padding is datapath.pad_to's: lower margins (o - n) / 2 per axis; the image padded as NumPy 'reflect' (mirror without
+ * repeating the edge voxel, periodic with period 2(n - 1) for margins larger than n - 1), or as 'edge' when ANY axis has
+ * size 1; the label with constant 0.  h_mode / h_mean / h_std: as fpl_gather_patches_norm (c <= 16; modes 0 raw, 1 fixed,
+ * 2 statistics, 3 statistics of the voxels > 0, whole volume when none).  The statistics of modes 2 / 3 come from the
+ * source volume (stats_after_pad = 0: NormalizeWithMeanStd listed before Pad) or from the padded volume (1: Pad first;
+ * it is walked through the pad map, not materialised).  They are fp64 per-block sums in `workspace` (8-byte aligned, at
+ * least fpl_pad_normalize_volume_workspace_bytes(c, d, h, w, od, oh, ow) bytes; may be NULL when no channel has mode 2 or
+ * 3) reduced in a fixed order; the block count depends on the sizes alone, so the output is bitwise reproducible. */
+int64_t fpl_pad_normalize_volume_workspace_bytes(int c, int d, int h, int w, int od, int oh, int ow);
+int fpl_pad_normalize_volume(const float* image, const uint8_t* label, int c, int d, int h, int w, int od, int oh, int ow,
+                             const int* h_mode, const float* h_mean, const float* h_std, int stats_after_pad,
+                             void* workspace, int64_t workspace_bytes, float* out_image, uint8_t* out_label, void* stream);
+
 /* ---- optimiser: torch.optim.Adam(params, lr, weight_decay=wd) of net_run/get_optimizer.py:16-17 (coupled L2) ----------
  * ONE launch over all tensors.  d_segs: DEVICE table of nseg rows of 48 bytes
  *   { float* param; const float* grad; float* exp_avg; float* exp_avg_sq; float* step; int32 numel; int32 pad }
